@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — agent-steps/s of the MAPF hot path (step + observe) on B200, next to the CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one joint step + one observation build over all worlds of the rank (mapf_step_observe, one launch):
 the rollout loop's per-step env work (runner.py:64-100) with the policy excluded (SURVEY.md §8d).
@@ -15,6 +15,7 @@ memory and every step's per-agent results are copied back and read on the host, 
 65 536 worlds split over the ranks, configs[4] and configs[3] (all ranks take part, times are max over ranks);
 `roofline` for the dominant kernel (the fused step_observe_kernel) from CUDA events inside the timed region; `cpu_baseline` = the C port
 of the reference's algorithm (oracle/) on this box's host cores.  `--impl reference` times that CPU path alone.
+`--dump-outputs DIR` writes what the last timed step returned (rank 0) to DIR/<name>.npy, see dump_outputs().
 BENCH_E2E_DEBUG=1 prints the wall time of every e2e call on stderr.
 """
 from __future__ import annotations
@@ -183,6 +184,36 @@ def build_scenario(worlds, seed):
     from primal_ppo_b200 import random_scenario
     return random_scenario(worlds, H, WD, N_AGENTS, density=(0.0, 0.3), queue_len=16, seed=seed,
                            unique_maps=min(256, worlds), fov=FOV, num_channel=CH)
+
+
+def bench_inputs(worlds, dev, rank):
+    """The headline loop's inputs: the worlds and a device-resident ring of 8 joint actions, seeded from the rank only."""
+    import torch
+    sc = build_scenario(worlds, seed=100 + rank)
+    gen = torch.Generator(device=dev); gen.manual_seed(1234 + rank)
+    ring = [torch.randint(0, 5, (worlds, N_AGENTS), generator=gen, device=dev, dtype=torch.int8) for _ in range(8)]
+    return sc, ring
+
+
+DUMP_WORLDS = 512         # 512 worlds x ~64 KB of outputs = 33 MB on disk
+
+
+def dump_outputs(out_dir, res):
+    """Writes what one `env.step_observe` returned -- the StepOut fields, obs and vec -- as float32 .npy files (float64
+    for int32 fields), restricted to a fixed sample of DUMP_WORLDS worlds drawn with seed 0 and kept in world order.  The
+    bench's inputs depend only on its arguments, so two builds run with the same arguments can be compared file by file."""
+    import torch
+    out, obs, vec = res
+    W = obs.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(W, size=min(W, DUMP_WORLDS), replace=False))
+    idx_t = torch.from_numpy(idx).to(obs.device)
+    arrays = {f: getattr(out, f) for f in ("status", "reward", "cost", "train_valid", "goals_reached", "violated",
+                                           "shadow_goals", "fixed_actions")}
+    arrays.update(obs=obs, vec=vec)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.index_select(0, idx_t).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if a.dtype == np.int32 else np.float32))
 
 
 def _max_over_ranks(x, dev, world_size):
@@ -477,7 +508,12 @@ def main():
     ap.add_argument("--ppo-steps", type=int, default=256, help="rollout length T of the PPO extra")
     ap.add_argument("--sustained-seconds", type=float, default=2.0)
     ap.add_argument("--python-ref-budget", type=float, default=8.0, help="seconds per config of Python-reference timing")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -497,12 +533,10 @@ def main():
     Wn, N = args.worlds, N_AGENTS
     K, Wu = args.steps, max(args.warmup, 3)
 
-    sc = build_scenario(Wn, seed=100 + rank)
+    sc, ring = bench_inputs(Wn, dev, rank)
     env = BatchedMapfGym(sc, device=dev, seed=1234 + rank, use_tape=False)
     obs = torch.empty((Wn, N, CH, FOV, FOV), dtype=torch.float32, device=dev)     # the policy's input tensors
     vec = torch.empty((Wn, N, 4), dtype=torch.float32, device=dev)
-    gen = torch.Generator(device=dev); gen.manual_seed(1234 + rank)
-    ring = [torch.randint(0, 5, (Wn, N), generator=gen, device=dev, dtype=torch.int8) for _ in range(8)]
     env.getAllObservations(out=(obs, vec))
 
     def barrier():
@@ -577,9 +611,11 @@ def main():
         t_start = torch.cuda.Event(enable_timing=True); t_end = torch.cuda.Event(enable_timing=True)
         t_start.record()
         for i in range(K):
-            env.step_observe(ring[i % 8], obs_out=(obs, vec))
+            last = env.step_observe(ring[i % 8], obs_out=(obs, vec))
         t_end.record()
         barrier()
+    if args.dump_outputs and rank == 0:           # before the sections below step the env again
+        dump_outputs(args.dump_outputs, last)
     total_ms = t_start.elapsed_time(t_end)
     # the dominant kernel's average launch duration over the timed region: K back-to-back launches between two CUDA events
     # on the launching stream (one launch per step and nothing else in between)

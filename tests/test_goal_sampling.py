@@ -2,10 +2,8 @@
 (mapf_gym.py:189-190, 623-627 -> util.getFreeCell, util.py:67-76 on worldWithAgentsAndGoals(), :200-209).
 
 The CUDA path is held bit-exact to this restatement (same Philox stream; tests/test_gpu_round2.py).  Here, on the CPU:
-properties of the restatement, and its DISTRIBUTION against the live reference (authoring container only) — the reference
-draws from NumPy's global MT19937, so only the distribution can agree."""
+properties of the restatement — the reference draws from NumPy's global MT19937, so only the distribution can agree."""
 import numpy as np
-import pytest
 
 from oracle import OracleMapfGym
 from oracle.oracle import checksum_rows
@@ -102,43 +100,6 @@ def test_oracle_checksum_is_position_sensitive():
     assert s1[0] != s2[0] and s1[1] == s2[1]
     z = np.zeros((3, 8), dtype=np.float32)
     assert len(set(checksum_rows(z).tolist())) == 1 and checksum_rows(z)[0] != 0
-
-
-@pytest.mark.reference
-def test_goal_sampling_distribution_matches_live_reference():
-    """The reference's own sampler (MapfGym.getNextGoal -> util.getFreeCell on worldWithAgentsAndGoals) on the same
-    mid-step world: same support, and a chi-square two-sample test on the cell histogram."""
-    import sys
-    from golden_util import GOLDEN_DIR
-    sys.path.insert(0, GOLDEN_DIR)
-    from ref_loader import load_reference, reference_available
-    if not reference_available():
-        pytest.skip("live reference not present (GPU box)")
-    W = 20000
-    sc, ob, starts, goals = _one_world_many_times(W)
-    orc = OracleMapfGym(sc, seed=9, threads=4, use_tape=False, goal_sampling=True)
-    a = np.zeros((W, 3), dtype=np.int8)
-    a[:, 0] = 1
-    orc.step(a)
-    g = orc.state()["goal"][:, 0].astype(np.int64)
-    ours = np.zeros((10, 10), dtype=np.int64)
-    np.add.at(ours, (g[:, 0], g[:, 1]), 1)
-
-    mapf_gym, util, AP = load_reference(3)
-    seqs = [util.Sequence(itemsIn=[tuple(int(x) for x in starts[i]), tuple(int(x) for x in goals[i, 0])]) for i in range(3)]
-    env = mapf_gym.FixedMapfGym(-(ob.astype(np.int64)), seqs, (0, 0), (0, 1))
-    env.agentList[0].takeStep(1)                             # the state jointStep is in when agent 0 arrives (:621-626)
-    assert np.array_equal(env.agentList[0].getPos(), env.agentList[0].getGoal())
-    np.random.seed(123)
-    ref = np.zeros((10, 10), dtype=np.int64)
-    for _ in range(W):
-        r, c = mapf_gym.MapfGym.getNextGoal(env, env.worldWithAgentsAndGoals(), 0)      # mapf_gym.py:189-190, 626
-        ref[r, c] += 1
-    assert ((ref > 0) == (ours > 0)).all(), "same support: exactly the free cells"
-    m = ref > 0
-    chi2 = float((((ref[m] - ours[m]) ** 2) / (ref[m] + ours[m])).sum())
-    n = int(m.sum())
-    assert chi2 < n + 6 * np.sqrt(2 * n), (chi2, n)
 
 
 def test_packed_results_decoder_matches_oracle_outputs():

@@ -40,41 +40,6 @@ def test_oracle_matches_reference_trace(case):
     _check_oracle_against(Golden(case), case)
 
 
-LIVE_CASES = {
-    "live_10x10_n8": (dict(map="density", size=(10, 10), density=(0.15, 0.25), N=8, W=10, T=30, Q=8), 101),
-    "live_8x8_n8_dense": (dict(map="density", size=(8, 8), density=(0.25, 0.3), N=8, W=16, T=24, Q=8, greedy=0.6), 102),
-    "live_40x40_n32": (dict(map="density", size=(40, 40), density=(0.0, 0.3), N=32, W=2, T=12, Q=6), 103),
-    "live_warehouse_n3_eval": (dict(map="warehouse", size=(10, 14), N=3, W=4, T=40, Q=8, human="fixed", use_da=True, use_hp=True), 104),
-}
-
-
-@pytest.mark.reference
-@pytest.mark.parametrize("name", sorted(LIVE_CASES))
-def test_oracle_matches_live_reference_on_fresh_scenarios(name, tmp_path):
-    """Beyond the committed fixtures: run the UNMODIFIED reference right now (only where /root/reference exists) on
-    scenarios drawn with seeds that are not in tests/golden, and hold the oracle to the same bit-exact standard."""
-    import sys
-    from golden_util import GOLDEN_DIR
-    sys.path.insert(0, GOLDEN_DIR)
-    from ref_loader import reference_available
-    if not reference_available():
-        pytest.skip("live reference not present (GPU box)")
-    import make_golden
-    case, seed = LIVE_CASES[name]
-    make_golden.run_case(name, case, seed, out_dir=str(tmp_path))
-    d = dict(np.load(tmp_path / (name + ".npz")))
-
-    class _G(Golden):
-        def __init__(self, d):
-            from primal_ppo_b200.scenario import Scenario
-            self.name, self.d = name, d
-            self.scenario = Scenario.from_npz_dict(d)
-            shape = tuple(int(x) for x in d["obs_shape"])
-            self.obs = np.unpackbits(d["obs_bits"])[:int(np.prod(shape))].reshape(shape)
-            self.T = int(d["actions"].shape[0])
-    _check_oracle_against(_G(d), name)
-
-
 def test_oracle_gae_matches_reference_runner():
     import os
     from golden_util import GOLDEN_DIR
