@@ -166,6 +166,25 @@ int mapf_observe_bf16(MapfEnv *env, uint16_t *obs_bf16, float *vec, void *stream
 int mapf_step_observe_bf16(MapfEnv *env, const int8_t *actions, const MapfStepOut *out, uint16_t *obs_bf16, float *vec,
                            void *stream);
 
+/* Optional bit-packed format (NOT the reference's layout): one bit per observation cell.  obs_bits is u32 [W,N,AW] with
+ * AW = MAPF_OBS_BITS_WORDS(C, F): bit k of agent (w, i) is obs[w, i].flatten()[k] in the reference's [C,F,F] order, held in
+ * word k / 32 at bit k % 32 (LSB first); the padding bits of an agent's last word are 0.  Every agent has its own
+ * word-aligned record.  64 B per agent at 6 x 9 x 9 instead of 1944 B in f32: what lets a rollout buffer hold the
+ * observations of a large batch (mapf_unpack_obs expands them for the network).  obs_bits must be 4-byte aligned (16-byte
+ * aligned buffers with AW % 4 == 0 take 16-byte stores); vec is f32 [W,N,4] as in mapf_observe. */
+#define MAPF_OBS_BITS_WORDS(C, F) (((C) * (F) * (F) + 31) / 32)
+int mapf_observe_bits(MapfEnv *env, uint32_t *obs_bits, float *vec, void *stream);
+int mapf_step_observe_bits(MapfEnv *env, const int8_t *actions, const MapfStepOut *out, uint32_t *obs_bits, float *vec,
+                           void *stream);
+
+/* Gather-and-expand of bit-packed observations (no env handle): obs_bits is [src_rows, agents, AW] (a row = one world of
+ * one step); out[r] = the f32 (out_bf16 = 0) or bf16 (out_bf16 = 1) 0/1 values [agents, C, F, F] of source row rows[r]
+ * (rows NULL: row r), for r < n_rows.  A row index outside [0, src_rows) gives an all-zero row.  obs_bits 4-byte aligned,
+ * out aligned to its element size (16-byte aligned buffers take the fast path). */
+int mapf_unpack_obs(const uint32_t *obs_bits, int64_t src_rows, int32_t agents, int32_t num_channel, int32_t fov,
+                    const int64_t *rows /* NULL = rows 0..n_rows-1 */, int64_t n_rows, int32_t out_bf16, void *out,
+                    void *stream);
+
 /* makeBfsMap (mapf_gym.py:211-244) for the CURRENT goals.  agent_list: n flat ids (w*N+i), or NULL for all W*N
  * agents in order.  out: int16 [n,H,Wd]: -1 obstacle (and cells outside a world's dims), -2 unreached, >=0 distance. */
 int mapf_bfs(MapfEnv *env, const int32_t *agent_list, int64_t n, int16_t *out, void *stream);

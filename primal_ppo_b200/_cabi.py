@@ -15,8 +15,14 @@ EXPORTED = ["mapf_abi_version", "mapf_last_error", "mapf_create", "mapf_destroy"
             "mapf_get_state", "mapf_get_counters", "mapf_step_observe_host", "mapf_step_observe",
             "mapf_sample_actions", "mapf_generate_scenario",
             "mapf_observe_bf16", "mapf_step_observe_bf16", "mapf_state_bytes", "mapf_save_state", "mapf_load_state",
-            "mapf_get_human", "mapf_host_layout", "mapf_step_observe_host_begin", "mapf_step_observe_host_wait", "mapf_decode_results_host", "mapf_checksum_rows", "mapf_adv_moments", "mapf_ppo_loss"]
+            "mapf_get_human", "mapf_host_layout", "mapf_step_observe_host_begin", "mapf_step_observe_host_wait", "mapf_decode_results_host", "mapf_checksum_rows", "mapf_adv_moments", "mapf_ppo_loss",
+            "mapf_observe_bits", "mapf_step_observe_bits", "mapf_unpack_obs"]
 ABI_VERSION = 2
+
+def obs_bits_words(C: int, F: int) -> int:
+    """MAPF_OBS_BITS_WORDS(C, F): u32 words of one agent's record in the bit-packed observation format."""
+    return (C * F * F + 31) // 32
+
 
 ERR_NO_VIABLE, ERR_FIX_ITER_CAP, ERR_BAD_ACTION, ERR_TAPE, ERR_NO_FREE_CELL = 1, 2, 4, 8, 64
 
@@ -98,6 +104,9 @@ def load_library():
     lib.mapf_step_observe.argtypes = [vp, vp, C.POINTER(MapfStepOut), vp, vp, vp]
     lib.mapf_observe_bf16.argtypes = [vp, vp, vp, vp]
     lib.mapf_step_observe_bf16.argtypes = [vp, vp, C.POINTER(MapfStepOut), vp, vp, vp]
+    lib.mapf_observe_bits.argtypes = [vp, vp, vp, vp]
+    lib.mapf_step_observe_bits.argtypes = [vp, vp, C.POINTER(MapfStepOut), vp, vp, vp]
+    lib.mapf_unpack_obs.argtypes = [vp, i64, i32, i32, i32, vp, i64, i32, vp, vp]
     lib.mapf_bfs.argtypes = [vp, vp, i64, vp, vp]
     lib.mapf_bfs_refresh.argtypes = [vp, vp, vp, vp]
     lib.mapf_gae.argtypes = [vp, vp, vp, vp, C.c_double, C.c_double, i32, i64, vp, vp, vp]

@@ -252,20 +252,24 @@ __device__ __forceinline__ int prefetch_ahead(const EnvView &v) {
     return k == 15 ? -1 : (k ? k : 4) * prefetch_batch(v);
 }
 
+// Output format of the observation kernels: the reference's f32 layout, the same 0/1 values as bf16, or one bit per cell
+// (u32 [W, N, AW], AW = MAPF_OBS_BITS_WORDS(C, F): each agent's C*F*F bits LSB first in its own word-aligned record).
+enum ObsFormat { OBS_F32 = 0, OBS_BF16 = 1, OBS_BITS = 2 };
+
 // launchers implemented in the .cu files
 cudaError_t launch_reset(const EnvView &v, cudaStream_t s);
 cudaError_t launch_step(const EnvView &v, const int8_t *actions, const int8_t *status_in, const MapfStepOut &out,
                         int mode, int *work_counter, cudaStream_t s);
 cudaError_t launch_step_wide(const EnvView &v, const int8_t *actions, const int8_t *status_in, const MapfStepOut &out,
                              int mode, cudaStream_t s);
-cudaError_t launch_observe(const EnvView &v, float *obs, float *vec, int *work_counter, cudaStream_t s, int out_bf16 = 0);
+cudaError_t launch_observe(const EnvView &v, float *obs, float *vec, int *work_counter, cudaStream_t s, int fmt = OBS_F32);
 bool step_observe_fusable(const EnvView &v);
 cudaError_t launch_step_observe(const EnvView &v, const int8_t *actions, const MapfStepOut &out, float *obs, float *vec,
-                                int *work_counter, cudaStream_t s, int out_bf16 = 0);
+                                int *work_counter, cudaStream_t s, int fmt = OBS_F32);
 bool step_observe_wide_fusable(const EnvView &v);
 cudaError_t launch_step_observe_wide(const EnvView &v, const int8_t *actions, const MapfStepOut &out, float *obs, float *vec,
-                                     int *work_counter, cudaStream_t s, int out_bf16 = 0);
-cudaError_t launch_observe_wide(const EnvView &v, float *obs, float *vec, int *work_counter, cudaStream_t s, int out_bf16 = 0);
+                                     int *work_counter, cudaStream_t s, int fmt = OBS_F32);
+cudaError_t launch_observe_wide(const EnvView &v, float *obs, float *vec, int *work_counter, cudaStream_t s, int fmt = OBS_F32);
 cudaError_t launch_bfs(const EnvView &v, const int32_t *agent_list, long long n, const int32_t *n_dev, int16_t *out,
                        int scatter, int *work_counter, cudaStream_t s);
 cudaError_t launch_arrivals(const EnvView &v, const uint8_t *goals, int32_t *list, int32_t *n_dev, cudaStream_t s);
@@ -285,6 +289,9 @@ cudaError_t launch_ppo_loss(const MapfPpoLossConfig &cfg, long long n, const flo
 
 cudaError_t launch_sample_actions(const float *ps, long long rows, unsigned long long seed, uint32_t draw, int8_t *actions,
                                   float *chosen_p, cudaStream_t s);
+
+cudaError_t launch_unpack_obs(const uint32_t *bits, long long src_rows, int N, int C, int F, const int64_t *rows,
+                              long long n_rows, int out_bf16, void *out, cudaStream_t s);
 
 cudaError_t launch_checksum_rows(const uint32_t *data, long long rows, long long words, unsigned long long *out, cudaStream_t s);
 

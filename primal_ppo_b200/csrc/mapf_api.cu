@@ -263,15 +263,15 @@ static cudaError_t do_step(MapfEnv *e, const int8_t *actions, const int8_t *stat
 // One env step of the rollout loop: the warp-per-world fused kernel (N <= 32, one observation chunk), else the
 // CTA-per-world fused kernel (N <= 128), else the two launches back to back.  MAPF_DBG_FLAGS bit 0 forces the two launches.
 static cudaError_t do_step_observe(MapfEnv *e, const int8_t *actions, const MapfStepOut &o, float *obs, float *vec,
-                                   cudaStream_t s, int out_bf16) {
+                                   cudaStream_t s, int fmt) {
     const EnvView &v = e->v;
     if (!(v.dbg_flags & 1)) {
-        if (step_observe_fusable(v)) return launch_step_observe(v, actions, o, obs, vec, WC(e, WC_FUSED), s, out_bf16);
-        if (step_observe_wide_fusable(v)) return launch_step_observe_wide(v, actions, o, obs, vec, WC(e, WC_FUSED_WIDE), s, out_bf16);
+        if (step_observe_fusable(v)) return launch_step_observe(v, actions, o, obs, vec, WC(e, WC_FUSED), s, fmt);
+        if (step_observe_wide_fusable(v)) return launch_step_observe_wide(v, actions, o, obs, vec, WC(e, WC_FUSED_WIDE), s, fmt);
     }
     cudaError_t err = do_step(e, actions, nullptr, o, MODE_FUSED, s);
     if (err != cudaSuccess) return err;
-    return launch_observe(v, obs, vec, WC(e, WC_OBSERVE), s, out_bf16);
+    return launch_observe(v, obs, vec, WC(e, WC_OBSERVE), s, fmt);
 }
 
 int mapf_evaluate(MapfEnv *e, const int8_t *actions, const MapfStepOut *out, void *stream) {
@@ -315,7 +315,7 @@ int mapf_step_observe(MapfEnv *e, const int8_t *actions, const MapfStepOut *out,
     if (int rc = check_vec(vec, "mapf_step_observe")) return rc;
     if (!actions || !out || !obs || !vec) return fail(MAPF_E_NULL, "mapf_step_observe: null argument");
     if (int rc = check_step_n(e, "mapf_step_observe")) return rc;
-    CU(do_step_observe(e, actions, *out, obs, vec, (cudaStream_t)stream, 0));
+    CU(do_step_observe(e, actions, *out, obs, vec, (cudaStream_t)stream, OBS_F32));
     return MAPF_OK;
 }
 
@@ -324,7 +324,7 @@ int mapf_observe_bf16(MapfEnv *e, uint16_t *obs_bf16, float *vec, void *stream) 
     NEED_ENV("mapf_observe_bf16");
     if (int rc = check_vec(vec, "mapf_observe_bf16")) return rc;
     if (!obs_bf16 || !vec) return fail(MAPF_E_NULL, "mapf_observe_bf16: null argument");
-    CU(launch_observe(e->v, reinterpret_cast<float *>(obs_bf16), vec, WC(e, WC_OBSERVE), (cudaStream_t)stream, 1));
+    CU(launch_observe(e->v, reinterpret_cast<float *>(obs_bf16), vec, WC(e, WC_OBSERVE), (cudaStream_t)stream, OBS_BF16));
     return MAPF_OK;
 }
 
@@ -333,7 +333,49 @@ int mapf_step_observe_bf16(MapfEnv *e, const int8_t *actions, const MapfStepOut 
     if (int rc = check_vec(vec, "mapf_step_observe_bf16")) return rc;
     if (!actions || !out || !obs_bf16 || !vec) return fail(MAPF_E_NULL, "mapf_step_observe_bf16: null argument");
     if (int rc = check_step_n(e, "mapf_step_observe_bf16")) return rc;
-    CU(do_step_observe(e, actions, *out, reinterpret_cast<float *>(obs_bf16), vec, (cudaStream_t)stream, 1));
+    CU(do_step_observe(e, actions, *out, reinterpret_cast<float *>(obs_bf16), vec, (cudaStream_t)stream, OBS_BF16));
+    return MAPF_OK;
+}
+
+/* bit-packed variants: one bit per observation cell, u32 [W,N,MAPF_OBS_BITS_WORDS(C,F)] */
+static int check_bits(const uint32_t *obs_bits, const char *name) {
+    if (reinterpret_cast<uintptr_t>(obs_bits) & 3) return fail(MAPF_E_BAD_CONFIG, "%s: obs_bits must be 4-byte aligned", name);
+    return MAPF_OK;
+}
+
+int mapf_observe_bits(MapfEnv *e, uint32_t *obs_bits, float *vec, void *stream) {
+    NEED_ENV("mapf_observe_bits");
+    if (!obs_bits || !vec) return fail(MAPF_E_NULL, "mapf_observe_bits: null argument");
+    if (int rc = check_vec(vec, "mapf_observe_bits")) return rc;
+    if (int rc = check_bits(obs_bits, "mapf_observe_bits")) return rc;
+    CU(launch_observe(e->v, reinterpret_cast<float *>(obs_bits), vec, WC(e, WC_OBSERVE), (cudaStream_t)stream, OBS_BITS));
+    return MAPF_OK;
+}
+
+int mapf_step_observe_bits(MapfEnv *e, const int8_t *actions, const MapfStepOut *out, uint32_t *obs_bits, float *vec,
+                           void *stream) {
+    NEED_ENV("mapf_step_observe_bits");
+    if (!actions || !out || !obs_bits || !vec) return fail(MAPF_E_NULL, "mapf_step_observe_bits: null argument");
+    if (int rc = check_vec(vec, "mapf_step_observe_bits")) return rc;
+    if (int rc = check_bits(obs_bits, "mapf_step_observe_bits")) return rc;
+    if (int rc = check_step_n(e, "mapf_step_observe_bits")) return rc;
+    CU(do_step_observe(e, actions, *out, reinterpret_cast<float *>(obs_bits), vec, (cudaStream_t)stream, OBS_BITS));
+    return MAPF_OK;
+}
+
+int mapf_unpack_obs(const uint32_t *obs_bits, int64_t src_rows, int32_t agents, int32_t num_channel, int32_t fov,
+                    const int64_t *rows, int64_t n_rows, int32_t out_bf16, void *out, void *stream) {
+    if (!obs_bits || !out) return fail(MAPF_E_NULL, "mapf_unpack_obs: null argument");
+    if (src_rows < 0 || n_rows < 0) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: negative row count");
+    if (agents < 1 || agents > 254) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: agents must be in 1..254");
+    if (num_channel != 5 && num_channel != 6) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: num_channel must be 5 or 6");
+    if (fov < 3 || fov > 31 || (fov & 1) == 0) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: fov must be odd in 3..31");
+    if (out_bf16 != 0 && out_bf16 != 1) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: out_bf16 must be 0 or 1");
+    if (int rc = check_bits(obs_bits, "mapf_unpack_obs")) return rc;
+    if (reinterpret_cast<uintptr_t>(out) & (out_bf16 ? 1 : 3))
+        return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: out must be aligned to its element size");
+    if (n_rows == 0) return MAPF_OK;
+    CU(launch_unpack_obs(obs_bits, src_rows, agents, num_channel, fov, rows, n_rows, out_bf16, out, (cudaStream_t)stream));
     return MAPF_OK;
 }
 
@@ -576,7 +618,7 @@ int mapf_step_observe_host_begin(MapfEnv *e, const int8_t *actions_host, void *r
         slot_bytes = (size_t)e->lay.slot_bytes;
     }
     o.train_valid = train_valid_dev;
-    CU(do_step_observe(e, e->d_actions[k], o, obs_dev, vec_dev, s, 0));
+    CU(do_step_observe(e, e->d_actions[k], o, obs_dev, vec_dev, s, OBS_F32));
     CU(cudaEventRecord(e->ev_step[k], s));
     CU(cudaStreamWaitEvent(cs, e->ev_step[k], 0));
     CU(cudaMemcpyAsync(result_slot_host, e->d_slot[k], slot_bytes, cudaMemcpyDeviceToHost, cs));   // ONE copy

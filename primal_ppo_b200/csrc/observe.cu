@@ -24,7 +24,7 @@ namespace {
 using namespace ow;
 
 // C_T/F_T > 0: compile-time channels / FOV (the training configuration 6 x 9 x 9); 0: runtime values from EnvView.
-template <int C_T, int F_T, bool VEC4>
+template <int C_T, int F_T, bool VEC4, bool BITS>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, 4)
 observe_kernel(const EnvView v, float *__restrict__ obs, float *__restrict__ vec, const ObsLayout L,
                int *__restrict__ work_counter) {
@@ -77,53 +77,63 @@ observe_kernel(const EnvView v, float *__restrict__ obs, float *__restrict__ vec
         }
         __syncwarp();
         const int nr = (int16_t)(cur.ht.y & 0xffff), nc = (int16_t)((uint32_t)cur.ht.y >> 16);   // human.getNextPos()
-        observe_world<C_T, F_T, VEC4>(v, L, m, lut, w, Grp<32>(lane), cur.pw, cur.gw, nr, nc, obs, vec);
+        observe_world<C_T, F_T, VEC4, 32, BITS>(v, L, m, lut, w, Grp<32>(lane), cur.pw, cur.gw, nr, nc, obs, vec);
         w = w1;
         cur = nxt;
     }
     finish_work(work_counter, gridDim.x * (blockDim.x >> 5), lane);
 }
 
-template <int C_T, int F_T, bool VEC4>
+template <int C_T, int F_T, bool VEC4, bool BITS = false>
 cudaError_t launch_t(const EnvView &v, float *obs, float *vec, const ObsLayout &L, int wpb, int *counter, cudaStream_t stream) {
     const size_t smem = L.total * wpb;
-    cudaError_t e = cudaFuncSetAttribute(observe_kernel<C_T, F_T, VEC4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(observe_kernel<C_T, F_T, VEC4, BITS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int dev = 0, sms = 148, per_sm = 1;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, observe_kernel<C_T, F_T, VEC4>, wpb * 32, smem);
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, observe_kernel<C_T, F_T, VEC4, BITS>, wpb * 32, smem);
     if (per_sm < 1) per_sm = 1;
     // Store-dominated worlds (>= 32 KB of observations each) run best with FEWER resident warps: the HBM write path prefers
     // fewer, longer write streams (write-pattern benchmark: 16 warps/SM beat 32 by 2 %), and this kernel has no other
     // latency to hide.  In-process A/B at 40x40x32: 1 / 2 / 3 / 4 CTAs per SM = 0.613 / 0.608 / 0.612 / 0.622 ms.
-    if ((size_t)v.N * L.PB * (L.out_bf16 ? 2 : 4) >= 32768 && per_sm > 2) per_sm = 2;
+    if (obs_world_bytes(L, v.N) >= 32768 && per_sm > 2) per_sm = 2;
     const int need = (v.W + wpb - 1) / wpb;
     const int blocks = need < sms * per_sm ? need : sms * per_sm;
-    observe_kernel<C_T, F_T, VEC4><<<blocks, wpb * 32, smem, stream>>>(v, obs, vec, L, counter);
+    observe_kernel<C_T, F_T, VEC4, BITS><<<blocks, wpb * 32, smem, stream>>>(v, obs, vec, L, counter);
     return cudaGetLastError();
 }
 
 }  // namespace
 
-cudaError_t launch_observe(const EnvView &v, float *obs, float *vec, int *work_counter, cudaStream_t stream, int out_bf16) {
+cudaError_t launch_observe(const EnvView &v, float *obs, float *vec, int *work_counter, cudaStream_t stream, int fmt) {
     const int PB = v.C * v.F * v.F;
     // worlds whose block needs several warp passes: one CTA per world with shared staging (observe_wide.cu)
     if ((v.N > 32 || (size_t)v.N * ((PB + 31) / 32 + 2) * 4 * 2 > 24 * 1024 || (v.dbg_flags & 4)) && !(v.dbg_flags & 2)) {
-        const cudaError_t e = launch_observe_wide(v, obs, vec, work_counter, stream, out_bf16);
+        const cudaError_t e = launch_observe_wide(v, obs, vec, work_counter, stream, fmt);
         if (e != cudaErrorNotSupported) return e;
     }
     // chunk of agents handled per phase-1 pass: as many as fit ~24 KB of bit-string scratch per warp
     int CH = v.N < 32 ? v.N : 32;
     while (CH > 4 && (size_t)CH * ((PB + 31) / 32 + 2) * 4 * 2 > 24 * 1024) CH >>= 1;
-    const size_t al = out_bf16 ? 8 : 4;               // elements per 16-byte store
-    const bool vec4 = ((size_t)v.N * PB) % al == 0 && (CH >= v.N || ((size_t)CH * PB) % al == 0) &&
-                      (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
+    const size_t al = fmt == OBS_BF16 ? 8 : 4;        // elements per 16-byte store
     ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, CH);
-    L.out_bf16 = out_bf16;
+    L.fmt = fmt;
+    // bits: every agent's record is AW words, so any chunk starts on a 16-byte boundary when AW % 4 == 0
+    const bool vec4 = (fmt == OBS_BITS ? bits_words(L.PB) % 4 == 0
+                                       : ((size_t)v.N * PB) % al == 0 && (CH >= v.N || ((size_t)CH * PB) % al == 0)) &&
+                      (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
     int wpb = WARPS_PER_BLOCK;
     while (wpb > 1 && L.total * wpb > 200 * 1024) wpb >>= 1;
     if (L.total * wpb > 227 * 1024) return cudaErrorInvalidConfiguration;
+    if (fmt == OBS_BITS) {
+        if (v.C == 6 && v.F == 9) {
+            return vec4 ? launch_t<6, 9, true, true>(v, obs, vec, L, wpb, work_counter, stream)
+                        : launch_t<6, 9, false, true>(v, obs, vec, L, wpb, work_counter, stream);
+        }
+        return vec4 ? launch_t<0, 0, true, true>(v, obs, vec, L, wpb, work_counter, stream)
+                    : launch_t<0, 0, false, true>(v, obs, vec, L, wpb, work_counter, stream);
+    }
     if (v.C == 6 && v.F == 9) {
         return vec4 ? launch_t<6, 9, true>(v, obs, vec, L, wpb, work_counter, stream)
                     : launch_t<6, 9, false>(v, obs, vec, L, wpb, work_counter, stream);

@@ -19,7 +19,7 @@ using namespace ow;
 
 constexpr int WIDE_WARPS = 8;
 
-template <int C_T, int F_T, bool VEC4>
+template <int C_T, int F_T, bool VEC4, bool BITS>
 __global__ void __launch_bounds__(WIDE_WARPS * 32)
 observe_wide_kernel(const EnvView v, float *__restrict__ obs, float *__restrict__ vec, const ObsLayout L,
                     const int shared_bytes, const int per_warp, int *__restrict__ work_counter) {
@@ -71,7 +71,7 @@ observe_wide_kernel(const EnvView v, float *__restrict__ obs, float *__restrict_
         // ---- chunks of agents, round-robin over the warps ---------------------------------------------------------------
         for (int k = warp; k < nchunks; k += WIDE_WARPS) {
             const int c0 = k * L.CH;
-            observe_chunk<C_T, F_T, VEC4>(v, L, m, lut, w, Grp<32>(lane), c0, min(L.CH, N - c0), nr, nc, rows, cols, obs, vec);
+            observe_chunk<C_T, F_T, VEC4, 32, BITS>(v, L, m, lut, w, Grp<32>(lane), c0, min(L.CH, N - c0), nr, nc, rows, cols, obs, vec);
         }
         __syncthreads();
         // ---- un-scatter so that the next world starts from a clean grid ------------------------------------------------
@@ -92,7 +92,7 @@ observe_wide_kernel(const EnvView v, float *__restrict__ obs, float *__restrict_
 }  // namespace
 
 // Returns cudaErrorNotSupported when the shape is better served (or only served) by the warp-per-world kernel.
-cudaError_t launch_observe_wide(const EnvView &v, float *obs, float *vec, int *work_counter, cudaStream_t stream, int out_bf16) {
+cudaError_t launch_observe_wide(const EnvView &v, float *obs, float *vec, int *work_counter, cudaStream_t stream, int fmt) {
     const int PB = v.C * v.F * v.F;
     // chunk size: per-warp scratch (aw + wb) of at most ~12 KB, and at least one chunk per warp when N allows it
     int CH = 32;
@@ -100,14 +100,15 @@ cudaError_t launch_observe_wide(const EnvView &v, float *obs, float *vec, int *w
     if ((size_t)CH * ((PB + 31) / 32 + 2) * 4 * 2 > 28 * 1024) return cudaErrorNotSupported;
     ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, CH);
     L.alias = 0;
-    L.out_bf16 = out_bf16;
+    L.fmt = fmt;
     // the CTA-shared part: [obits | abits | grid | goals+cells]; make_layout put goals at off_goal (after the staging)
     const int shared_bytes = (int)(L.off_goal + (((size_t)v.N * 8 + 15) / 16) * 16);
     const int per_warp = (int)((((size_t)CH * L.AST * 4 + 15) / 16) * 16 + (((size_t)L.WB * 4 + 15) / 16) * 16);
     const size_t smem = (size_t)shared_bytes + (size_t)per_warp * WIDE_WARPS;
     if (smem > 200 * 1024) return cudaErrorNotSupported;
-    const size_t al = out_bf16 ? 8 : 4;
-    const bool vec4 = ((size_t)CH * PB) % al == 0 && ((size_t)v.N * PB) % al == 0 && (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
+    const size_t al = fmt == OBS_BF16 ? 8 : 4;
+    const bool vec4 = (fmt == OBS_BITS ? bits_words(L.PB) % 4 == 0 : ((size_t)CH * PB) % al == 0 && ((size_t)v.N * PB) % al == 0) &&
+                      (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
     int dev = 0, sms = 148, per_sm = 1;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -121,8 +122,13 @@ cudaError_t launch_observe_wide(const EnvView &v, float *obs, float *vec, int *w
         const int blocks = v.W < sms * per_sm ? v.W : sms * per_sm;                                                \
         observe_wide_kernel<__VA_ARGS__><<<blocks, WIDE_WARPS * 32, smem, stream>>>(v, obs, vec, L, shared_bytes, per_warp, work_counter); \
     } while (0)
-    if (v.C == 6 && v.F == 9) { if (vec4) LAUNCH(6, 9, true); else LAUNCH(6, 9, false); }
-    else { if (vec4) LAUNCH(0, 0, true); else LAUNCH(0, 0, false); }
+    if (fmt == OBS_BITS) {
+        if (v.C == 6 && v.F == 9) { if (vec4) LAUNCH(6, 9, true, true); else LAUNCH(6, 9, false, true); }
+        else { if (vec4) LAUNCH(0, 0, true, true); else LAUNCH(0, 0, false, true); }
+    } else {
+        if (v.C == 6 && v.F == 9) { if (vec4) LAUNCH(6, 9, true, false); else LAUNCH(6, 9, false, false); }
+        else { if (vec4) LAUNCH(0, 0, true, false); else LAUNCH(0, 0, false, false); }
+    }
 #undef LAUNCH
     return cudaGetLastError();
 }

@@ -11,13 +11,23 @@ __host__ __device__ inline size_t align16(size_t x) { return (x + 15) & ~(size_t
 
 constexpr int OBW = 4;   // packed obstacle words prefetched per lane (PW <= 128: up to 64x64 cells; 40x40 needs 52)
 
+// u32 stride of one agent's bit string in shared memory: one spare word (phase 1b reads word k+1), odd so that lane-strided
+// accesses are bank-conflict free
+__host__ __device__ inline int agent_stride(int PB) {
+    const int aw = (PB + 31) / 32 + 1;
+    return (aw & 1) ? aw : aw + 1;
+}
+
+// u32 words of one agent's record in OBS_BITS output: MAPF_OBS_BITS_WORDS(C, F)
+__host__ __device__ inline int bits_words(int PB) { return (PB + 31) / 32; }
+
 struct ObsLayout {
     int PB;      // bits per agent = C*F*F
     int AST;     // u32 stride of one agent's padded bit string (odd -> conflict-free lane-strided access)
     int CH;      // agents per chunk (<= 32)
     int WB;      // u32 words of the chunk bit string
     int alias;   // 1: the chunk bit string overlays the staging area (single chunk per world)
-    int out_bf16; // 0: f32 observations (the reference's layout); 1: the same 0/1 values as bf16 (optional, half the bytes)
+    int fmt;     // ObsFormat: OBS_F32 (the reference's layout), OBS_BF16 (same 0/1 values, half the bytes) or OBS_BITS
     int step_n, step_e;   // (32 G) / PB, (32 G) % PB: how (agent, bit) advances when the word index advances by G (the group width)
     size_t off_abits, off_grid, off_goal, off_aw, off_wb, total;
 };
@@ -26,13 +36,11 @@ struct ObsLayout {
 inline ObsLayout make_layout(int HP, int RW, int GS, int N, int C, int F, int CH, int G = 32) {
     ObsLayout L;
     L.PB = C * F * F;
-    int aw = (L.PB + 31) / 32 + 1;
-    if ((aw & 1) == 0) aw++;
-    L.AST = aw;
+    L.AST = agent_stride(L.PB);
     L.CH = CH;
     L.WB = (CH * L.PB + 31) / 32 + 2;
     L.alias = (CH >= N) ? 1 : 0;
-    L.out_bf16 = 0;
+    L.fmt = OBS_F32;
     L.step_n = (32 * G) / L.PB;
     L.step_e = (32 * G) % L.PB;
     size_t o = align16((size_t)HP * RW * 4);
@@ -49,6 +57,12 @@ inline ObsLayout make_layout(int HP, int RW, int GS, int N, int C, int F, int CH
     (void)staging;
     L.total = o;
     return L;
+}
+
+// Observation bytes one world stores in L's format (the launch rules that prefer fewer write streams key on it)
+inline size_t obs_world_bytes(const ObsLayout &L, int N) {
+    if (L.fmt == OBS_BITS) return (size_t)N * bits_words(L.PB) * 4;
+    return (size_t)N * L.PB * (L.fmt == OBS_BF16 ? 2 : 4);
 }
 
 __device__ __forceinline__ void or_bits(uint32_t *words, int p, uint32_t val, int nbits) {
@@ -96,10 +110,77 @@ __device__ __forceinline__ ObsSmem obs_carve(unsigned char *base, const ObsLayou
     return m;
 }
 
+// Phases 1b and 2 of the observation build: `nch` per-agent bit strings of PB bits (stride AST words, in shared memory)
+// are compacted into one contiguous bit string `wb` and expanded into f32 (fmt OBS_F32) or bf16 (OBS_BF16) 0/1 values at
+// agent c0 of row `row` of `obs` ([rows, N, PB] f32 or bf16 elements) with streaming stores.  Shared by observe_chunk and unpack_obs_kernel (obs_bits.cu), which stages packed records.
+template <bool VEC4, int G>
+__device__ __forceinline__ void expand_records(const uint32_t *aw, const int AST, uint32_t *wb, const uint4 *lut,
+                                               const Grp<G> &g, const int nch, const int PB, const int step_n,
+                                               const int step_e, const int fmt, float *obs, const size_t row, const int N,
+                                               const int c0) {
+    const int lane = g.gl;
+    // ---- phase 1b: compact to one contiguous bit string (word m <- 32 bits starting at agent n, bit e) ----------------
+    const int TB = nch * PB;
+    const int nwords = (TB + 31) >> 5;
+    {
+        int n = (lane << 5) / PB, e = (lane << 5) - n * PB;
+        for (int m = lane; m < nwords; m += G) {
+            const uint32_t *src = aw + n * AST;
+            uint32_t x = __funnelshift_r(src[e >> 5], src[(e >> 5) + 1], e & 31);
+            const int valid = PB - e;
+            if (valid < 32) {
+                x &= (1u << valid) - 1u;
+                if (n + 1 < nch) x |= aw[(n + 1) * AST] << valid;
+            }
+            wb[m] = x;
+            n += step_n; e += step_e;
+            if (e >= PB) { e -= PB; n += 1; }
+        }
+    }
+    g.sync();
+    // ---- phase 2: bits -> floats, streaming stores ---------------------------------------------------------------------
+    if (fmt == OBS_BF16) {
+        // optional bf16 output: 8 bits -> 8 bf16 (1.0 = 0x3F80) -> one 16-byte store; the expansion is plain ALU
+        uint16_t *dst16 = reinterpret_cast<uint16_t *>(obs) + (row * N + c0) * PB;
+        if (VEC4) {
+            const int n8 = TB >> 3;
+            for (int q = lane; q < n8; q += G) {
+                const uint32_t b = wb[q >> 2] >> ((q & 3) << 3);
+                const uint32_t x0 = (b & 1u) * 0x3F80u | (b & 2u) * 0x1FC00000u;
+                const uint32_t x1 = ((b >> 2) & 1u) * 0x3F80u | ((b >> 2) & 2u) * 0x1FC00000u;
+                const uint32_t x2 = ((b >> 4) & 1u) * 0x3F80u | ((b >> 4) & 2u) * 0x1FC00000u;
+                const uint32_t x3 = ((b >> 6) & 1u) * 0x3F80u | ((b >> 6) & 2u) * 0x1FC00000u;
+                st_stream_v4(reinterpret_cast<float *>(dst16 + ((size_t)q << 3)), x0, x1, x2, x3);
+            }
+            for (int f = (n8 << 3) + lane; f < TB; f += G) dst16[f] = ((wb[f >> 5] >> (f & 31)) & 1u) ? 0x3F80 : 0;
+        } else {
+            for (int f = lane; f < TB; f += G) dst16[f] = ((wb[f >> 5] >> (f & 31)) & 1u) ? 0x3F80 : 0;
+        }
+        g.sync();
+        return;
+    }
+    float *dst = obs + (row * N + c0) * PB;
+    if (VEC4) {
+        const int n4 = TB >> 2;
+        const int sh = (lane & 7) << 2;
+        const uint32_t *wp = wb + (lane >> 3);
+        float *d4 = dst + (lane << 2);
+#pragma unroll 4
+        for (int q = lane; q < n4; q += G, wp += G / 8, d4 += 4 * G) {
+            const uint4 val = lut[(*wp >> sh) & 15u];
+            st_stream_v4(d4, val.x, val.y, val.z, val.w);
+        }
+    } else {
+        for (int f = lane; f < TB; f += G) dst[f] = ((wb[f >> 5] >> (f & 31)) & 1u) ? 1.0f : 0.0f;
+    }
+    g.sync();
+}
+
 // One chunk of agents [c0, c0 + nch) of a staged world by one warp: phase 1 (per-agent bit strings), phase 1b
-// (compaction), phase 2 (bits -> f32, streaming stores).  `aw` / `wb` are this warp's scratch; everything else of `m` is
-// read-only here and may be shared by the warps of a CTA.
-template <int C_T, int F_T, bool VEC4, int G = 32>
+// (compaction), phase 2 (bits -> f32 / bf16, streaming stores) — or, in OBS_BITS, a direct store of the phase-1 strings.
+// `aw` / `wb` are this warp's scratch; everything else of `m` is read-only here and may be shared by the warps of a CTA.
+// BITS: the OBS_BITS instantiation (a separate one, so that the f32 / bf16 kernels compile exactly as without it).
+template <int C_T, int F_T, bool VEC4, int G = 32, bool BITS = false>
 __device__ __forceinline__ void observe_chunk(const EnvView &v, const ObsLayout &L, const ObsSmem &m, const uint4 *lut,
                                               const int w, const Grp<G> &g, const int c0, const int nch, const int nr,
                                               const int nc, const int rows, const int cols, float *__restrict__ obs,
@@ -204,61 +285,28 @@ __device__ __forceinline__ void observe_chunk(const EnvView &v, const ObsLayout 
             reinterpret_cast<float4 *>(vec)[(size_t)w * N + i] = o4;
         }
         g.sync();
-        // ---- phase 1b: compact to one contiguous bit string (word m <- 32 bits starting at agent n, bit e) --------
-        const int TB = nch * PB;
-        const int nwords = (TB + 31) >> 5;
-        {
-            int n = (lane << 5) / PB, e = (lane << 5) - n * PB;
-            for (int m = lane; m < nwords; m += G) {
-                const uint32_t *src = aw + n * AST;
-                uint32_t x = __funnelshift_r(src[e >> 5], src[(e >> 5) + 1], e & 31);
-                const int valid = PB - e;
-                if (valid < 32) {
-                    x &= (1u << valid) - 1u;
-                    if (n + 1 < nch) x |= aw[(n + 1) * AST] << valid;
-                }
-                wb[m] = x;
-                n += L.step_n; e += L.step_e;
-                if (e >= PB) { e -= PB; n += 1; }
-            }
-        }
-        g.sync();
-        // ---- phase 2: bits -> floats, streaming stores ---------------------------------------------------------
-        if (L.out_bf16) {
-            // optional bf16 output: 8 bits -> 8 bf16 (1.0 = 0x3F80) -> one 16-byte store; the expansion is plain ALU
-            uint16_t *dst16 = reinterpret_cast<uint16_t *>(obs) + ((size_t)w * N + c0) * PB;
+        if (BITS) {
+            // ---- bits output: the per-agent strings ARE the records (AW words each, padding bits 0); phases 1b and 2 are
+            //      skipped.  The chunk's nch * AW words are contiguous in HBM: 16-byte streaming stores when AW % 4 == 0.
+            const int AW = bits_words(PB);
+            uint32_t *dstw = reinterpret_cast<uint32_t *>(obs) + ((size_t)w * N + c0) * AW;
             if (VEC4) {
-                const int n8 = TB >> 3;
-                for (int q = lane; q < n8; q += G) {
-                    const uint32_t b = wb[q >> 2] >> ((q & 3) << 3);
-                    const uint32_t x0 = (b & 1u) * 0x3F80u | (b & 2u) * 0x1FC00000u;
-                    const uint32_t x1 = ((b >> 2) & 1u) * 0x3F80u | ((b >> 2) & 2u) * 0x1FC00000u;
-                    const uint32_t x2 = ((b >> 4) & 1u) * 0x3F80u | ((b >> 4) & 2u) * 0x1FC00000u;
-                    const uint32_t x3 = ((b >> 6) & 1u) * 0x3F80u | ((b >> 6) & 2u) * 0x1FC00000u;
-                    st_stream_v4(reinterpret_cast<float *>(dst16 + ((size_t)q << 3)), x0, x1, x2, x3);
+                const int n4 = (nch * AW) >> 2;
+                for (int q = lane; q < n4; q += G) {
+                    const int a = (q << 2) / AW, k = (q << 2) - a * AW;
+                    const uint32_t *src = aw + a * AST + k;
+                    st_stream_v4(reinterpret_cast<float *>(dstw + ((size_t)q << 2)), src[0], src[1], src[2], src[3]);
                 }
-                for (int f = (n8 << 3) + lane; f < TB; f += G) dst16[f] = ((wb[f >> 5] >> (f & 31)) & 1u) ? 0x3F80 : 0;
             } else {
-                for (int f = lane; f < TB; f += G) dst16[f] = ((wb[f >> 5] >> (f & 31)) & 1u) ? 0x3F80 : 0;
+                for (int m = lane; m < nch * AW; m += G) {
+                    const int a = m / AW;
+                    dstw[m] = aw[a * AST + (m - a * AW)];
+                }
             }
             g.sync();
             return;
         }
-        float *dst = obs + ((size_t)w * N + c0) * PB;
-        if (VEC4) {
-            const int n4 = TB >> 2;
-            const int sh = (lane & 7) << 2;
-            const uint32_t *wp = wb + (lane >> 3);
-            float *d4 = dst + (lane << 2);
-#pragma unroll 4
-            for (int q = lane; q < n4; q += G, wp += G / 8, d4 += 4 * G) {
-                const uint4 val = lut[(*wp >> sh) & 15u];
-                st_stream_v4(d4, val.x, val.y, val.z, val.w);
-            }
-        } else {
-            for (int f = lane; f < TB; f += G) dst[f] = ((wb[f >> 5] >> (f & 31)) & 1u) ? 1.0f : 0.0f;
-        }
-        g.sync();
+        expand_records<VEC4, G>(aw, AST, wb, lut, g, nch, PB, L.step_n, L.step_e, L.fmt, obs, (size_t)w, N, c0);
     }
 }
 
@@ -266,7 +314,7 @@ __device__ __forceinline__ void observe_chunk(const EnvView &v, const ObsLayout 
 // from HBM); (nr, nc) = human.getNextPos(); the obstacle bit rows are already staged in m.obits and m.abits / m.grid
 // are clean on entry.  On exit they are clean again unless L.alias (then the caller re-zeroes them for the next world).
 // C_T/F_T > 0: compile-time channels / FOV (the training configuration 6 x 9 x 9); 0: runtime values from EnvView.
-template <int C_T, int F_T, bool VEC4, int G = 32>
+template <int C_T, int F_T, bool VEC4, int G = 32, bool BITS = false>
 __device__ __forceinline__ void observe_world(const EnvView &v, const ObsLayout &L, const ObsSmem &m, const uint4 *lut,
                                               const int w, const Grp<G> &g, const uint32_t pw_reg, const uint32_t gw_reg,
                                               const int nr, const int nc, float *__restrict__ obs,
@@ -291,7 +339,7 @@ __device__ __forceinline__ void observe_world(const EnvView &v, const ObsLayout 
         g.sync();
 
         for (int c0 = 0; c0 < N; c0 += CH)
-            observe_chunk<C_T, F_T, VEC4, G>(v, L, m, lut, w, g, c0, min(CH, N - c0), nr, nc, rows, cols, obs, vec);
+            observe_chunk<C_T, F_T, VEC4, G, BITS>(v, L, m, lut, w, g, c0, min(CH, N - c0), nr, nc, rows, cols, obs, vec);
         if (!L.alias) {
             // un-scatter this world's agents so the next world starts from a clean grid
             for (int i = lane; i < N; i += G) {

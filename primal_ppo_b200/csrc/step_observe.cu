@@ -24,7 +24,7 @@ using namespace ow;
 // Why groups: with 8 agents per world (BASELINE configs[1]) a warp-per-world step keeps 8 of 32 lanes busy and a world still
 // costs ~15 us of dependent work, so the step phase — not the 15 KB of stores per world — bounded the launch (0.62 of the
 // HBM roofline at 65 536 x 20x20x8).
-template <int C_T, int F_T, bool VEC4, int MINB, int G>
+template <int C_T, int F_T, bool VEC4, int MINB, int G, bool BITS>
 __global__ void __launch_bounds__(WARPS_PER_BLOCK * 32, MINB)
 step_observe_kernel(const EnvView v, const int8_t *__restrict__ actions, const MapfStepOut out, float *__restrict__ obs,
                     float *__restrict__ vec, const ObsLayout L, const int per_group, const int step_off,
@@ -92,7 +92,7 @@ step_observe_kernel(const EnvView v, const int8_t *__restrict__ actions, const M
             g.sync();
             // the human has ticked: its getNextPos() is the `next` field of the following trace entry
             const int nr = (int16_t)(cur.ht2.y & 0xffff), nc = (int16_t)((uint32_t)cur.ht2.y >> 16);
-            observe_world<C_T, F_T, VEC4, G>(v, L, m, lut, w, g, new_pw, new_gw, nr, nc, obs, vec);
+            observe_world<C_T, F_T, VEC4, G, BITS>(v, L, m, lut, w, g, new_pw, new_gw, nr, nc, obs, vec);
         }
         wb = wb1;
         w = w1;
@@ -101,7 +101,7 @@ step_observe_kernel(const EnvView v, const int8_t *__restrict__ actions, const M
     finish_work(work_counter, gridDim.x * (blockDim.x >> 5), lane);
 }
 
-template <int C_T, int F_T, bool VEC4, int MINB, int G>
+template <int C_T, int F_T, bool VEC4, int MINB, int G, bool BITS>
 cudaError_t launch_tb(const EnvView &v, const int8_t *actions, const MapfStepOut &out, float *obs, float *vec,
                       const ObsLayout &L, int *counter, cudaStream_t stream) {
     constexpr int MPW = 32 / G;
@@ -110,7 +110,7 @@ cudaError_t launch_tb(const EnvView &v, const int8_t *actions, const MapfStepOut
     const int wpb = WARPS_PER_BLOCK;
     const size_t smem = (size_t)per_group * MPW * wpb;
     if (smem > 227 * 1024) return cudaErrorInvalidConfiguration;
-    auto kern = step_observe_kernel<C_T, F_T, VEC4, MINB, G>;
+    auto kern = step_observe_kernel<C_T, F_T, VEC4, MINB, G, BITS>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int dev = 0, sms = 148, per_sm = 1;
@@ -128,14 +128,14 @@ cudaError_t launch_tb(const EnvView &v, const int8_t *actions, const MapfStepOut
 // As in observe.cu fewer write streams help store-dominated worlds (>= 32 KB of observations each), but here the step
 // phase needs warps to hide behind: in-process A/B at 40x40x32: 2 / 3 / 4 CTAs per SM = 0.772 / 0.722 / 0.731 ms.  The
 // 3-CTA instantiation is also COMPILED for 3 CTAs (80 registers instead of 64, no spills): 0.706 vs 0.721 ms.
-template <int C_T, int F_T, bool VEC4>
+template <int C_T, int F_T, bool VEC4, bool BITS = false>
 cudaError_t launch_t(const EnvView &v, const int8_t *actions, const MapfStepOut &out, float *obs, float *vec,
                      const ObsLayout &L, int G, int *counter, cudaStream_t stream) {
-    const bool big = (size_t)v.N * L.PB * (L.out_bf16 ? 2 : 4) >= 32768;
-    if (G == 8) return launch_tb<C_T, F_T, VEC4, 4, 8>(v, actions, out, obs, vec, L, counter, stream);
-    if (G == 16) return launch_tb<C_T, F_T, VEC4, 4, 16>(v, actions, out, obs, vec, L, counter, stream);
-    if (big) return launch_tb<C_T, F_T, VEC4, 3, 32>(v, actions, out, obs, vec, L, counter, stream);
-    return launch_tb<C_T, F_T, VEC4, 4, 32>(v, actions, out, obs, vec, L, counter, stream);
+    const bool big = obs_world_bytes(L, v.N) >= 32768;
+    if (G == 8) return launch_tb<C_T, F_T, VEC4, 4, 8, BITS>(v, actions, out, obs, vec, L, counter, stream);
+    if (G == 16) return launch_tb<C_T, F_T, VEC4, 4, 16, BITS>(v, actions, out, obs, vec, L, counter, stream);
+    if (big) return launch_tb<C_T, F_T, VEC4, 3, 32, BITS>(v, actions, out, obs, vec, L, counter, stream);
+    return launch_tb<C_T, F_T, VEC4, 4, 32, BITS>(v, actions, out, obs, vec, L, counter, stream);
 }
 
 }  // namespace
@@ -151,12 +151,12 @@ static int obs_chunk(const EnvView &v) {
 // Lanes per world: the narrowest lane group that holds the agents (8 / 16 / 32), provided the worlds are small enough for
 // a warp to stage 32 / G of them (shared memory for at least three CTAs per SM) and below the store-dominated regime;
 // MAPF_DBG_FLAGS bit 28 keeps one world per warp (A/B runs).
-static int group_width(const EnvView &v, int out_bf16) {
+static int group_width(const EnvView &v, int fmt) {
     if (v.N > 16 || (v.dbg_flags & (1 << 28)) || obs_chunk(v) < v.N) return 32;
-    const int PB = v.C * v.F * v.F;
-    if ((size_t)v.N * PB * (out_bf16 ? 2 : 4) >= 32768) return 32;
     const int G = v.N <= 8 ? 8 : 16;
-    const ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, obs_chunk(v), G);
+    ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, obs_chunk(v), G);
+    L.fmt = fmt;
+    if (obs_world_bytes(L, v.N) >= 32768) return 32;
     const size_t per_cta = (L.total + sw::step_scratch_bytes(G)) * (32 / G) * WARPS_PER_BLOCK;
     if (per_cta > 72 * 1024) return 32;
     if (v.PW > sw::SOBW * G * 4) return 32;       // keep the register-prefetched obstacle words useful
@@ -172,13 +172,22 @@ bool step_observe_fusable(const EnvView &v) {
 }
 
 cudaError_t launch_step_observe(const EnvView &v, const int8_t *actions, const MapfStepOut &out, float *obs, float *vec,
-                                int *work_counter, cudaStream_t stream, int out_bf16) {
+                                int *work_counter, cudaStream_t stream, int fmt) {
     const int PB = v.C * v.F * v.F;
     const int CH = obs_chunk(v);
-    const bool vec4 = ((size_t)v.N * PB) % (out_bf16 ? 8 : 4) == 0 && (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
-    const int G = group_width(v, out_bf16);
+    const int G = group_width(v, fmt);
     ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, CH, G);
-    L.out_bf16 = out_bf16;
+    L.fmt = fmt;
+    const bool vec4 = (fmt == OBS_BITS ? bits_words(L.PB) % 4 == 0 : ((size_t)v.N * PB) % (fmt == OBS_BF16 ? 8 : 4) == 0) &&
+                      (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
+    if (fmt == OBS_BITS) {
+        if (v.C == 6 && v.F == 9) {
+            return vec4 ? launch_t<6, 9, true, true>(v, actions, out, obs, vec, L, G, work_counter, stream)
+                        : launch_t<6, 9, false, true>(v, actions, out, obs, vec, L, G, work_counter, stream);
+        }
+        return vec4 ? launch_t<0, 0, true, true>(v, actions, out, obs, vec, L, G, work_counter, stream)
+                    : launch_t<0, 0, false, true>(v, actions, out, obs, vec, L, G, work_counter, stream);
+    }
     if (v.C == 6 && v.F == 9) {
         return vec4 ? launch_t<6, 9, true>(v, actions, out, obs, vec, L, G, work_counter, stream)
                     : launch_t<6, 9, false>(v, actions, out, obs, vec, L, G, work_counter, stream);

@@ -26,7 +26,7 @@ using namespace sww;
 // WARPS per CTA / MINB resident CTAs per SM the kernel is compiled for.  The step phase of a world is latency-bound
 // (~20 us: eight barrier-separated phases, global loads, thread-0 sections) and only hides under the stores of OTHER
 // worlds, so what matters is the number of worlds in flight per SM = resident CTAs; small CTAs give more of them.
-template <int C_T, int F_T, bool VEC4, int FW_WARPS, int MINB>
+template <int C_T, int F_T, bool VEC4, bool BITS, int FW_WARPS, int MINB>
 __global__ void __launch_bounds__(FW_WARPS * 32, MINB)
 step_observe_wide_kernel(const EnvView v, const int8_t *__restrict__ actions, const MapfStepOut out, float *__restrict__ obs,
                          float *__restrict__ vec, const ObsLayout L, const int shared_bytes, const int scratch_off,
@@ -87,7 +87,7 @@ step_observe_wide_kernel(const EnvView v, const int8_t *__restrict__ actions, co
         // ---- phase B: chunks of agents, round-robin over the warps -----------------------------------------------------------
         for (int k = warp; k < nchunks; k += FW_WARPS) {
             const int c0 = k * L.CH;
-            observe_chunk<C_T, F_T, VEC4>(v, L, m, lut, w, Grp<32>(lane), c0, min(L.CH, N - c0), nr, nc, rows, cols, obs, vec);
+            observe_chunk<C_T, F_T, VEC4, 32, BITS>(v, L, m, lut, w, Grp<32>(lane), c0, min(L.CH, N - c0), nr, nc, rows, cols, obs, vec);
         }
         __syncthreads();
         for (int i = tid; i < N; i += blockDim.x) {        // un-scatter: the next world starts from a clean grid
@@ -111,7 +111,7 @@ struct WidePlan {
     bool ok;
 };
 
-WidePlan make_plan(const EnvView &v, int out_bf16, int FW_WARPS) {
+WidePlan make_plan(const EnvView &v, int fmt, int FW_WARPS) {
     WidePlan p;
     p.ok = false;
     const int PB = v.C * v.F * v.F;
@@ -124,7 +124,7 @@ WidePlan make_plan(const EnvView &v, int out_bf16, int FW_WARPS) {
     // Balanced chunks: with `r` rounds every warp builds r chunks of CH = ceil(N / (warps * r)) agents, rounded up so that a
     // chunk's block stays 16-byte aligned (vector stores); the smallest r whose scratch fits the budget wins.  (Power-of-two
     // chunks left 33 agents as 5 chunks of 8 on 4 warps — one warp with twice the work — and 48 agents as 6.)
-    const int need_al = out_bf16 ? 8 : 4;
+    const int need_al = fmt == OBS_BF16 ? 8 : 4;                   // (bits: records are word-aligned; f32 rule kept)
     int g = need_al;
     while (g > 1 && PB % g) g >>= 1;
     const int mult = need_al / g;                                   // CH must be a multiple of this
@@ -139,7 +139,7 @@ WidePlan make_plan(const EnvView &v, int out_bf16, int FW_WARPS) {
     if (per_warp_bytes(CH) > 28 * 1024) return p;
     p.L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, CH);
     p.L.alias = 0;
-    p.L.out_bf16 = out_bf16;
+    p.L.fmt = fmt;
     // [obits | abits | grid | goals + cells] shared by the CTA, then the per-warp observation scratch (aw, wb).  The step
     // phase's scratch is dead once the post-step cells / goals have been handed over, and the observation scratch is dead
     // during the step phase: they overlay each other (a __syncthreads separates the two uses).
@@ -161,30 +161,31 @@ bool step_observe_wide_fusable(const EnvView &v) {
 }
 
 cudaError_t launch_step_observe_wide(const EnvView &v, const int8_t *actions, const MapfStepOut &out, float *obs, float *vec,
-                                     int *work_counter, cudaStream_t stream, int out_bf16) {
+                                     int *work_counter, cudaStream_t stream, int fmt) {
     // Default: 4-warp CTAs when six of them fit an SM (measured on 80x80x128, ms per step for FOV 9 / 15 / 21 / 31:
     // two launches 0.861 / 0.971 / 0.950 / 1.032; 8 warps x 3: 1.033 / 1.018 / 0.887 / 1.027; 4 warps x 6: 0.701 / 0.898 /
     // 0.870 / 1.077 — at FOV 31 the per-warp observation scratch leaves three 4-warp CTAs, too few warps for the stores).
     int variant = (v.dbg_flags >> 24) & 7;                  // experiments: 1 = 8w x 3, 2 = 4w x 6, 3 = 4w x 8, 4 = 2w x 16
     if (variant == 0) {
-        const WidePlan p4 = make_plan(v, out_bf16, 4);
+        const WidePlan p4 = make_plan(v, fmt, 4);
         // ... and eight of them (compiled for 64 registers) when eight fit: mid-size worlds (33..100 agents) have a short
         // store phase per world, so they need even more worlds in flight (40x40x64: 0.771 vs 0.806 ms; 80x80x64: 0.384 vs 0.406)
         variant = !(p4.ok && p4.smem <= 40 * 1024) ? 1 : (p4.smem <= 28 * 1024 ? 3 : 2);
         // ... and up to 64 agents, 2-warp CTAs x 16: 33..64-agent worlds have the shortest store phase of all (64-124 KB) against
         // the same ~20 us step phase (40x40x33: 0.927 vs 1.139 ms; 40x40x48: 0.574 vs 0.680; 24x24x40: 0.609 vs 0.750)
         if (v.N <= 64) {
-            const WidePlan p2 = make_plan(v, out_bf16, 2);
+            const WidePlan p2 = make_plan(v, fmt, 2);
             if (p2.ok && p2.smem <= 24 * 1024) variant = 4;
         }
     }
     const int warps = variant == 1 ? 8 : (variant == 4 ? 2 : 4);
-    WidePlan p = make_plan(v, out_bf16, warps);
-    if (!p.ok && warps != 8) { variant = 1; p = make_plan(v, out_bf16, 8); }
+    WidePlan p = make_plan(v, fmt, warps);
+    if (!p.ok && warps != 8) { variant = 1; p = make_plan(v, fmt, 8); }
     if (!p.ok) return cudaErrorNotSupported;
     const int PB = v.C * v.F * v.F;
-    const size_t al = out_bf16 ? 8 : 4;
-    const bool vec4 = ((size_t)p.L.CH * PB) % al == 0 && ((size_t)v.N * PB) % al == 0 && (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
+    const size_t al = fmt == OBS_BF16 ? 8 : 4;
+    const bool vec4 = (fmt == OBS_BITS ? bits_words(p.L.PB) % 4 == 0 : ((size_t)p.L.CH * PB) % al == 0 && ((size_t)v.N * PB) % al == 0) &&
+                      (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
     int dev = 0, sms = 148, per_sm = 1;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -207,8 +208,13 @@ cudaError_t launch_step_observe_wide(const EnvView &v, const int8_t *actions, co
         else if (variant == 4) LAUNCH(2, 16, __VA_ARGS__);                                                         \
         else LAUNCH(4, 8, __VA_ARGS__);                                                                            \
     } while (0)
-    if (v.C == 6 && v.F == 9) { if (vec4) LAUNCH_V(6, 9, true); else LAUNCH_V(6, 9, false); }
-    else { if (vec4) LAUNCH_V(0, 0, true); else LAUNCH_V(0, 0, false); }
+    if (fmt == OBS_BITS) {
+        if (v.C == 6 && v.F == 9) { if (vec4) LAUNCH_V(6, 9, true, true); else LAUNCH_V(6, 9, false, true); }
+        else { if (vec4) LAUNCH_V(0, 0, true, true); else LAUNCH_V(0, 0, false, true); }
+    } else {
+        if (v.C == 6 && v.F == 9) { if (vec4) LAUNCH_V(6, 9, true, false); else LAUNCH_V(6, 9, false, false); }
+        else { if (vec4) LAUNCH_V(0, 0, true, false); else LAUNCH_V(0, 0, false, false); }
+    }
 #undef LAUNCH_V
 #undef LAUNCH
     return cudaGetLastError();

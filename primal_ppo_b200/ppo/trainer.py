@@ -110,7 +110,7 @@ class PPOLearner:
 
 @dataclass
 class RolloutBuffer:
-    obs: torch.Tensor            # f32 [T+1, W, N, C, F, F]
+    obs: torch.Tensor            # f32 [T+1, W, N, C, F, F] (or bf16; or bit-packed int32 [T+1, W, N, AW])
     vec: torch.Tensor            # f32 [T+1, W, N, 4]
     actions: torch.Tensor        # i8  [T, W, N]
     ps: torch.Tensor             # f32 [T, W, N, 5]
@@ -126,15 +126,23 @@ class RolloutBuffer:
     fixed_actions: torch.Tensor  # i8  [T, W, N]
     returns: Optional[torch.Tensor] = None
     cost_returns: Optional[torch.Tensor] = None
+    obs_cf: tuple = (0, 0)                        # (C, F) of the observations (what bit-packed rows expand to)
+    unpack_dtype: torch.dtype = torch.float32     # dtype bit-packed observations expand to (f32, or bf16 under bf16 autocast)
 
     @staticmethod
-    def allocate(T, W, N, C, F, device, obs_dtype=torch.float32):
+    def allocate(T, W, N, C, F, device, obs_dtype=torch.float32, unpack_dtype=torch.float32):
+        """obs_dtype: torch.float32 (the reference's layout), torch.bfloat16, or "bits" (one bit per cell: int32
+        [T+1, W, N, AW], 64 B per agent at 6 x 9 x 9 instead of 1944 B; expanded to `unpack_dtype` when read)."""
+        from .._cabi import obs_bits_words
         z = lambda *s, dt=torch.float32: torch.empty(s, dtype=dt, device=device)
-        return RolloutBuffer(obs=z(T + 1, W, N, C, F, F, dt=obs_dtype), vec=z(T + 1, W, N, 4), actions=z(T, W, N, dt=torch.int8),
+        obs = (z(T + 1, W, N, obs_bits_words(C, F), dt=torch.int32) if obs_dtype == "bits"
+               else z(T + 1, W, N, C, F, F, dt=obs_dtype))
+        return RolloutBuffer(obs=obs, vec=z(T + 1, W, N, 4), actions=z(T, W, N, dt=torch.int8),
                              ps=z(T, W, N, 5), values=z(T, W, N), cost_values=z(T, W, N), rewards=z(T, W, N),
                              cost_rewards=z(T, W, N), train_valid=z(T, W, N, 5), status=z(T, W, N, dt=torch.int8),
                              goals_reached=z(T, W, N, dt=torch.uint8), violated=z(T, W, N, dt=torch.uint8),
-                             shadow_goals=z(T, W, dt=torch.int32), fixed_actions=z(T, W, N, dt=torch.int8))
+                             shadow_goals=z(T, W, dt=torch.int32), fixed_actions=z(T, W, N, dt=torch.int8),
+                             obs_cf=(C, F), unpack_dtype=unpack_dtype)
 
     def minibatch(self, rows: torch.Tensor) -> Dict[str, torch.Tensor]:
         """rows: flat indices into the [T*W] (time, world) rows; a row carries all N agents of one world."""
@@ -142,7 +150,13 @@ class RolloutBuffer:
 
         def g(x):
             return x[:T].reshape(T * W, *x.shape[2:]).index_select(0, rows)
-        return dict(obs=g(self.obs), vec=g(self.vec), actions=g(self.actions), ps=g(self.ps), values=g(self.values),
+        if self.obs.dtype == torch.int32:        # bit-packed: gather and expand in one kernel pass
+            from ..vec_env import unpack_observations
+            obs = unpack_observations(self.obs[:T].reshape(T * W, *self.obs.shape[2:]), *self.obs_cf, rows=rows,
+                                      dtype=self.unpack_dtype)
+        else:
+            obs = g(self.obs)
+        return dict(obs=obs, vec=g(self.vec), actions=g(self.actions), ps=g(self.ps), values=g(self.values),
                     cost_values=g(self.cost_values), returns=g(self.returns), cost_returns=g(self.cost_returns),
                     train_valid=g(self.train_valid))
 
@@ -159,7 +173,9 @@ class VecPPOTrainer:
         """fresh_worlds: callable(rollout_index) -> scenario with the env's shapes; when given, every rollout starts on
         new worlds, as the reference does (`env = MapfGym()` in `Runner.run`, runner.py:30).
         obs_dtype=torch.bfloat16 stores the rollout's observations in the env's optional bf16 format (same values, half
-        the memory and half the env's store traffic); it needs amp_dtype=torch.bfloat16."""
+        the memory and half the env's store traffic); it needs amp_dtype=torch.bfloat16.
+        obs_dtype="bits" stores them bit-packed (one bit per cell, 1/30 of the f32 memory); each forward chunk and each
+        minibatch is expanded by one kernel pass into bf16 when amp_dtype is torch.bfloat16, f32 otherwise."""
         if obs_dtype == torch.bfloat16 and amp_dtype != torch.bfloat16:
             raise ValueError("bf16 observations need amp_dtype=torch.bfloat16 (the fp32 convolution would reject them)")
         self.env, self.policy, self.cfg, self.group = env, policy, cfg, group
@@ -170,7 +186,9 @@ class VecPPOTrainer:
         self.chunk = forward_chunk_rows
         self.seed, self.sample_calls = seed, 0
         self.fresh_worlds, self.rollouts = fresh_worlds, 0
-        self.buf = RolloutBuffer.allocate(self.T, env.W, env.N, env.C, env.F, env.device, obs_dtype)
+        self.unpack_dtype = torch.bfloat16 if amp_dtype == torch.bfloat16 else torch.float32
+        self.buf = RolloutBuffer.allocate(self.T, env.W, env.N, env.C, env.F, env.device, obs_dtype, self.unpack_dtype)
+        self._obs_scratch = None         # expanded observations of one forward chunk (bit-packed rollouts only)
         self.gen = torch.Generator(device=env.device); self.gen.manual_seed(seed)
         env.getAllObservations(out=(self.buf.obs[0], self.buf.vec[0]))
 
@@ -178,10 +196,17 @@ class VecPPOTrainer:
     def _forward(self, obs, vec, ps, values, cost_values):
         W, N = obs.shape[:2]
         step = max(1, self.chunk // N)
+        if obs.dtype == torch.int32 and self._obs_scratch is None:
+            C, F = self.buf.obs_cf
+            self._obs_scratch = torch.empty((min(W, step), N, C, F, F), dtype=self.unpack_dtype, device=obs.device)
         for lo in range(0, W, step):
             hi = min(W, lo + step)
+            x = obs[lo:hi]
+            if obs.dtype == torch.int32:
+                from ..vec_env import unpack_observations
+                x = unpack_observations(x, *self.buf.obs_cf, dtype=self.unpack_dtype, out=self._obs_scratch[:hi - lo])
             with torch.autocast(obs.device.type, dtype=self.amp_dtype, enabled=self.amp_dtype is not None):
-                o = self.policy(obs[lo:hi], vec[lo:hi])
+                o = self.policy(x, vec[lo:hi])
             if ps is not None:
                 ps[lo:hi] = o.policy.float()
             values[lo:hi] = o.value.float().squeeze(-1)

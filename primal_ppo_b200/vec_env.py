@@ -10,6 +10,8 @@ Reference call                                     | batched call
 ---------------------------------------------------|---------------------------------------------------------
 ``env = FixedMapfGym(obst, seqs, hStart, hGoal)``  | ``env = BatchedMapfGym(scenario)``  (``scenario.py``)
 ``obs, vec = env.getAllObservations()``            | same -> f32 [W,N,C,F,F], f32 [W,N,4]
+(bit-packed observations, not in the reference)    | ``getAllObservations(out=(bits, vec))`` with int32 ``env.obs_bits_shape``;
+                                                   | ``unpack_observations(bits, C, F)`` -> f32 / bf16 [W,N,C,F,F]
 ``st = env.getActionStatus(a)``                    | same -> int8 [W,N]
 ``r, sg = env.calculateActionReward(a, st)``       | same -> f32 [W,N], int32 [W]
 ``c = env.calculateCostReward(a)``                 | same -> f32 [W,N]
@@ -263,7 +265,8 @@ class BatchedMapfGym:
         o = self._out if out is None else out
         obs, vec = self._obs_buffers(obs_out)
         so = self._step_out(o)
-        fn = self._lib.mapf_step_observe_bf16 if obs.dtype == torch.bfloat16 else self._lib.mapf_step_observe
+        fn = {torch.bfloat16: self._lib.mapf_step_observe_bf16, torch.int32: self._lib.mapf_step_observe_bits}.get(
+            obs.dtype, self._lib.mapf_step_observe)
         _cabi.check(fn(self._h, _ptr(a), C.byref(so), _ptr(obs), _ptr(vec), self._stream()), "mapf_step_observe")
         self._eval_key = None
         return o, obs, vec
@@ -277,15 +280,28 @@ class BatchedMapfGym:
             return self._obs, self._vec
         obs, vec = out
         assert obs.is_contiguous() and vec.is_contiguous() and vec.dtype == torch.float32
-        assert obs.dtype in (torch.float32, torch.bfloat16), "observations are f32 (reference layout) or, optionally, bf16"
-        assert obs.numel() == self.W * self.N * self.C * self.F * self.F and vec.numel() == self.W * self.N * 4
+        assert obs.dtype in (torch.float32, torch.bfloat16, torch.int32), \
+            "observations are f32 (reference layout) or, optionally, bf16 or bit-packed int32 (obs_bits_shape)"
+        if obs.dtype == torch.int32:
+            assert tuple(obs.shape) == self.obs_bits_shape, f"bit-packed observations need shape {self.obs_bits_shape}"
+        else:
+            assert obs.numel() == self.W * self.N * self.C * self.F * self.F
+        assert vec.numel() == self.W * self.N * 4
         return obs, vec
+
+    @property
+    def obs_bits_shape(self):
+        """Shape of the bit-packed observations (int32 [W, N, AW], AW = ``MAPF_OBS_BITS_WORDS(C, F)``): bit k of agent
+        (w, i) is ``obs[w, i].flatten()[k]``, in word k // 32 at bit k % 32; ``unpack_observations`` expands them."""
+        return (self.W, self.N, _cabi.obs_bits_words(self.C, self.F))
 
     def getAllObservations(self, out=None):
         """``getAllObservations`` (mapf_gym.py:327-336).  ``out=(obs, vec)`` writes straight into the policy's input
-        tensors; otherwise env-owned tensors are (re)used."""
+        tensors; otherwise env-owned tensors are (re)used.  ``obs`` selects the format by dtype: f32, bf16, or int32 of
+        ``obs_bits_shape`` (one bit per cell)."""
         obs, vec = self._obs_buffers(out)
-        fn = self._lib.mapf_observe_bf16 if obs.dtype == torch.bfloat16 else self._lib.mapf_observe
+        fn = {torch.bfloat16: self._lib.mapf_observe_bf16, torch.int32: self._lib.mapf_observe_bits}.get(
+            obs.dtype, self._lib.mapf_observe)
         _cabi.check(fn(self._h, _ptr(obs), _ptr(vec), self._stream()), "mapf_observe")
         return obs, vec
 
@@ -536,6 +552,41 @@ def checksum_rows(t: torch.Tensor) -> torch.Tensor:
     stream = C.c_void_p(torch.cuda.current_stream(t.device).cuda_stream)
     with torch.cuda.device(t.device):
         _cabi.check(lib.mapf_checksum_rows(_ptr(t), rows, row_bytes, _ptr(out), stream), "mapf_checksum_rows")
+    return out
+
+
+def _stream_ptr(device):
+    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
+def unpack_observations(bits: torch.Tensor, C: int, F: int, rows: Optional[torch.Tensor] = None,
+                        dtype=torch.float32, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Expand bit-packed observations (``mapf_unpack_obs``) into the network's 0/1 values in ONE kernel pass.
+
+    bits: int32 [..., N, AW] on the GPU (AW = ``MAPF_OBS_BITS_WORDS(C, F)``); its leading dimensions are the source rows.
+    rows: optional int64 index into the source rows (a minibatch gather): the result is [len(rows), N, C, F, F], and an
+    index outside [0, rows) gives an all-zero row.  Without it the result is bits.shape[:-1] + (C, F, F).
+    dtype: torch.float32 or torch.bfloat16.  out: a contiguous tensor of that shape and dtype to write into."""
+    lib = _cabi.load_library()
+    assert bits.is_cuda and bits.dtype == torch.int32 and bits.is_contiguous() and bits.dim() >= 2
+    assert dtype in (torch.float32, torch.bfloat16), "observations expand to f32 or bf16"
+    N, AW = int(bits.shape[-2]), int(bits.shape[-1])
+    assert AW == _cabi.obs_bits_words(C, F), f"last dimension {AW} is not MAPF_OBS_BITS_WORDS({C}, {F})"
+    src_rows = bits.numel() // max(N * AW, 1)
+    if rows is None:
+        n_rows, shape, idx = src_rows, tuple(bits.shape[:-1]) + (C, F, F), None
+    else:
+        idx = rows.to(device=bits.device, dtype=torch.int64).contiguous()
+        n_rows, shape = int(idx.numel()), (int(idx.numel()), N, C, F, F)
+    if out is None:
+        out = torch.empty(shape, dtype=dtype, device=bits.device)
+    assert out.is_contiguous() and out.dtype == dtype and tuple(out.shape) == shape and out.device == bits.device
+    if n_rows == 0:
+        return out
+    stream = _stream_ptr(bits.device)            # (`C` is the channel count here, not the ctypes module)
+    with torch.cuda.device(bits.device):
+        _cabi.check(lib.mapf_unpack_obs(_ptr(bits), src_rows, N, int(C), int(F), _ptr(idx), n_rows,
+                                        int(dtype == torch.bfloat16), _ptr(out), stream), "mapf_unpack_obs")
     return out
 
 

@@ -11,8 +11,26 @@ other = os.path.abspath(sys.argv[1])
 W, N = 65536, 32
 sc = random_scenario(W, 40, 40, N, density=(0.0, 0.3), queue_len=16, seed=100, unique_maps=256)
 envs = {"new": BatchedMapfGym(sc, use_tape=False)}
+import ctypes
+
+
+class _OlderBuild(ctypes.CDLL):
+    """A build from before some entry points existed: the binding's missing names become inert stubs (never called here)."""
+    def __getattr__(self, name):
+        try:
+            return super().__getattr__(name)
+        except AttributeError:
+            if name.startswith("__"):
+                raise
+            stub = type("MissingEntryPoint", (), {})()
+            setattr(self, name, stub)
+            return stub
+
+
 cabi._lib = None; cabi.LIB_PATH = other
+_cdll, ctypes.CDLL = ctypes.CDLL, _OlderBuild
 envs["base"] = BatchedMapfGym(sc, use_tape=False)
+ctypes.CDLL = _cdll
 dev = envs["new"].device
 obs = torch.empty((W, N, 6, 9, 9), device=dev); vec = torch.empty((W, N, 4), device=dev)
 gen = torch.Generator(device=dev); gen.manual_seed(1)
