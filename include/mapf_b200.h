@@ -295,15 +295,33 @@ int mapf_step_observe_host(MapfEnv *env, const int8_t *actions_host, const MapfS
  *                          path: at 65 536 x 32 agents the full slab is 25 MB per step and GPU, the compact one 4.5 MB.
  *   | MAPF_HOST_TRAIN_VALID: train_valid f32[W,N,5] appended (needs train_valid_dev; the caller's tensor is the copy
  *                          source, so the next begin waits for this step's copy).
+ *   | MAPF_HOST_OBS:        the step's observations and vec appended, for a runner whose policy reads them on the host
+ *                          (the reference's getAllObservations, runner.py:31,100).  The observation block starts at
+ *                          off_obs = slot_bytes of the same flags without MAPF_HOST_OBS and holds obs_dev as written:
+ *                          W*N*C*F*F*4 (f32), W*N*C*F*F*2 (bf16) or W*N*MAPF_OBS_BITS_WORDS(C,F)*4 (bits) bytes, rounded up
+ *                          to 256; vec f32[W,N,4] (W*N*16 bytes) follows it.  mapf_host_layout reports the total slot_bytes.
+ *                          Both are copied from the caller's obs_dev / vec_dev, so a later begin whose outputs (obs_dev,
+ *                          vec_dev, train_valid_dev) overlap them waits for this step's copy; one that writes into other
+ *                          buffers (a rollout buffer's step t+1) does not.  Only later begins are ordered behind the
+ *                          copy: any other writer to those buffers must first wait for that step (mapf_step_observe_host_wait).
+ *                          A bit-packed slot is expanded on the host by
+ *                          mapf_unpack_obs_host.
+ * Observation format of obs_dev (orthogonal to the wire format; at most one of the two):
+ *   default f32 [W,N,C,F,F] (mapf_step_observe); MAPF_HOST_OBS_BF16: bf16 [W,N,C,F,F] (mapf_step_observe_bf16);
+ *   MAPF_HOST_OBS_BITS: u32 [W,N,MAPF_OBS_BITS_WORDS(C,F)] (mapf_step_observe_bits, obs_dev 4-byte aligned).  Setting both
+ *   is MAPF_E_BAD_CONFIG.
  * mapf_step_observe_host_begin: actions_host -> device (own copy stream, double-buffered), ONE fused step+observe launch
  * on `stream` writing obs_dev / vec_dev (and train_valid_dev if given) and the env's device slot, then ONE device-to-host
- * copy of the slot into result_slot_host on the copy stream.  Returns without any host synchronisation: work queued on
+ * copy of the slot into result_slot_host on the copy stream (plus the train_valid / observation copies the flags ask for).  Returns without any host synchronisation: work queued on
  * `stream` afterwards (the policy forward) sees obs_dev / vec_dev of this step.  The env keeps two device slots, so two
  * begins may be in flight; result_slot_host must stay untouched until the matching wait.
  * mapf_step_observe_host_wait(env, age): block the host until the results of the most recent begin (age 0) or of the one
- * before it (age 1) have landed in their result_slot_host. */
+ * before it (age 1) have landed in their result_slot_host, the MAPF_HOST_TRAIN_VALID / MAPF_HOST_OBS copies included. */
 #define MAPF_HOST_TRAIN_VALID 1
 #define MAPF_HOST_COMPACT 2
+#define MAPF_HOST_OBS_BF16 4
+#define MAPF_HOST_OBS_BITS 8
+#define MAPF_HOST_OBS 16
 typedef struct MapfHostLayout {
     int64_t slot_bytes; /* bytes of one result slot for the flags passed to mapf_host_layout */
     int64_t off_reward, off_cost, off_shadow_goals, off_status, off_goals_reached, off_violated, off_fixed_actions,
@@ -311,13 +329,20 @@ typedef struct MapfHostLayout {
 } MapfHostLayout;
 int mapf_host_layout(MapfEnv *env, int flags, MapfHostLayout *out);
 int mapf_step_observe_host_begin(MapfEnv *env, const int8_t *actions_host, void *result_slot_host, int flags,
-                                 float *obs_dev, float *vec_dev, float *train_valid_dev, void *stream);
+                                 void *obs_dev, float *vec_dev, float *train_valid_dev, void *stream);
 int mapf_step_observe_host_wait(MapfEnv *env, int age);
 
 /* HOST function (no GPU work): expand n packed results (MapfStepOut.packed / a compact slot's `packed` field) into the
  * reference's per-agent arrays; any pointer of `out` may be NULL; out->train_valid / shadow_goals / good_actions are not
  * touched.  Bit-identical to the arrays the full format carries. */
 int mapf_decode_results_host(const uint16_t *packed, int64_t n, const MapfStepOutHost *out);
+
+/* HOST function (no GPU work): mapf_unpack_obs on host memory, for a CPU-side consumer of bit-packed observations (the
+ * observation block of a MAPF_HOST_OBS | MAPF_HOST_OBS_BITS slot).  Same arguments, checks, bit order and results: out[r]
+ * = the f32 / bf16 0/1 values [agents, C, F, F] of source row rows[r] (rows NULL: row r); a row index outside
+ * [0, src_rows) gives an all-zero row. */
+int mapf_unpack_obs_host(const uint32_t *obs_bits, int64_t src_rows, int32_t agents, int32_t num_channel, int32_t fov,
+                         const int64_t *rows /* NULL = rows 0..n_rows-1 */, int64_t n_rows, int32_t out_bf16, void *out);
 
 /* ---- learner-side glue: the elementwise part of the PPO-Lagrangian minibatch loss (SURVEY 8 f3) ----------------------- */
 

@@ -16,7 +16,7 @@ EXPORTED = ["mapf_abi_version", "mapf_last_error", "mapf_create", "mapf_destroy"
             "mapf_sample_actions", "mapf_generate_scenario",
             "mapf_observe_bf16", "mapf_step_observe_bf16", "mapf_state_bytes", "mapf_save_state", "mapf_load_state",
             "mapf_get_human", "mapf_host_layout", "mapf_step_observe_host_begin", "mapf_step_observe_host_wait", "mapf_decode_results_host", "mapf_checksum_rows", "mapf_adv_moments", "mapf_ppo_loss",
-            "mapf_observe_bits", "mapf_step_observe_bits", "mapf_unpack_obs"]
+            "mapf_observe_bits", "mapf_step_observe_bits", "mapf_unpack_obs", "mapf_unpack_obs_host"]
 ABI_VERSION = 2
 
 def obs_bits_words(C: int, F: int) -> int:
@@ -62,7 +62,7 @@ class MapfHostLayout(C.Structure):
                  "off_violated", "off_fixed_actions", "off_train_valid", "off_packed")]
 
 
-HOST_TRAIN_VALID, HOST_COMPACT = 1, 2
+HOST_TRAIN_VALID, HOST_COMPACT, HOST_OBS_BF16, HOST_OBS_BITS, HOST_OBS = 1, 2, 4, 8, 16
 
 
 class MapfPpoLossConfig(C.Structure):
@@ -107,6 +107,7 @@ def load_library():
     lib.mapf_observe_bits.argtypes = [vp, vp, vp, vp]
     lib.mapf_step_observe_bits.argtypes = [vp, vp, C.POINTER(MapfStepOut), vp, vp, vp]
     lib.mapf_unpack_obs.argtypes = [vp, i64, i32, i32, i32, vp, i64, i32, vp, vp]
+    lib.mapf_unpack_obs_host.argtypes = [vp, i64, i32, i32, i32, vp, i64, i32, vp]
     lib.mapf_bfs.argtypes = [vp, vp, i64, vp, vp]
     lib.mapf_bfs_refresh.argtypes = [vp, vp, vp, vp]
     lib.mapf_gae.argtypes = [vp, vp, vp, vp, C.c_double, C.c_double, i32, i64, vp, vp, vp]

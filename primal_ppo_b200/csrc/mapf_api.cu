@@ -30,7 +30,10 @@ struct MapfEnv {
     cudaStream_t copy_stream, h2d_stream;
     cudaEvent_t ev_step[2], ev_copied[2], ev_h2d[2];
     bool tv_copy_pending[2];                 // that begin also copied the caller's trainValid tensor
-    int next_slot;                           // slot the next begin uses; the most recent begin used next_slot ^ 1
+    // device ranges [begin, end) of the caller's obs_dev / vec_dev that a MAPF_HOST_OBS begin of slot k copies to the host
+    // (empty when it copied none); a later begin whose outputs overlap one of them waits for that copy
+    uintptr_t obs_src[2][2], vec_src[2][2];
+    int next_slot;                          // slot the next begin uses; the most recent begin used next_slot ^ 1
     int begun;                               // number of begins so far (saturating at 2)
 };
 
@@ -582,30 +585,66 @@ int queue_actions(MapfEnv *e, int k, const int8_t *actions_host, cudaStream_t s)
     return MAPF_OK;
 }
 
+// The observation format obs_dev is written in, from the flags of the split-phase call; -1 when both format flags are set.
+int host_obs_format(int flags) {
+    const bool bf16 = flags & MAPF_HOST_OBS_BF16, bits = flags & MAPF_HOST_OBS_BITS;
+    if (bf16 && bits) return -1;
+    return bits ? OBS_BITS : bf16 ? OBS_BF16 : OBS_F32;
+}
+
+size_t obs_bytes(const EnvView &v, int fmt) {
+    const size_t WN = (size_t)v.W * v.N, PB = (size_t)v.C * v.F * v.F;
+    return fmt == OBS_BITS ? WN * MAPF_OBS_BITS_WORDS(v.C, v.F) * 4 : WN * PB * (fmt == OBS_BF16 ? 2 : 4);
+}
+
+bool overlaps(uintptr_t lo, uintptr_t hi, const uintptr_t r[2]) { return lo < r[1] && r[0] < hi; }
+
 }  // namespace
 
 int mapf_host_layout(MapfEnv *e, int flags, MapfHostLayout *out) {
     if (!e || !out) return fail(MAPF_E_NULL, "mapf_host_layout: null argument");
+    const int fmt = host_obs_format(flags);
+    if (fmt < 0) return fail(MAPF_E_BAD_CONFIG, "mapf_host_layout: MAPF_HOST_OBS_BF16 and MAPF_HOST_OBS_BITS are exclusive");
+    auto up = [](size_t x) { return (int64_t)((x + 255) & ~(size_t)255); };
     *out = (flags & MAPF_HOST_COMPACT) ? e->lay_c : e->lay;
     if (flags & MAPF_HOST_TRAIN_VALID) {
         out->off_train_valid = out->slot_bytes;
-        out->slot_bytes += (int64_t)((((size_t)e->v.W * e->v.N * NA * 4) + 255) & ~(size_t)255);
+        out->slot_bytes += up((size_t)e->v.W * e->v.N * NA * 4);
     }
+    if (flags & MAPF_HOST_OBS) out->slot_bytes += up(obs_bytes(e->v, fmt)) + up((size_t)e->v.W * e->v.N * 16);
     return MAPF_OK;
 }
 
 int mapf_step_observe_host_begin(MapfEnv *e, const int8_t *actions_host, void *result_slot_host, int flags,
-                                 float *obs_dev, float *vec_dev, float *train_valid_dev, void *stream) {
+                                 void *obs_dev, float *vec_dev, float *train_valid_dev, void *stream) {
     NEED_ENV("mapf_step_observe_host_begin");
     if (int rc = check_vec(vec_dev, "mapf_step_observe_host_begin")) return rc;
     if (!actions_host || !result_slot_host || !obs_dev || !vec_dev) return fail(MAPF_E_NULL, "mapf_step_observe_host_begin: null argument");
-    const bool with_tv = flags & MAPF_HOST_TRAIN_VALID, compact = flags & MAPF_HOST_COMPACT;
+    const bool with_tv = flags & MAPF_HOST_TRAIN_VALID, compact = flags & MAPF_HOST_COMPACT, with_obs = flags & MAPF_HOST_OBS;
     if (with_tv && !train_valid_dev) return fail(MAPF_E_NULL, "mapf_step_observe_host_begin: MAPF_HOST_TRAIN_VALID needs train_valid_dev");
+    const int fmt = host_obs_format(flags);
+    if (fmt < 0)
+        return fail(MAPF_E_BAD_CONFIG, "mapf_step_observe_host_begin: MAPF_HOST_OBS_BF16 and MAPF_HOST_OBS_BITS are exclusive");
+    if (fmt == OBS_BITS)
+        if (int rc = check_bits(static_cast<const uint32_t *>(obs_dev), "mapf_step_observe_host_begin")) return rc;
     if (int rc = check_step_n(e, "mapf_step_observe_host_begin")) return rc;
     const EnvView &v = e->v;
+    const size_t WN = (size_t)v.W * v.N, n_obs = obs_bytes(v, fmt);
     cudaStream_t s = (cudaStream_t)stream, cs = e->copy_stream;
     const int k = e->next_slot;
     if (int rc = queue_actions(e, k, actions_host, s)) return rc;
+    // The observation copies of the previous begin read the caller's obs_dev / vec_dev while this step runs.  Only a step
+    // that writes into one of those ranges waits for them (the copies of the begin before that were awaited by
+    // queue_actions): a rollout that gives every step its own buffers keeps two steps overlapped.
+    if (e->begun >= 1) {
+        const uintptr_t ob = reinterpret_cast<uintptr_t>(obs_dev), vc = reinterpret_cast<uintptr_t>(vec_dev),
+                        tv = reinterpret_cast<uintptr_t>(train_valid_dev);
+        const uintptr_t *po = e->obs_src[k ^ 1], *pv = e->vec_src[k ^ 1];
+        bool hit = overlaps(ob, ob + n_obs, po) || overlaps(ob, ob + n_obs, pv) || overlaps(vc, vc + WN * 16, po) ||
+                   overlaps(vc, vc + WN * 16, pv);
+        if (train_valid_dev) hit = hit || overlaps(tv, tv + WN * NA * 4, po) || overlaps(tv, tv + WN * NA * 4, pv);
+        if (hit) CU(cudaStreamWaitEvent(s, e->ev_copied[k ^ 1], 0));
+    }
     MapfStepOut o;
     size_t slot_bytes;
     if (compact) {
@@ -618,15 +657,23 @@ int mapf_step_observe_host_begin(MapfEnv *e, const int8_t *actions_host, void *r
         slot_bytes = (size_t)e->lay.slot_bytes;
     }
     o.train_valid = train_valid_dev;
-    CU(do_step_observe(e, e->d_actions[k], o, obs_dev, vec_dev, s, OBS_F32));
+    CU(do_step_observe(e, e->d_actions[k], o, static_cast<float *>(obs_dev), vec_dev, s, fmt));
     CU(cudaEventRecord(e->ev_step[k], s));
     CU(cudaStreamWaitEvent(cs, e->ev_step[k], 0));
-    CU(cudaMemcpyAsync(result_slot_host, e->d_slot[k], slot_bytes, cudaMemcpyDeviceToHost, cs));   // ONE copy
-    if (with_tv)
-        CU(cudaMemcpyAsync(static_cast<char *>(result_slot_host) + slot_bytes, train_valid_dev,
-                           (size_t)v.W * v.N * NA * 4, cudaMemcpyDeviceToHost, cs));
+    char *const host = static_cast<char *>(result_slot_host);
+    CU(cudaMemcpyAsync(host, e->d_slot[k], slot_bytes, cudaMemcpyDeviceToHost, cs));   // ONE copy
+    const size_t up_tv = (WN * NA * 4 + 255) & ~(size_t)255;
+    if (with_tv) CU(cudaMemcpyAsync(host + slot_bytes, train_valid_dev, WN * NA * 4, cudaMemcpyDeviceToHost, cs));
+    const uintptr_t ob = reinterpret_cast<uintptr_t>(obs_dev), vc = reinterpret_cast<uintptr_t>(vec_dev);
+    if (with_obs) {
+        const size_t off_obs = slot_bytes + (with_tv ? up_tv : 0), off_vec = off_obs + ((n_obs + 255) & ~(size_t)255);
+        CU(cudaMemcpyAsync(host + off_obs, obs_dev, n_obs, cudaMemcpyDeviceToHost, cs));
+        CU(cudaMemcpyAsync(host + off_vec, vec_dev, WN * 16, cudaMemcpyDeviceToHost, cs));
+    }
     CU(cudaEventRecord(e->ev_copied[k], cs));
     e->tv_copy_pending[k] = with_tv;
+    e->obs_src[k][0] = with_obs ? ob : 0; e->obs_src[k][1] = with_obs ? ob + n_obs : 0;
+    e->vec_src[k][0] = with_obs ? vc : 0; e->vec_src[k][1] = with_obs ? vc + WN * 16 : 0;
     e->next_slot = k ^ 1;
     if (e->begun < 2) e->begun++;
     return MAPF_OK;
@@ -648,6 +695,43 @@ int mapf_decode_results_host(const uint16_t *packed, int64_t n, const MapfStepOu
         if (out->goals_reached) out->goals_reached[i] = (uint8_t)((p >> 3) & 1u);
         if (out->violated) out->violated[i] = (uint8_t)((p >> 4) & 1u);
         if (out->fixed_actions) out->fixed_actions[i] = (int8_t)((p >> 5) & 7u);
+    }
+    return MAPF_OK;
+}
+
+int mapf_unpack_obs_host(const uint32_t *obs_bits, int64_t src_rows, int32_t agents, int32_t num_channel, int32_t fov,
+                         const int64_t *rows, int64_t n_rows, int32_t out_bf16, void *out) {
+    if (!obs_bits || !out) return fail(MAPF_E_NULL, "mapf_unpack_obs_host: null argument");
+    if (src_rows < 0 || n_rows < 0) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: negative row count");
+    if (agents < 1 || agents > 254) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: agents must be in 1..254");
+    if (num_channel != 5 && num_channel != 6) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: num_channel must be 5 or 6");
+    if (fov < 3 || fov > 31 || (fov & 1) == 0) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: fov must be odd in 3..31");
+    if (out_bf16 != 0 && out_bf16 != 1) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: out_bf16 must be 0 or 1");
+    if (int rc = check_bits(obs_bits, "mapf_unpack_obs_host")) return rc;
+    if (reinterpret_cast<uintptr_t>(out) & (out_bf16 ? 1 : 3))
+        return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: out must be aligned to its element size");
+    // byte -> its eight 0/1 values, LSB first: one table lookup and copy per 8 cells
+    static const struct Lut {
+        float f[256][8];
+        uint16_t h[256][8];
+        Lut() {
+            for (int b = 0; b < 256; ++b)
+                for (int i = 0; i < 8; ++i) { f[b][i] = (b >> i) & 1 ? 1.0f : 0.0f; h[b][i] = (b >> i) & 1 ? 0x3f80 : 0; }
+        }
+    } lut;
+    const int PB = num_channel * fov * fov, AW = MAPF_OBS_BITS_WORDS(num_channel, fov);
+    const size_t esz = out_bf16 ? 2 : 4, row_out = (size_t)agents * PB * esz;
+    for (int64_t r = 0; r < n_rows; ++r) {
+        const int64_t s = rows ? rows[r] : r;
+        char *dst = static_cast<char *>(out) + (size_t)r * row_out;
+        if (s < 0 || s >= src_rows) { memset(dst, 0, row_out); continue; }
+        const uint32_t *src = obs_bits + (size_t)s * agents * AW;
+        for (int a = 0; a < agents; ++a, src += AW, dst += (size_t)PB * esz)
+            for (int c = 0; c < PB; c += 8) {
+                const unsigned byte = (src[c >> 5] >> (c & 31)) & 0xffu;
+                const int n = PB - c < 8 ? PB - c : 8;
+                memcpy(dst + c * esz, out_bf16 ? (const void *)lut.h[byte] : (const void *)lut.f[byte], n * esz);
+            }
     }
     return MAPF_OK;
 }
@@ -701,6 +785,7 @@ int mapf_step_observe_host(MapfEnv *e, const int8_t *actions_host, const MapfSte
     if (out->fixed_actions) CU(cudaMemcpyAsync(out->fixed_actions, o.fixed_actions, WN, cudaMemcpyDeviceToHost, cs));
     CU(cudaEventRecord(e->ev_copied[k], cs));
     e->tv_copy_pending[k] = false;
+    e->obs_src[k][0] = e->obs_src[k][1] = e->vec_src[k][0] = e->vec_src[k][1] = 0;
     e->next_slot = k ^ 1;
     if (e->begun < 2) e->begun++;
     const size_t PB = (size_t)v.C * v.F * v.F;

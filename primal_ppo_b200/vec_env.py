@@ -424,8 +424,14 @@ class BatchedMapfGym:
 
 
     # ---- split-phase host call: step t's results travel to the host while step t+1 computes -------------------------
-    def host_layout(self, with_train_valid: bool = False, compact: bool = False) -> "_cabi.MapfHostLayout":
-        flags = (_cabi.HOST_TRAIN_VALID if with_train_valid else 0) | (_cabi.HOST_COMPACT if compact else 0)
+    def host_layout(self, with_train_valid: bool = False, compact: bool = False, obs=None) -> "_cabi.MapfHostLayout":
+        """``mapf_host_layout``.  obs (None, torch.float32, torch.bfloat16 or "bits"): the slot also carries the step's
+        observations in that format and vec (MAPF_HOST_OBS), after ``host_layout(with_train_valid, compact).slot_bytes``."""
+        flags = ((_cabi.HOST_TRAIN_VALID if with_train_valid else 0) | (_cabi.HOST_COMPACT if compact else 0)
+                 | _host_obs_flags(obs))
+        return self._host_layout(flags)
+
+    def _host_layout(self, flags: int) -> "_cabi.MapfHostLayout":
         if flags not in self._host_layouts:
             L = _cabi.MapfHostLayout()
             _cabi.check(self._lib.mapf_host_layout(self._h, flags, C.byref(L)), "mapf_host_layout")
@@ -433,14 +439,19 @@ class BatchedMapfGym:
         return self._host_layouts[flags]
 
     def make_host_ring(self, slots: int = 2, action_slots: int = 2, with_train_valid: bool = False, compact: bool = False,
-                       numa_bind: bool = True):
+                       numa_bind: bool = True, obs=None):
         """ONE pinned slab holding `slots` result slots (the layout ``mapf_host_layout`` reports: every per-agent result of
         a step is contiguous, so a step's results come back with one copy) and an int8 [action_slots, W, N] action ring.
         compact=True: the 2-byte-per-agent wire format (``packed`` u16 [W,N] + ``shadow_goals``; ``decode_slot`` expands it
         on the host, bit for bit) instead of the 12-byte-per-agent f32 slab — what keeps eight GPUs of one box off the
         host's PCIe / memory ceiling.  Returns ``{"slots": [dict of views per slot], "action_ring": ..., ...}``.
-        numa_bind: allocate while the calling thread is bound to the CPUs next to this GPU (first touch places the pages)."""
-        L = self.host_layout(with_train_valid, compact)
+        numa_bind: allocate while the calling thread is bound to the CPUs next to this GPU (first touch places the pages).
+        obs (None, torch.float32, torch.bfloat16 or "bits"): every slot also receives the step's observations in that format
+        and vec (MAPF_HOST_OBS), as host views ``obs`` (f32 / bf16 [W,N,C,F,F] or int32 ``obs_bits_shape``) and ``vec``
+        (f32 [W,N,4]); ``step_observe_host_begin`` then needs an ``obs_dev`` of that format.  ``unpack_observations``
+        expands a bit-packed host ``obs``."""
+        L = self.host_layout(with_train_valid, compact, obs)
+        obs_flags = _host_obs_flags(obs)
         W, N = self.W, self.N
         sb = int(L.slot_bytes)
         act_bytes = (max(1, action_slots) * W * N + 255) // 256 * 256
@@ -468,21 +479,50 @@ class BatchedMapfGym:
                          fixed_actions=f(L.off_fixed_actions, W * N, torch.int8, (W, N)))
             if with_train_valid:
                 d["train_valid"] = f(L.off_train_valid, W * N * 20, torch.float32, (W, N, 5))
+            if obs_flags:
+                dt, shape = self._obs_format(obs_flags)
+                off_obs = int(self.host_layout(with_train_valid, compact).slot_bytes)
+                n_obs = int(np.prod(shape)) * torch.empty((), dtype=dt).element_size()
+                d["obs"] = f(off_obs, n_obs, dt, shape)
+                d["vec"] = f(off_obs + (n_obs + 255) // 256 * 256, W * N * 16, torch.float32, (W, N, 4))
             views.append(d)
         ring = slab[slots * sb:slots * sb + max(1, action_slots) * W * N].view(torch.int8).view(max(1, action_slots), W, N)
         return {"slots": views, "action_ring": ring, "_slab": slab, "with_train_valid": bool(with_train_valid),
-                "compact": bool(compact), "slot_bytes": sb,
-                "flags": (_cabi.HOST_TRAIN_VALID if with_train_valid else 0) | (_cabi.HOST_COMPACT if compact else 0)}
+                "compact": bool(compact), "slot_bytes": sb, "obs": obs,
+                "flags": (_cabi.HOST_TRAIN_VALID if with_train_valid else 0) | (_cabi.HOST_COMPACT if compact else 0)
+                | obs_flags}
+
+    def _obs_format(self, flags: int):
+        """(dtype, shape) of observations in the format the MAPF_HOST_OBS_* bits of `flags` select."""
+        if flags & _cabi.HOST_OBS_BITS:
+            return torch.int32, self.obs_bits_shape
+        dt = torch.bfloat16 if flags & _cabi.HOST_OBS_BF16 else torch.float32
+        return dt, (self.W, self.N, self.C, self.F, self.F)
 
     def step_observe_host_begin(self, actions: torch.Tensor, slot: dict, obs_dev: torch.Tensor, vec_dev: torch.Tensor,
                                 train_valid_dev: Optional[torch.Tensor] = None, with_train_valid: bool = False):
         """Queue one env step for a HOST runner and return immediately: `actions` (int8 [W,N] host tensor, ideally a slice of
         the ring's pinned slab) -> device, ONE fused step+observe launch into obs_dev / vec_dev, all per-agent results ->
         `slot` (one of ``make_host_ring()["slots"]``; its format — full or compact — is the ring's) with ONE device-to-host
-        copy.  ``host_wait(age)`` makes a slot readable.  Returns (h2d_bytes, d2h_bytes)."""
+        copy.  ``obs_dev`` selects the observation format by dtype, as in ``step_observe``: f32, bf16, or int32 of
+        ``obs_bits_shape``.  A ring made with ``obs=`` also receives obs_dev / vec_dev in the slot's ``obs`` / ``vec``; obs_dev
+        must then be in the ring's format.  ``host_wait(age)`` makes a slot readable.  Returns (h2d_bytes, d2h_bytes)."""
         assert not actions.is_cuda and actions.dtype == torch.int8 and actions.is_contiguous() and actions.numel() == self.W * self.N
+        obs_dev, vec_dev = self._obs_buffers((obs_dev, vec_dev))
         compact = "packed" in slot
-        flags = (_cabi.HOST_TRAIN_VALID if with_train_valid else 0) | (_cabi.HOST_COMPACT if compact else 0)
+        flags = ((_cabi.HOST_TRAIN_VALID if with_train_valid else 0) | (_cabi.HOST_COMPACT if compact else 0)
+                 | _OBS_FORMAT_FLAG[obs_dev.dtype])
+        # the trainValid block (and after it the observation block) is placed by the flags: they must be the ring's
+        if with_train_valid and "train_valid" not in slot:
+            raise _cabi.MapfError("step_observe_host_begin: with_train_valid=True needs a ring made with with_train_valid=True")
+        if "obs" in slot and not with_train_valid and "train_valid" in slot:
+            raise _cabi.MapfError("step_observe_host_begin: this ring's slots hold train_valid before the observations; "
+                                  "pass with_train_valid=True")
+        if "obs" in slot:
+            if slot["obs"].dtype != obs_dev.dtype:
+                raise _cabi.MapfError(f"step_observe_host_begin: the ring holds {slot['obs'].dtype} observations, "
+                                      f"obs_dev is {obs_dev.dtype}")
+            flags |= _cabi.HOST_OBS
         tvd = train_valid_dev
         if with_train_valid and tvd is None:
             tvd = self._out.train_valid
@@ -490,12 +530,26 @@ class BatchedMapfGym:
                                                            _ptr(obs_dev), _ptr(vec_dev), _ptr(tvd), self._stream()),
                     "mapf_step_observe_host_begin")
         self._eval_key = None
-        return actions.numel(), int(self.host_layout(with_train_valid, compact).slot_bytes)
+        return actions.numel(), int(self._host_layout(flags).slot_bytes)
 
     def host_wait(self, age: int = 0):
         """Block until the results of the most recent ``step_observe_host_begin`` (age 0) or the one before (age 1) are in
         their host slot."""
         _cabi.check(self._lib.mapf_step_observe_host_wait(self._h, int(age)), "mapf_step_observe_host_wait")
+
+
+_OBS_FORMAT_FLAG = {torch.float32: 0, torch.bfloat16: _cabi.HOST_OBS_BF16, torch.int32: _cabi.HOST_OBS_BITS}
+
+
+def _host_obs_flags(obs) -> int:
+    """MAPF_HOST_OBS and the format flag for a ring's `obs` argument (None: no observations in the slot)."""
+    if obs is None:
+        return 0
+    if isinstance(obs, str) and obs == "bits":
+        return _cabi.HOST_OBS | _cabi.HOST_OBS_BITS
+    if obs in (torch.float32, torch.bfloat16):
+        return _cabi.HOST_OBS | _OBS_FORMAT_FLAG[obs]
+    raise ValueError(f"obs must be None, torch.float32, torch.bfloat16 or 'bits', got {obs!r}")
 
 
 def decode_results(packed: torch.Tensor, out: Optional[dict] = None) -> dict:
@@ -563,12 +617,14 @@ def unpack_observations(bits: torch.Tensor, C: int, F: int, rows: Optional[torch
                         dtype=torch.float32, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Expand bit-packed observations (``mapf_unpack_obs``) into the network's 0/1 values in ONE kernel pass.
 
-    bits: int32 [..., N, AW] on the GPU (AW = ``MAPF_OBS_BITS_WORDS(C, F)``); its leading dimensions are the source rows.
+    bits: int32 [..., N, AW] (AW = ``MAPF_OBS_BITS_WORDS(C, F)``); its leading dimensions are the source rows.  On the GPU
+    the unpack kernel runs; a CPU tensor (a bit-packed host slot of ``make_host_ring(obs="bits")``) is expanded on the host
+    by ``mapf_unpack_obs_host``, with the same results.
     rows: optional int64 index into the source rows (a minibatch gather): the result is [len(rows), N, C, F, F], and an
     index outside [0, rows) gives an all-zero row.  Without it the result is bits.shape[:-1] + (C, F, F).
     dtype: torch.float32 or torch.bfloat16.  out: a contiguous tensor of that shape and dtype to write into."""
     lib = _cabi.load_library()
-    assert bits.is_cuda and bits.dtype == torch.int32 and bits.is_contiguous() and bits.dim() >= 2
+    assert bits.dtype == torch.int32 and bits.is_contiguous() and bits.dim() >= 2
     assert dtype in (torch.float32, torch.bfloat16), "observations expand to f32 or bf16"
     N, AW = int(bits.shape[-2]), int(bits.shape[-1])
     assert AW == _cabi.obs_bits_words(C, F), f"last dimension {AW} is not MAPF_OBS_BITS_WORDS({C}, {F})"
@@ -582,6 +638,10 @@ def unpack_observations(bits: torch.Tensor, C: int, F: int, rows: Optional[torch
         out = torch.empty(shape, dtype=dtype, device=bits.device)
     assert out.is_contiguous() and out.dtype == dtype and tuple(out.shape) == shape and out.device == bits.device
     if n_rows == 0:
+        return out
+    if not bits.is_cuda:
+        _cabi.check(lib.mapf_unpack_obs_host(_ptr(bits), src_rows, N, int(C), int(F), _ptr(idx), n_rows,
+                                             int(dtype == torch.bfloat16), _ptr(out)), "mapf_unpack_obs_host")
         return out
     stream = _stream_ptr(bits.device)            # (`C` is the channel count here, not the ctypes module)
     with torch.cuda.device(bits.device):
