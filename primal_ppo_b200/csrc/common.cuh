@@ -16,6 +16,7 @@
 // this state and is recomputed in registers at the start of every step (SURVEY.md Appendix A.1).
 #pragma once
 #include <cuda_runtime.h>
+#include <limits.h>
 #include <stdint.h>
 
 #include "../../include/mapf_b200.h"
@@ -25,6 +26,8 @@ namespace mapf {
 constexpr int NA = 5;                 // EnvParameters.N_ACTIONS (alg_parameters.py:31)
 constexpr int WARPS_PER_BLOCK = 8;    // one warp per world, 8 worlds per 256-thread CTA
 constexpr unsigned FULL = 0xffffffffu;
+
+__host__ __device__ inline size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
 
 // status codes of getActionStatus (mapf_gym.py:440-444)
 constexpr int ST_STATIC = -1, ST_HUMAN = -2, ST_AGENT = -3, ST_REPEAT = -4, ST_OK = 1;
@@ -218,6 +221,23 @@ __device__ __forceinline__ void finish_work(int *counter, int total_warps, int l
         const int d = atomicAdd(counter + 1, 1);
         if (d == total_warps - 1) { counter[0] = 0; counter[1] = 0; }
     }
+}
+
+// Launch of a persistent kernel: as many CTAs as are resident at once on the current device (at most max_per_sm per SM)
+// and no more than need_blocks.  A failed runtime call is returned and nothing is launched.
+template <typename... P, typename... A>
+cudaError_t launch_persistent(void (*kern)(P...), int threads, size_t smem, long long need_blocks, int max_per_sm,
+                              cudaStream_t stream, const A &...args) {
+    int dev = 0, sms = 0, per_sm = 0;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e == cudaSuccess) e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem);
+    if (e != cudaSuccess) return e;
+    per_sm = per_sm < 1 ? 1 : (per_sm > max_per_sm ? max_per_sm : per_sm);
+    const long long cap = (long long)sms * per_sm;
+    kern<<<(int)(need_blocks < cap ? need_blocks : cap), threads, smem, stream>>>(args...);
+    return cudaGetLastError();
 }
 
 // Batched state prefetch.  A world's state is ~0.9 KB spread over a dozen SoA arrays; loaded world by world it reaches

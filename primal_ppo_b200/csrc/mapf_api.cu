@@ -55,6 +55,9 @@ static int cuda_fail(cudaError_t e, const char *what) {
         if (e_ != cudaSuccess) return cuda_fail(e_, #call);   \
     } while (0)
 
+// every part of a host result slot starts on a 256-byte boundary
+static int64_t round256(size_t x) { return (int64_t)((x + 255) & ~(size_t)255); }
+
 namespace mapf {
 namespace {
 
@@ -169,25 +172,24 @@ int mapf_create(const MapfConfig *cfg, MapfEnv **out) {
     alloc((void **)&e->d_count, 4);
     // result-slot layout: f32 fields first, then the byte fields; every field 256-byte aligned
     {
-        auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
         MapfHostLayout &L = e->lay;
-        size_t o = 0;
-        L.off_reward = (int64_t)o; o += up(WN * 4);
-        L.off_cost = (int64_t)o; o += up(WN * 4);
-        L.off_shadow_goals = (int64_t)o; o += up(W * 4);
-        L.off_status = (int64_t)o; o += up(WN);
-        L.off_goals_reached = (int64_t)o; o += up(WN);
-        L.off_violated = (int64_t)o; o += up(WN);
-        L.off_fixed_actions = (int64_t)o; o += up(WN);
+        int64_t o = 0;
+        L.off_reward = o; o += round256(WN * 4);
+        L.off_cost = o; o += round256(WN * 4);
+        L.off_shadow_goals = o; o += round256(W * 4);
+        L.off_status = o; o += round256(WN);
+        L.off_goals_reached = o; o += round256(WN);
+        L.off_violated = o; o += round256(WN);
+        L.off_fixed_actions = o; o += round256(WN);
         L.off_train_valid = -1;
         L.off_packed = -1;
-        L.slot_bytes = (int64_t)o;
+        L.slot_bytes = o;
         MapfHostLayout &Lc = e->lay_c;
         Lc.off_reward = Lc.off_cost = Lc.off_status = Lc.off_goals_reached = Lc.off_violated = Lc.off_fixed_actions = -1;
         Lc.off_train_valid = -1;
         Lc.off_packed = 0;
-        Lc.off_shadow_goals = (int64_t)up(WN * 2);
-        Lc.slot_bytes = Lc.off_shadow_goals + (int64_t)up(W * 4);
+        Lc.off_shadow_goals = round256(WN * 2);
+        Lc.slot_bytes = Lc.off_shadow_goals + round256(W * 4);
     }
     for (int k = 0; k < 2; ++k) {
         alloc((void **)&e->d_slot[k], (size_t)e->lay.slot_bytes);
@@ -242,9 +244,13 @@ int mapf_reset(MapfEnv *e, const MapfScenario *sc, void *stream) {
     return MAPF_OK;
 }
 
-#define NEED_ENV(name)                                                                     \
-    if (!e) return fail(MAPF_E_NULL, name ": null env");                                   \
-    if (!e->has_scenario) return fail(MAPF_E_STATE, name ": mapf_reset has not been called"); \
+static int check_env(const MapfEnv *e, const char *name) {
+    if (!e) return fail(MAPF_E_NULL, "%s: null env", name);
+    if (!e->has_scenario) return fail(MAPF_E_STATE, "%s: mapf_reset has not been called", name);
+    return MAPF_OK;
+}
+#define NEED_ENV(name)                                  \
+    if (int rc_ = check_env(e, name)) return rc_;       \
     ON_DEVICE(e->cfg.device)
 #define WC(e, k) ((e)->d_work + 2 * (k))
 
@@ -305,78 +311,74 @@ int mapf_step(MapfEnv *e, const int8_t *actions, const MapfStepOut *out, void *s
     return MAPF_OK;
 }
 
-int mapf_observe(MapfEnv *e, float *obs, float *vec, void *stream) {
-    NEED_ENV("mapf_observe");
-    if (int rc = check_vec(vec, "mapf_observe")) return rc;
-    if (!obs || !vec) return fail(MAPF_E_NULL, "mapf_observe: null argument");
-    CU(launch_observe(e->v, obs, vec, WC(e, WC_OBSERVE), (cudaStream_t)stream));
-    return MAPF_OK;
-}
-
-int mapf_step_observe(MapfEnv *e, const int8_t *actions, const MapfStepOut *out, float *obs, float *vec, void *stream) {
-    NEED_ENV("mapf_step_observe");
-    if (int rc = check_vec(vec, "mapf_step_observe")) return rc;
-    if (!actions || !out || !obs || !vec) return fail(MAPF_E_NULL, "mapf_step_observe: null argument");
-    if (int rc = check_step_n(e, "mapf_step_observe")) return rc;
-    CU(do_step_observe(e, actions, *out, obs, vec, (cudaStream_t)stream, OBS_F32));
-    return MAPF_OK;
-}
-
-/* bf16 variants: the same 0/1 observation values, half the bytes (optional format for GPU-resident training) */
-int mapf_observe_bf16(MapfEnv *e, uint16_t *obs_bf16, float *vec, void *stream) {
-    NEED_ENV("mapf_observe_bf16");
-    if (int rc = check_vec(vec, "mapf_observe_bf16")) return rc;
-    if (!obs_bf16 || !vec) return fail(MAPF_E_NULL, "mapf_observe_bf16: null argument");
-    CU(launch_observe(e->v, reinterpret_cast<float *>(obs_bf16), vec, WC(e, WC_OBSERVE), (cudaStream_t)stream, OBS_BF16));
-    return MAPF_OK;
-}
-
-int mapf_step_observe_bf16(MapfEnv *e, const int8_t *actions, const MapfStepOut *out, uint16_t *obs_bf16, float *vec, void *stream) {
-    NEED_ENV("mapf_step_observe_bf16");
-    if (int rc = check_vec(vec, "mapf_step_observe_bf16")) return rc;
-    if (!actions || !out || !obs_bf16 || !vec) return fail(MAPF_E_NULL, "mapf_step_observe_bf16: null argument");
-    if (int rc = check_step_n(e, "mapf_step_observe_bf16")) return rc;
-    CU(do_step_observe(e, actions, *out, reinterpret_cast<float *>(obs_bf16), vec, (cudaStream_t)stream, OBS_BF16));
-    return MAPF_OK;
-}
-
-/* bit-packed variants: one bit per observation cell, u32 [W,N,MAPF_OBS_BITS_WORDS(C,F)] */
+/* bit-packed output: one bit per observation cell, u32 [W,N,MAPF_OBS_BITS_WORDS(C,F)] */
 static int check_bits(const uint32_t *obs_bits, const char *name) {
     if (reinterpret_cast<uintptr_t>(obs_bits) & 3) return fail(MAPF_E_BAD_CONFIG, "%s: obs_bits must be 4-byte aligned", name);
     return MAPF_OK;
 }
 
-int mapf_observe_bits(MapfEnv *e, uint32_t *obs_bits, float *vec, void *stream) {
-    NEED_ENV("mapf_observe_bits");
-    if (!obs_bits || !vec) return fail(MAPF_E_NULL, "mapf_observe_bits: null argument");
-    if (int rc = check_vec(vec, "mapf_observe_bits")) return rc;
-    if (int rc = check_bits(obs_bits, "mapf_observe_bits")) return rc;
-    CU(launch_observe(e->v, reinterpret_cast<float *>(obs_bits), vec, WC(e, WC_OBSERVE), (cudaStream_t)stream, OBS_BITS));
+// The observation entry points in format `fmt`: mapf_observe* (step = false; actions and out are not used) and
+// mapf_step_observe*.
+static int observe_call(const char *name, MapfEnv *e, bool step, const int8_t *actions, const MapfStepOut *out, void *obs,
+                        float *vec, void *stream, int fmt) {
+    NEED_ENV(name);
+    if (!obs || !vec || (step && (!actions || !out))) return fail(MAPF_E_NULL, "%s: null argument", name);
+    if (int rc = check_vec(vec, name)) return rc;
+    if (fmt == OBS_BITS)
+        if (int rc = check_bits(static_cast<const uint32_t *>(obs), name)) return rc;
+    if (step) {
+        if (int rc = check_step_n(e, name)) return rc;
+        CU(do_step_observe(e, actions, *out, static_cast<float *>(obs), vec, (cudaStream_t)stream, fmt));
+    } else {
+        CU(launch_observe(e->v, static_cast<float *>(obs), vec, WC(e, WC_OBSERVE), (cudaStream_t)stream, fmt));
+    }
     return MAPF_OK;
+}
+
+int mapf_observe(MapfEnv *e, float *obs, float *vec, void *stream) {
+    return observe_call("mapf_observe", e, false, nullptr, nullptr, obs, vec, stream, OBS_F32);
+}
+
+int mapf_step_observe(MapfEnv *e, const int8_t *actions, const MapfStepOut *out, float *obs, float *vec, void *stream) {
+    return observe_call("mapf_step_observe", e, true, actions, out, obs, vec, stream, OBS_F32);
+}
+
+/* bf16 variants: the same 0/1 observation values, half the bytes (optional format for GPU-resident training) */
+int mapf_observe_bf16(MapfEnv *e, uint16_t *obs_bf16, float *vec, void *stream) {
+    return observe_call("mapf_observe_bf16", e, false, nullptr, nullptr, obs_bf16, vec, stream, OBS_BF16);
+}
+
+int mapf_step_observe_bf16(MapfEnv *e, const int8_t *actions, const MapfStepOut *out, uint16_t *obs_bf16, float *vec, void *stream) {
+    return observe_call("mapf_step_observe_bf16", e, true, actions, out, obs_bf16, vec, stream, OBS_BF16);
+}
+
+int mapf_observe_bits(MapfEnv *e, uint32_t *obs_bits, float *vec, void *stream) {
+    return observe_call("mapf_observe_bits", e, false, nullptr, nullptr, obs_bits, vec, stream, OBS_BITS);
 }
 
 int mapf_step_observe_bits(MapfEnv *e, const int8_t *actions, const MapfStepOut *out, uint32_t *obs_bits, float *vec,
                            void *stream) {
-    NEED_ENV("mapf_step_observe_bits");
-    if (!actions || !out || !obs_bits || !vec) return fail(MAPF_E_NULL, "mapf_step_observe_bits: null argument");
-    if (int rc = check_vec(vec, "mapf_step_observe_bits")) return rc;
-    if (int rc = check_bits(obs_bits, "mapf_step_observe_bits")) return rc;
-    if (int rc = check_step_n(e, "mapf_step_observe_bits")) return rc;
-    CU(do_step_observe(e, actions, *out, reinterpret_cast<float *>(obs_bits), vec, (cudaStream_t)stream, OBS_BITS));
+    return observe_call("mapf_step_observe_bits", e, true, actions, out, obs_bits, vec, stream, OBS_BITS);
+}
+
+// argument checks shared by mapf_unpack_obs and mapf_unpack_obs_host
+static int check_unpack(const char *name, const uint32_t *obs_bits, int64_t src_rows, int32_t agents, int32_t num_channel,
+                        int32_t fov, int64_t n_rows, int32_t out_bf16, const void *out) {
+    if (!obs_bits || !out) return fail(MAPF_E_NULL, "%s: null argument", name);
+    if (src_rows < 0 || n_rows < 0) return fail(MAPF_E_BAD_CONFIG, "%s: negative row count", name);
+    if (agents < 1 || agents > 254) return fail(MAPF_E_BAD_CONFIG, "%s: agents must be in 1..254", name);
+    if (num_channel != 5 && num_channel != 6) return fail(MAPF_E_BAD_CONFIG, "%s: num_channel must be 5 or 6", name);
+    if (fov < 3 || fov > 31 || (fov & 1) == 0) return fail(MAPF_E_BAD_CONFIG, "%s: fov must be odd in 3..31", name);
+    if (out_bf16 != 0 && out_bf16 != 1) return fail(MAPF_E_BAD_CONFIG, "%s: out_bf16 must be 0 or 1", name);
+    if (int rc = check_bits(obs_bits, name)) return rc;
+    if (reinterpret_cast<uintptr_t>(out) & (out_bf16 ? 1 : 3))
+        return fail(MAPF_E_BAD_CONFIG, "%s: out must be aligned to its element size", name);
     return MAPF_OK;
 }
 
 int mapf_unpack_obs(const uint32_t *obs_bits, int64_t src_rows, int32_t agents, int32_t num_channel, int32_t fov,
                     const int64_t *rows, int64_t n_rows, int32_t out_bf16, void *out, void *stream) {
-    if (!obs_bits || !out) return fail(MAPF_E_NULL, "mapf_unpack_obs: null argument");
-    if (src_rows < 0 || n_rows < 0) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: negative row count");
-    if (agents < 1 || agents > 254) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: agents must be in 1..254");
-    if (num_channel != 5 && num_channel != 6) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: num_channel must be 5 or 6");
-    if (fov < 3 || fov > 31 || (fov & 1) == 0) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: fov must be odd in 3..31");
-    if (out_bf16 != 0 && out_bf16 != 1) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: out_bf16 must be 0 or 1");
-    if (int rc = check_bits(obs_bits, "mapf_unpack_obs")) return rc;
-    if (reinterpret_cast<uintptr_t>(out) & (out_bf16 ? 1 : 3))
-        return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs: out must be aligned to its element size");
+    if (int rc = check_unpack("mapf_unpack_obs", obs_bits, src_rows, agents, num_channel, fov, n_rows, out_bf16, out)) return rc;
     if (n_rows == 0) return MAPF_OK;
     CU(launch_unpack_obs(obs_bits, src_rows, agents, num_channel, fov, rows, n_rows, out_bf16, out, (cudaStream_t)stream));
     return MAPF_OK;
@@ -599,19 +601,34 @@ size_t obs_bytes(const EnvView &v, int fmt) {
 
 bool overlaps(uintptr_t lo, uintptr_t hi, const uintptr_t r[2]) { return lo < r[1] && r[0] < hi; }
 
+// The host result slot of the split-phase call for `flags`: the device slot (full or compact), then trainValid
+// (MAPF_HOST_TRAIN_VALID), then the observations in format `fmt` and vec (MAPF_HOST_OBS).  off_obs / off_vec are where
+// the last two start.
+struct HostSlot {
+    MapfHostLayout lay;
+    int64_t off_obs, off_vec;
+};
+HostSlot host_slot(const MapfEnv *e, int flags, int fmt) {
+    const size_t WN = (size_t)e->v.W * e->v.N;
+    HostSlot h;
+    h.lay = (flags & MAPF_HOST_COMPACT) ? e->lay_c : e->lay;
+    if (flags & MAPF_HOST_TRAIN_VALID) {
+        h.lay.off_train_valid = h.lay.slot_bytes;
+        h.lay.slot_bytes += round256(WN * NA * 4);
+    }
+    h.off_obs = h.lay.slot_bytes;
+    h.off_vec = h.off_obs + round256(obs_bytes(e->v, fmt));
+    if (flags & MAPF_HOST_OBS) h.lay.slot_bytes = h.off_vec + round256(WN * 16);
+    return h;
+}
+
 }  // namespace
 
 int mapf_host_layout(MapfEnv *e, int flags, MapfHostLayout *out) {
     if (!e || !out) return fail(MAPF_E_NULL, "mapf_host_layout: null argument");
     const int fmt = host_obs_format(flags);
     if (fmt < 0) return fail(MAPF_E_BAD_CONFIG, "mapf_host_layout: MAPF_HOST_OBS_BF16 and MAPF_HOST_OBS_BITS are exclusive");
-    auto up = [](size_t x) { return (int64_t)((x + 255) & ~(size_t)255); };
-    *out = (flags & MAPF_HOST_COMPACT) ? e->lay_c : e->lay;
-    if (flags & MAPF_HOST_TRAIN_VALID) {
-        out->off_train_valid = out->slot_bytes;
-        out->slot_bytes += up((size_t)e->v.W * e->v.N * NA * 4);
-    }
-    if (flags & MAPF_HOST_OBS) out->slot_bytes += up(obs_bytes(e->v, fmt)) + up((size_t)e->v.W * e->v.N * 16);
+    *out = host_slot(e, flags, fmt).lay;
     return MAPF_OK;
 }
 
@@ -661,14 +678,13 @@ int mapf_step_observe_host_begin(MapfEnv *e, const int8_t *actions_host, void *r
     CU(cudaEventRecord(e->ev_step[k], s));
     CU(cudaStreamWaitEvent(cs, e->ev_step[k], 0));
     char *const host = static_cast<char *>(result_slot_host);
+    const HostSlot h = host_slot(e, flags, fmt);
     CU(cudaMemcpyAsync(host, e->d_slot[k], slot_bytes, cudaMemcpyDeviceToHost, cs));   // ONE copy
-    const size_t up_tv = (WN * NA * 4 + 255) & ~(size_t)255;
-    if (with_tv) CU(cudaMemcpyAsync(host + slot_bytes, train_valid_dev, WN * NA * 4, cudaMemcpyDeviceToHost, cs));
+    if (with_tv) CU(cudaMemcpyAsync(host + h.lay.off_train_valid, train_valid_dev, WN * NA * 4, cudaMemcpyDeviceToHost, cs));
     const uintptr_t ob = reinterpret_cast<uintptr_t>(obs_dev), vc = reinterpret_cast<uintptr_t>(vec_dev);
     if (with_obs) {
-        const size_t off_obs = slot_bytes + (with_tv ? up_tv : 0), off_vec = off_obs + ((n_obs + 255) & ~(size_t)255);
-        CU(cudaMemcpyAsync(host + off_obs, obs_dev, n_obs, cudaMemcpyDeviceToHost, cs));
-        CU(cudaMemcpyAsync(host + off_vec, vec_dev, WN * 16, cudaMemcpyDeviceToHost, cs));
+        CU(cudaMemcpyAsync(host + h.off_obs, obs_dev, n_obs, cudaMemcpyDeviceToHost, cs));
+        CU(cudaMemcpyAsync(host + h.off_vec, vec_dev, WN * 16, cudaMemcpyDeviceToHost, cs));
     }
     CU(cudaEventRecord(e->ev_copied[k], cs));
     e->tv_copy_pending[k] = with_tv;
@@ -701,15 +717,8 @@ int mapf_decode_results_host(const uint16_t *packed, int64_t n, const MapfStepOu
 
 int mapf_unpack_obs_host(const uint32_t *obs_bits, int64_t src_rows, int32_t agents, int32_t num_channel, int32_t fov,
                          const int64_t *rows, int64_t n_rows, int32_t out_bf16, void *out) {
-    if (!obs_bits || !out) return fail(MAPF_E_NULL, "mapf_unpack_obs_host: null argument");
-    if (src_rows < 0 || n_rows < 0) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: negative row count");
-    if (agents < 1 || agents > 254) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: agents must be in 1..254");
-    if (num_channel != 5 && num_channel != 6) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: num_channel must be 5 or 6");
-    if (fov < 3 || fov > 31 || (fov & 1) == 0) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: fov must be odd in 3..31");
-    if (out_bf16 != 0 && out_bf16 != 1) return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: out_bf16 must be 0 or 1");
-    if (int rc = check_bits(obs_bits, "mapf_unpack_obs_host")) return rc;
-    if (reinterpret_cast<uintptr_t>(out) & (out_bf16 ? 1 : 3))
-        return fail(MAPF_E_BAD_CONFIG, "mapf_unpack_obs_host: out must be aligned to its element size");
+    if (int rc = check_unpack("mapf_unpack_obs_host", obs_bits, src_rows, agents, num_channel, fov, n_rows, out_bf16, out))
+        return rc;
     // byte -> its eight 0/1 values, LSB first: one table lookup and copy per 8 cells
     static const struct Lut {
         float f[256][8];

@@ -28,10 +28,7 @@ unpack_obs_kernel(const uint32_t *__restrict__ bits, const long long src_rows, c
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint32_t *const aw = reinterpret_cast<uint32_t *>(smem_raw + (size_t)warp * per_warp);
     uint32_t *const wb = reinterpret_cast<uint32_t *>(smem_raw + (size_t)warp * per_warp + align16((size_t)CH * AST * 4));
-    if (threadIdx.x < 16) {
-        const uint32_t one = 0x3f800000u, t = threadIdx.x;
-        lut[t] = make_uint4((t & 1u) ? one : 0u, (t & 2u) ? one : 0u, (t & 4u) ? one : 0u, (t & 8u) ? one : 0u);
-    }
+    fill_lut(lut, threadIdx.x);
     __syncthreads();
     const Grp<32> g(lane);
     const size_t row_words = (size_t)N * AW;
@@ -57,30 +54,13 @@ unpack_obs_kernel(const uint32_t *__restrict__ bits, const long long src_rows, c
 
 cudaError_t launch_unpack_obs(const uint32_t *bits, long long src_rows, int N, int C, int F, const int64_t *rows,
                               long long n_rows, int out_bf16, void *out, cudaStream_t stream) {
-    const int PB = C * F * F, AW = bits_words(PB), AST = agent_stride(PB);
-    // agents per chunk: the rule of the observation kernels (~24 KB of bit-string scratch per warp at most)
-    int CH = N < 32 ? N : 32;
-    while (CH > 4 && (size_t)CH * (AW + 2) * 4 * 2 > 24 * 1024) CH >>= 1;
-    const int WB = (CH * PB + 31) / 32 + 2;
-    const int per_warp = (int)(align16((size_t)CH * AST * 4) + align16((size_t)WB * 4));
-    const size_t smem = (size_t)per_warp * UNPACK_WARPS;
+    const int PB = C * F * F, CH = obs_chunk(N, PB);
+    const int per_warp = (int)warp_scratch_bytes(CH, PB);
     const int fmt = out_bf16 ? OBS_BF16 : OBS_F32;
-    const size_t al = out_bf16 ? 8 : 4;                     // elements per 16-byte store
-    const bool vec4 = ((size_t)N * PB) % al == 0 && (CH >= N || ((size_t)CH * PB) % al == 0) &&
-                      (reinterpret_cast<uintptr_t>(out) & 15) == 0;
-    auto kern = vec4 ? unpack_obs_kernel<true> : unpack_obs_kernel<false>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    int dev = 0, sms = 148, per_sm = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, UNPACK_WARPS * 32, smem);
-    if (per_sm < 1) per_sm = 1;
-    const long long need = (n_rows + UNPACK_WARPS - 1) / UNPACK_WARPS;
-    const int blocks = (int)(need < (long long)sms * per_sm ? need : (long long)sms * per_sm);
-    kern<<<blocks, UNPACK_WARPS * 32, smem, stream>>>(bits, src_rows, N, PB, AW, AST, CH, per_warp, (32 * 32) / PB,
-                                                      (32 * 32) % PB, rows, n_rows, fmt, out);
-    return cudaGetLastError();
+    auto kern = obs_vec4(fmt, N, PB, CH, out) ? unpack_obs_kernel<true> : unpack_obs_kernel<false>;
+    return launch_persistent(kern, UNPACK_WARPS * 32, (size_t)per_warp * UNPACK_WARPS, (n_rows + UNPACK_WARPS - 1) / UNPACK_WARPS,
+                             INT_MAX, stream, bits, src_rows, N, PB, bits_words(PB), agent_stride(PB), CH, per_warp,
+                             (32 * 32) / PB, (32 * 32) % PB, rows, n_rows, fmt, out);
 }
 
 }  // namespace mapf

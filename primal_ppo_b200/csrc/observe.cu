@@ -36,10 +36,7 @@ observe_kernel(const EnvView v, float *__restrict__ obs, float *__restrict__ vec
     uint32_t *const obits = m.obits, *const abits = m.abits;
     uint8_t *const grid = m.grid;
 
-    if (threadIdx.x < 16) {
-        const uint32_t one = 0x3f800000u, t = threadIdx.x;
-        lut[t] = make_uint4((t & 1u) ? one : 0u, (t & 2u) ? one : 0u, (t & 4u) ? one : 0u, (t & 8u) ? one : 0u);
-    }
+    fill_lut(lut, threadIdx.x);
     __syncthreads();
 
     // dynamic world scheduling: w (inputs in registers) is processed while w1, claimed at the top of the iteration, is
@@ -84,62 +81,29 @@ observe_kernel(const EnvView v, float *__restrict__ obs, float *__restrict__ vec
     finish_work(work_counter, gridDim.x * (blockDim.x >> 5), lane);
 }
 
-template <int C_T, int F_T, bool VEC4, bool BITS = false>
-cudaError_t launch_t(const EnvView &v, float *obs, float *vec, const ObsLayout &L, int wpb, int *counter, cudaStream_t stream) {
-    const size_t smem = L.total * wpb;
-    cudaError_t e = cudaFuncSetAttribute(observe_kernel<C_T, F_T, VEC4, BITS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    int dev = 0, sms = 148, per_sm = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, observe_kernel<C_T, F_T, VEC4, BITS>, wpb * 32, smem);
-    if (per_sm < 1) per_sm = 1;
-    // Store-dominated worlds (>= 32 KB of observations each) run best with FEWER resident warps: the HBM write path prefers
-    // fewer, longer write streams (write-pattern benchmark: 16 warps/SM beat 32 by 2 %), and this kernel has no other
-    // latency to hide.  In-process A/B at 40x40x32: 1 / 2 / 3 / 4 CTAs per SM = 0.613 / 0.608 / 0.612 / 0.622 ms.
-    if (obs_world_bytes(L, v.N) >= 32768 && per_sm > 2) per_sm = 2;
-    const int need = (v.W + wpb - 1) / wpb;
-    const int blocks = need < sms * per_sm ? need : sms * per_sm;
-    observe_kernel<C_T, F_T, VEC4, BITS><<<blocks, wpb * 32, smem, stream>>>(v, obs, vec, L, counter);
-    return cudaGetLastError();
-}
-
 }  // namespace
 
 cudaError_t launch_observe(const EnvView &v, float *obs, float *vec, int *work_counter, cudaStream_t stream, int fmt) {
-    const int PB = v.C * v.F * v.F;
+    const int PB = v.C * v.F * v.F, CH = obs_chunk(v.N, PB);
     // worlds whose block needs several warp passes: one CTA per world with shared staging (observe_wide.cu)
-    if ((v.N > 32 || (size_t)v.N * ((PB + 31) / 32 + 2) * 4 * 2 > 24 * 1024 || (v.dbg_flags & 4)) && !(v.dbg_flags & 2)) {
+    if ((v.N > 32 || CH < v.N || (v.dbg_flags & 4)) && !(v.dbg_flags & 2)) {
         const cudaError_t e = launch_observe_wide(v, obs, vec, work_counter, stream, fmt);
         if (e != cudaErrorNotSupported) return e;
     }
-    // chunk of agents handled per phase-1 pass: as many as fit ~24 KB of bit-string scratch per warp
-    int CH = v.N < 32 ? v.N : 32;
-    while (CH > 4 && (size_t)CH * ((PB + 31) / 32 + 2) * 4 * 2 > 24 * 1024) CH >>= 1;
-    const size_t al = fmt == OBS_BF16 ? 8 : 4;        // elements per 16-byte store
     ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, CH);
     L.fmt = fmt;
-    // bits: every agent's record is AW words, so any chunk starts on a 16-byte boundary when AW % 4 == 0
-    const bool vec4 = (fmt == OBS_BITS ? bits_words(L.PB) % 4 == 0
-                                       : ((size_t)v.N * PB) % al == 0 && (CH >= v.N || ((size_t)CH * PB) % al == 0)) &&
-                      (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
     int wpb = WARPS_PER_BLOCK;
     while (wpb > 1 && L.total * wpb > 200 * 1024) wpb >>= 1;
     if (L.total * wpb > 227 * 1024) return cudaErrorInvalidConfiguration;
-    if (fmt == OBS_BITS) {
-        if (v.C == 6 && v.F == 9) {
-            return vec4 ? launch_t<6, 9, true, true>(v, obs, vec, L, wpb, work_counter, stream)
-                        : launch_t<6, 9, false, true>(v, obs, vec, L, wpb, work_counter, stream);
-        }
-        return vec4 ? launch_t<0, 0, true, true>(v, obs, vec, L, wpb, work_counter, stream)
-                    : launch_t<0, 0, false, true>(v, obs, vec, L, wpb, work_counter, stream);
-    }
-    if (v.C == 6 && v.F == 9) {
-        return vec4 ? launch_t<6, 9, true>(v, obs, vec, L, wpb, work_counter, stream)
-                    : launch_t<6, 9, false>(v, obs, vec, L, wpb, work_counter, stream);
-    }
-    return vec4 ? launch_t<0, 0, true>(v, obs, vec, L, wpb, work_counter, stream)
-                : launch_t<0, 0, false>(v, obs, vec, L, wpb, work_counter, stream);
+    // Store-dominated worlds (>= 32 KB of observations each) run best with FEWER resident warps: the HBM write path prefers
+    // fewer, longer write streams (write-pattern benchmark: 16 warps/SM beat 32 by 2 %), and this kernel has no other
+    // latency to hide.  In-process A/B at 40x40x32: 1 / 2 / 3 / 4 CTAs per SM = 0.613 / 0.608 / 0.612 / 0.622 ms.
+    const int max_per_sm = obs_world_bytes(L, v.N) >= 32768 ? 2 : INT_MAX;
+    return dispatch_obs(fmt, v.C, v.F, obs_vec4(fmt, v.N, PB, CH, obs), [&](auto t) {
+        using T = decltype(t);
+        return launch_persistent(observe_kernel<T::C_T, T::F_T, T::VEC4, T::BITS>, wpb * 32, L.total * wpb,
+                                 (v.W + wpb - 1) / wpb, max_per_sm, stream, v, obs, vec, L, work_counter);
+    });
 }
 
 }  // namespace mapf

@@ -38,10 +38,7 @@ observe_wide_kernel(const EnvView v, float *__restrict__ obs, float *__restrict_
     unsigned char *mine = smem_raw + shared_bytes + (size_t)warp * per_warp;
     m.aw = reinterpret_cast<uint32_t *>(mine);
     m.wb = reinterpret_cast<uint32_t *>(mine + ((size_t)L.CH * L.AST * 4 + 15) / 16 * 16);
-    if (tid < 16) {
-        const uint32_t one = 0x3f800000u, t = tid;
-        lut[t] = make_uint4((t & 1u) ? one : 0u, (t & 2u) ? one : 0u, (t & 4u) ? one : 0u, (t & 8u) ? one : 0u);
-    }
+    fill_lut(lut, tid);
     for (int k = tid; k < nob; k += blockDim.x) m.abits[k] = 0;
     for (int k = tid; k < (HP * GS) / 16; k += blockDim.x) reinterpret_cast<uint4 *>(m.grid)[k] = make_uint4(0, 0, 0, 0);
     const int nchunks = (N + L.CH - 1) / L.CH;
@@ -96,41 +93,19 @@ cudaError_t launch_observe_wide(const EnvView &v, float *obs, float *vec, int *w
     const int PB = v.C * v.F * v.F;
     // chunk size: per-warp scratch (aw + wb) of at most ~12 KB, and at least one chunk per warp when N allows it
     int CH = 32;
-    while (CH > 2 && ((size_t)CH * ((PB + 31) / 32 + 2) * 4 * 2 > 12 * 1024 || (v.N + CH - 1) / CH < WIDE_WARPS)) CH >>= 1;
-    if ((size_t)CH * ((PB + 31) / 32 + 2) * 4 * 2 > 28 * 1024) return cudaErrorNotSupported;
+    while (CH > 2 && (chunk_scratch(CH, PB) > 12 * 1024 || (v.N + CH - 1) / CH < WIDE_WARPS)) CH >>= 1;
+    if (chunk_scratch(CH, PB) > 28 * 1024) return cudaErrorNotSupported;
     ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, CH);
     L.alias = 0;
     L.fmt = fmt;
-    // the CTA-shared part: [obits | abits | grid | goals+cells]; make_layout put goals at off_goal (after the staging)
-    const int shared_bytes = (int)(L.off_goal + (((size_t)v.N * 8 + 15) / 16) * 16);
-    const int per_warp = (int)((((size_t)CH * L.AST * 4 + 15) / 16) * 16 + (((size_t)L.WB * 4 + 15) / 16) * 16);
+    const int shared_bytes = (int)cta_shared_bytes(L, v.N), per_warp = (int)warp_scratch_bytes(CH, PB);
     const size_t smem = (size_t)shared_bytes + (size_t)per_warp * WIDE_WARPS;
     if (smem > 200 * 1024) return cudaErrorNotSupported;
-    const size_t al = fmt == OBS_BF16 ? 8 : 4;
-    const bool vec4 = (fmt == OBS_BITS ? bits_words(L.PB) % 4 == 0 : ((size_t)CH * PB) % al == 0 && ((size_t)v.N * PB) % al == 0) &&
-                      (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
-    int dev = 0, sms = 148, per_sm = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaError_t e;
-#define LAUNCH(...)                                                                                                \
-    do {                                                                                                           \
-        e = cudaFuncSetAttribute(observe_wide_kernel<__VA_ARGS__>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);  \
-        if (e != cudaSuccess) return e;                                                                            \
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, observe_wide_kernel<__VA_ARGS__>, WIDE_WARPS * 32, smem);     \
-        if (per_sm < 1) per_sm = 1;                                                                                \
-        const int blocks = v.W < sms * per_sm ? v.W : sms * per_sm;                                                \
-        observe_wide_kernel<__VA_ARGS__><<<blocks, WIDE_WARPS * 32, smem, stream>>>(v, obs, vec, L, shared_bytes, per_warp, work_counter); \
-    } while (0)
-    if (fmt == OBS_BITS) {
-        if (v.C == 6 && v.F == 9) { if (vec4) LAUNCH(6, 9, true, true); else LAUNCH(6, 9, false, true); }
-        else { if (vec4) LAUNCH(0, 0, true, true); else LAUNCH(0, 0, false, true); }
-    } else {
-        if (v.C == 6 && v.F == 9) { if (vec4) LAUNCH(6, 9, true, false); else LAUNCH(6, 9, false, false); }
-        else { if (vec4) LAUNCH(0, 0, true, false); else LAUNCH(0, 0, false, false); }
-    }
-#undef LAUNCH
-    return cudaGetLastError();
+    return dispatch_obs(fmt, v.C, v.F, obs_vec4(fmt, v.N, PB, CH, obs), [&](auto t) {
+        using T = decltype(t);
+        return launch_persistent(observe_wide_kernel<T::C_T, T::F_T, T::VEC4, T::BITS>, WIDE_WARPS * 32, smem, v.W, INT_MAX,
+                                 stream, v, obs, vec, L, shared_bytes, per_warp, work_counter);
+    });
 }
 
 }  // namespace mapf

@@ -1,13 +1,14 @@
 // observe_world.cuh — observation building of ONE world by one warp: the device code shared by observe_kernel
-// (observe.cu) and the fused step_observe_kernel (step_observe.cu).  See observe.cu for the design notes and the
-// reference lines (mapf_gym.py:192-198, 246-336).
+// (observe.cu) and the fused step_observe_kernel (step_observe.cu), and the per-chunk code the CTA-per-world kernels
+// (observe_wide.cu, step_observe_wide.cu) and the unpack kernel (obs_bits.cu) share with them.  Also the host-side
+// launch planning of all of them: chunk size, shared-memory layout, when 16-byte stores are allowed, and the mapping of
+// the runtime format / shape onto a kernel instantiation.  See observe.cu for the design notes and the reference lines
+// (mapf_gym.py:192-198, 246-336).
 #pragma once
 #include "common.cuh"
 
 namespace mapf {
 namespace ow {
-
-__host__ __device__ inline size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
 
 constexpr int OBW = 4;   // packed obstacle words prefetched per lane (PW <= 128: up to 64x64 cells; 40x40 needs 52)
 
@@ -65,6 +66,53 @@ inline size_t obs_world_bytes(const ObsLayout &L, int N) {
     return (size_t)N * L.PB * (L.fmt == OBS_BF16 ? 2 : 4);
 }
 
+// Bit-string scratch of one warp for a chunk of CH agents, as the chunk-size rules of the launchers estimate it: CH agent
+// strings of (PB + 31) / 32 + 2 words, twice (per-agent strings aw, chunk string wb).
+inline size_t chunk_scratch(int CH, int PB) { return (size_t)CH * ((PB + 31) / 32 + 2) * 4 * 2; }
+
+// Agents per chunk of the warp-per-world kernels and of the unpack kernel: as many as fit ~24 KB of scratch per warp.
+inline int obs_chunk(int N, int PB) {
+    int CH = N < 32 ? N : 32;
+    while (CH > 4 && chunk_scratch(CH, PB) > 24 * 1024) CH >>= 1;
+    return CH;
+}
+
+// CTA-per-world kernels: the staging part of L ([obits | abits | grid | goals + cells]) is shared by the CTA, and each warp
+// has its own scratch behind it (aw: CH agent strings at stride AST, then wb: the chunk bit string).
+inline size_t cta_shared_bytes(const ObsLayout &L, int N) { return L.off_goal + align16((size_t)N * 8); }
+inline size_t warp_scratch_bytes(int CH, int PB) {
+    return align16((size_t)CH * agent_stride(PB) * 4) + align16((size_t)((CH * PB + 31) / 32 + 2) * 4);
+}
+
+// 16-byte stores (VEC4) need `obs` and the start of every chunk of CH agents 16-byte aligned.  Bits: every record is AW
+// words.  f32 / bf16 (4 / 8 elements per store): N * PB, and CH * PB when a world takes several chunks.
+inline bool obs_vec4(int fmt, int N, int PB, int CH, const void *obs) {
+    if (reinterpret_cast<uintptr_t>(obs) & 15) return false;
+    if (fmt == OBS_BITS) return bits_words(PB) % 4 == 0;
+    const size_t al = fmt == OBS_BF16 ? 8 : 4;
+    return ((size_t)N * PB) % al == 0 && (CH >= N || ((size_t)CH * PB) % al == 0);
+}
+
+// Compile-time parameters of an observation kernel: C_T / F_T = 6 / 9 (the training configuration) or 0 / 0 (runtime values
+// from EnvView), VEC4 (16-byte stores), BITS (OBS_BITS output).
+template <int C_, int F_, bool VEC4_, bool BITS_>
+struct ObsVariant {
+    static constexpr int C_T = C_, F_T = F_;
+    static constexpr bool VEC4 = VEC4_, BITS = BITS_;
+};
+
+// Calls fn(ObsVariant<...>()) for the runtime format, channels x FOV and store width.
+template <typename Fn>
+cudaError_t dispatch_obs(int fmt, int C, int F, bool vec4, Fn &&fn) {
+    const bool c69 = C == 6 && F == 9;
+    if (fmt == OBS_BITS) {
+        if (c69) return vec4 ? fn(ObsVariant<6, 9, true, true>()) : fn(ObsVariant<6, 9, false, true>());
+        return vec4 ? fn(ObsVariant<0, 0, true, true>()) : fn(ObsVariant<0, 0, false, true>());
+    }
+    if (c69) return vec4 ? fn(ObsVariant<6, 9, true, false>()) : fn(ObsVariant<6, 9, false, false>());
+    return vec4 ? fn(ObsVariant<0, 0, true, false>()) : fn(ObsVariant<0, 0, false, false>());
+}
+
 __device__ __forceinline__ void or_bits(uint32_t *words, int p, uint32_t val, int nbits) {
     const int k = p >> 5, s = p & 31;
     words[k] |= val << s;
@@ -109,6 +157,15 @@ __device__ __forceinline__ ObsSmem obs_carve(unsigned char *base, const ObsLayou
     m.wb = reinterpret_cast<uint32_t *>(base + L.off_wb);
     return m;
 }
+
+// nibble -> four 0/1 floats for phase 2's 16-byte stores; filled by threads t < 16, the caller synchronises
+__device__ __forceinline__ void fill_lut(uint4 *lut, const uint32_t t) {
+    if (t < 16) {
+        const uint32_t one = 0x3f800000u;
+        lut[t] = make_uint4((t & 1u) ? one : 0u, (t & 2u) ? one : 0u, (t & 4u) ? one : 0u, (t & 8u) ? one : 0u);
+    }
+}
+
 
 // Phases 1b and 2 of the observation build: `nch` per-agent bit strings of PB bits (stride AST words, in shared memory)
 // are compacted into one contiguous bit string `wb` and expanded into f32 (fmt OBS_F32) or bf16 (OBS_BF16) 0/1 values at

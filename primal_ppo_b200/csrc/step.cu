@@ -73,27 +73,14 @@ cudaError_t launch_step(const EnvView &v, const int8_t *actions, const int8_t *s
                         int mode, int *work_counter, cudaStream_t stream) {
     const int per_warp = (int)warp_smem_bytes(v.HP, v.RW, v.GS);
     const size_t smem = (size_t)per_warp * WARPS_PER_BLOCK;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const int need = (v.W + WARPS_PER_BLOCK - 1) / WARPS_PER_BLOCK;
-    const dim3 block(WARPS_PER_BLOCK * 32);
-    cudaError_t e = cudaSuccess;
-#define LAUNCH(M)                                                                                                  \
-    do {                                                                                                           \
-        e = cudaFuncSetAttribute(step_kernel<M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);          \
-        int per_sm = 1;                                                                                            \
-        if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, step_kernel<M>, WARPS_PER_BLOCK * 32, smem); \
-        if (per_sm < 1) per_sm = 1;                                                                                \
-        const int blocks = need < sms * per_sm ? need : sms * per_sm;                                              \
-        if (e == cudaSuccess) step_kernel<M><<<blocks, block, smem, stream>>>(v, actions, status_in, out, per_warp, work_counter); \
-    } while (0)
-    if (mode == MODE_EVALUATE) LAUNCH(MODE_EVALUATE);
-    else if (mode == MODE_JOINT) LAUNCH(MODE_JOINT);
-    else LAUNCH(MODE_FUSED);
-#undef LAUNCH
-    if (e != cudaSuccess) return e;
-    return cudaGetLastError();
+    auto launch = [&](auto kern) {
+        return launch_persistent(kern, WARPS_PER_BLOCK * 32, smem, need, INT_MAX, stream, v, actions, status_in, out, per_warp,
+                                 work_counter);
+    };
+    if (mode == MODE_EVALUATE) return launch(step_kernel<MODE_EVALUATE>);
+    if (mode == MODE_JOINT) return launch(step_kernel<MODE_JOINT>);
+    return launch(step_kernel<MODE_FUSED>);
 }
 
 }  // namespace mapf

@@ -44,10 +44,7 @@ step_observe_kernel(const EnvView v, const int8_t *__restrict__ actions, const M
     s.obits = m.obits;
     s.grid = m.grid;
     carve_step_scratch(s, base + step_off, G);
-    if (threadIdx.x < 16) {
-        const uint32_t one = 0x3f800000u, t = threadIdx.x;
-        lut[t] = make_uint4((t & 1u) ? one : 0u, (t & 2u) ? one : 0u, (t & 4u) ? one : 0u, (t & 8u) ? one : 0u);
-    }
+    fill_lut(lut, threadIdx.x);
     __syncthreads();
 
     // claim-then-load (see observe.cu).  ONE claim per warp hands out 32 / G consecutive worlds, one per lane group: the
@@ -101,60 +98,16 @@ step_observe_kernel(const EnvView v, const int8_t *__restrict__ actions, const M
     finish_work(work_counter, gridDim.x * (blockDim.x >> 5), lane);
 }
 
-template <int C_T, int F_T, bool VEC4, int MINB, int G, bool BITS>
-cudaError_t launch_tb(const EnvView &v, const int8_t *actions, const MapfStepOut &out, float *obs, float *vec,
-                      const ObsLayout &L, int *counter, cudaStream_t stream) {
-    constexpr int MPW = 32 / G;
-    const int step_off = (int)L.total;
-    const int per_group = step_off + (int)step_scratch_bytes(G);
-    const int wpb = WARPS_PER_BLOCK;
-    const size_t smem = (size_t)per_group * MPW * wpb;
-    if (smem > 227 * 1024) return cudaErrorInvalidConfiguration;
-    auto kern = step_observe_kernel<C_T, F_T, VEC4, MINB, G, BITS>;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    int dev = 0, sms = 148, per_sm = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, wpb * 32, smem);
-    if (per_sm < 1) per_sm = 1;
-    if (per_sm > MINB) per_sm = MINB;
-    const int need = (v.W + wpb * MPW - 1) / (wpb * MPW);
-    const int blocks = need < sms * per_sm ? need : sms * per_sm;
-    kern<<<blocks, wpb * 32, smem, stream>>>(v, actions, out, obs, vec, L, per_group, step_off, counter);
-    return cudaGetLastError();
-}
-
-// As in observe.cu fewer write streams help store-dominated worlds (>= 32 KB of observations each), but here the step
-// phase needs warps to hide behind: in-process A/B at 40x40x32: 2 / 3 / 4 CTAs per SM = 0.772 / 0.722 / 0.731 ms.  The
-// 3-CTA instantiation is also COMPILED for 3 CTAs (80 registers instead of 64, no spills): 0.706 vs 0.721 ms.
-template <int C_T, int F_T, bool VEC4, bool BITS = false>
-cudaError_t launch_t(const EnvView &v, const int8_t *actions, const MapfStepOut &out, float *obs, float *vec,
-                     const ObsLayout &L, int G, int *counter, cudaStream_t stream) {
-    const bool big = obs_world_bytes(L, v.N) >= 32768;
-    if (G == 8) return launch_tb<C_T, F_T, VEC4, 4, 8, BITS>(v, actions, out, obs, vec, L, counter, stream);
-    if (G == 16) return launch_tb<C_T, F_T, VEC4, 4, 16, BITS>(v, actions, out, obs, vec, L, counter, stream);
-    if (big) return launch_tb<C_T, F_T, VEC4, 3, 32, BITS>(v, actions, out, obs, vec, L, counter, stream);
-    return launch_tb<C_T, F_T, VEC4, 4, 32, BITS>(v, actions, out, obs, vec, L, counter, stream);
-}
-
 }  // namespace
-
-// chunk of agents handled per phase-1 pass of the observation build (same rule as launch_observe)
-static int obs_chunk(const EnvView &v) {
-    const int PB = v.C * v.F * v.F;
-    int CH = v.N < 32 ? v.N : 32;
-    while (CH > 4 && (size_t)CH * ((PB + 31) / 32 + 2) * 4 * 2 > 24 * 1024) CH >>= 1;
-    return CH;
-}
 
 // Lanes per world: the narrowest lane group that holds the agents (8 / 16 / 32), provided the worlds are small enough for
 // a warp to stage 32 / G of them (shared memory for at least three CTAs per SM) and below the store-dominated regime;
 // MAPF_DBG_FLAGS bit 28 keeps one world per warp (A/B runs).
 static int group_width(const EnvView &v, int fmt) {
-    if (v.N > 16 || (v.dbg_flags & (1 << 28)) || obs_chunk(v) < v.N) return 32;
+    const int CH = obs_chunk(v.N, v.C * v.F * v.F);
+    if (v.N > 16 || (v.dbg_flags & (1 << 28)) || CH < v.N) return 32;
     const int G = v.N <= 8 ? 8 : 16;
-    ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, obs_chunk(v), G);
+    ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, CH, G);
     L.fmt = fmt;
     if (obs_world_bytes(L, v.N) >= 32768) return 32;
     const size_t per_cta = (L.total + sw::step_scratch_bytes(G)) * (32 / G) * WARPS_PER_BLOCK;
@@ -166,34 +119,37 @@ static int group_width(const EnvView &v, int fmt) {
 // The fused kernel covers lane = agent worlds whose observation is built in one chunk (every training configuration);
 // anything else (N > 32, FOV 31 with 32 agents, ...) is served by the CTA-per-world fused kernel (step_observe_wide.cu).
 bool step_observe_fusable(const EnvView &v) {
-    if (v.N > 32 || obs_chunk(v) < v.N) return false;
-    const ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, obs_chunk(v));
+    const int CH = obs_chunk(v.N, v.C * v.F * v.F);
+    if (v.N > 32 || CH < v.N) return false;
+    const ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, CH);
     return (L.total + sw::step_scratch_bytes(32)) * WARPS_PER_BLOCK <= 200 * 1024;
 }
 
 cudaError_t launch_step_observe(const EnvView &v, const int8_t *actions, const MapfStepOut &out, float *obs, float *vec,
                                 int *work_counter, cudaStream_t stream, int fmt) {
-    const int PB = v.C * v.F * v.F;
-    const int CH = obs_chunk(v);
-    const int G = group_width(v, fmt);
+    const int PB = v.C * v.F * v.F, CH = obs_chunk(v.N, PB);
+    const int G = group_width(v, fmt), wpg = WARPS_PER_BLOCK * (32 / G);     // worlds per CTA
     ObsLayout L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, CH, G);
     L.fmt = fmt;
-    const bool vec4 = (fmt == OBS_BITS ? bits_words(L.PB) % 4 == 0 : ((size_t)v.N * PB) % (fmt == OBS_BF16 ? 8 : 4) == 0) &&
-                      (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
-    if (fmt == OBS_BITS) {
-        if (v.C == 6 && v.F == 9) {
-            return vec4 ? launch_t<6, 9, true, true>(v, actions, out, obs, vec, L, G, work_counter, stream)
-                        : launch_t<6, 9, false, true>(v, actions, out, obs, vec, L, G, work_counter, stream);
-        }
-        return vec4 ? launch_t<0, 0, true, true>(v, actions, out, obs, vec, L, G, work_counter, stream)
-                    : launch_t<0, 0, false, true>(v, actions, out, obs, vec, L, G, work_counter, stream);
-    }
-    if (v.C == 6 && v.F == 9) {
-        return vec4 ? launch_t<6, 9, true>(v, actions, out, obs, vec, L, G, work_counter, stream)
-                    : launch_t<6, 9, false>(v, actions, out, obs, vec, L, G, work_counter, stream);
-    }
-    return vec4 ? launch_t<0, 0, true>(v, actions, out, obs, vec, L, G, work_counter, stream)
-                : launch_t<0, 0, false>(v, actions, out, obs, vec, L, G, work_counter, stream);
+    const int step_off = (int)L.total, per_group = step_off + (int)step_scratch_bytes(G);
+    const size_t smem = (size_t)per_group * wpg;
+    if (smem > 227 * 1024) return cudaErrorInvalidConfiguration;
+    const int need = (v.W + wpg - 1) / wpg;
+    // As in observe.cu fewer write streams help store-dominated worlds (>= 32 KB of observations each), but here the step
+    // phase needs warps to hide behind: in-process A/B at 40x40x32: 2 / 3 / 4 CTAs per SM = 0.772 / 0.722 / 0.731 ms.  The
+    // 3-CTA instantiation is also COMPILED for 3 CTAs (80 registers instead of 64, no spills): 0.706 vs 0.721 ms.
+    const bool big = obs_world_bytes(L, v.N) >= 32768;
+    return dispatch_obs(fmt, v.C, v.F, obs_vec4(fmt, v.N, PB, CH, obs), [&](auto t) {
+        using T = decltype(t);
+        auto launch = [&](auto kern, int minb) {
+            return launch_persistent(kern, WARPS_PER_BLOCK * 32, smem, need, minb, stream, v, actions, out, obs, vec, L,
+                                     per_group, step_off, work_counter);
+        };
+        if (G == 8) return launch(step_observe_kernel<T::C_T, T::F_T, T::VEC4, 4, 8, T::BITS>, 4);
+        if (G == 16) return launch(step_observe_kernel<T::C_T, T::F_T, T::VEC4, 4, 16, T::BITS>, 4);
+        if (big) return launch(step_observe_kernel<T::C_T, T::F_T, T::VEC4, 3, 32, T::BITS>, 3);
+        return launch(step_observe_kernel<T::C_T, T::F_T, T::VEC4, 4, 32, T::BITS>, 4);
+    });
 }
 
 }  // namespace mapf

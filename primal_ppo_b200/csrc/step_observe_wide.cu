@@ -49,10 +49,7 @@ step_observe_wide_kernel(const EnvView v, const int8_t *__restrict__ actions, co
     s.obits = m.obits;
     s.grid = m.grid;
     carve_scratch(s, smem_raw + scratch_off);
-    if (tid < 16) {
-        const uint32_t one = 0x3f800000u, t = tid;
-        lut[t] = make_uint4((t & 1u) ? one : 0u, (t & 2u) ? one : 0u, (t & 4u) ? one : 0u, (t & 8u) ? one : 0u);
-    }
+    fill_lut(lut, tid);
     for (int k = tid; k < nob; k += blockDim.x) m.abits[k] = 0;
     for (int k = tid; k < (HP * GS) / 16; k += blockDim.x) reinterpret_cast<uint4 *>(m.grid)[k] = make_uint4(0, 0, 0, 0);
     const int nchunks = (N + L.CH - 1) / L.CH;
@@ -117,10 +114,9 @@ WidePlan make_plan(const EnvView &v, int fmt, int FW_WARPS) {
     const int PB = v.C * v.F * v.F;
     // chunk size: at least one chunk per warp when N allows it; per-warp scratch (aw + wb) small enough for six resident
     // CTAs (~36 KB each) while the chunk keeps at least 8 agents (phase 1 runs one lane per agent), 12 KB at most
-    const size_t staged = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, 8).off_goal + (((size_t)v.N * 8 + 15) / 16) * 16;
+    const size_t staged = cta_shared_bytes(make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, 8), v.N);
     size_t budget = staged < 36 * 1024 ? (36 * 1024 - staged) / FW_WARPS : 0;
     if (budget > 12 * 1024) budget = 12 * 1024;
-    auto per_warp_bytes = [&](int ch) { return (size_t)ch * ((PB + 31) / 32 + 2) * 4 * 2; };
     // Balanced chunks: with `r` rounds every warp builds r chunks of CH = ceil(N / (warps * r)) agents, rounded up so that a
     // chunk's block stays 16-byte aligned (vector stores); the smallest r whose scratch fits the budget wins.  (Power-of-two
     // chunks left 33 agents as 5 chunks of 8 on 4 warps — one warp with twice the work — and 48 agents as 6.)
@@ -133,20 +129,20 @@ WidePlan make_plan(const EnvView &v, int fmt, int FW_WARPS) {
         int ch = (v.N + FW_WARPS * r - 1) / (FW_WARPS * r);
         ch = (ch + mult - 1) / mult * mult;
         if (ch > 32) continue;
-        if (per_warp_bytes(ch) <= 12 * 1024 && (ch <= 8 || per_warp_bytes(ch) <= budget)) CH = ch;
+        if (chunk_scratch(ch, PB) <= 12 * 1024 && (ch <= 8 || chunk_scratch(ch, PB) <= budget)) CH = ch;
     }
     if (CH == 0) CH = mult <= 2 ? 2 : mult;
-    if (per_warp_bytes(CH) > 28 * 1024) return p;
+    if (chunk_scratch(CH, PB) > 28 * 1024) return p;
     p.L = make_layout(v.HP, v.RW, v.GS, v.N, v.C, v.F, CH);
     p.L.alias = 0;
     p.L.fmt = fmt;
     // [obits | abits | grid | goals + cells] shared by the CTA, then the per-warp observation scratch (aw, wb).  The step
     // phase's scratch is dead once the post-step cells / goals have been handed over, and the observation scratch is dead
     // during the step phase: they overlay each other (a __syncthreads separates the two uses).
-    p.shared_bytes = (int)(p.L.off_goal + (((size_t)v.N * 8 + 15) / 16) * 16);
+    p.shared_bytes = (int)cta_shared_bytes(p.L, v.N);
     p.scratch_off = p.shared_bytes;
-    p.per_warp = (int)((((size_t)CH * p.L.AST * 4 + 15) / 16) * 16 + (((size_t)p.L.WB * 4 + 15) / 16) * 16);
-    const size_t obs_scratch = (size_t)p.per_warp * FW_WARPS, step_scratch = al16(scratch_bytes());
+    p.per_warp = (int)warp_scratch_bytes(CH, PB);
+    const size_t obs_scratch = (size_t)p.per_warp * FW_WARPS, step_scratch = align16(scratch_bytes());
     p.smem = (size_t)p.shared_bytes + (obs_scratch > step_scratch ? obs_scratch : step_scratch);
     p.ok = p.smem <= 200 * 1024;
     return p;
@@ -182,42 +178,17 @@ cudaError_t launch_step_observe_wide(const EnvView &v, const int8_t *actions, co
     WidePlan p = make_plan(v, fmt, warps);
     if (!p.ok && warps != 8) { variant = 1; p = make_plan(v, fmt, 8); }
     if (!p.ok) return cudaErrorNotSupported;
-    const int PB = v.C * v.F * v.F;
-    const size_t al = fmt == OBS_BF16 ? 8 : 4;
-    const bool vec4 = (fmt == OBS_BITS ? bits_words(p.L.PB) % 4 == 0 : ((size_t)p.L.CH * PB) % al == 0 && ((size_t)v.N * PB) % al == 0) &&
-                      (reinterpret_cast<uintptr_t>(obs) & 15) == 0;
-    int dev = 0, sms = 148, per_sm = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    cudaError_t e;
-#define LAUNCH(WARPS_, MINB_, ...)                                                                                 \
-    do {                                                                                                           \
-        auto kern = step_observe_wide_kernel<__VA_ARGS__, WARPS_, MINB_>;                                          \
-        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem);                  \
-        if (e != cudaSuccess) return e;                                                                            \
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WARPS_ * 32, p.smem);                         \
-        if (per_sm < 1) per_sm = 1;                                                                                \
-        const int blocks = v.W < sms * per_sm ? v.W : sms * per_sm;                                                \
-        kern<<<blocks, WARPS_ * 32, p.smem, stream>>>(v, actions, out, obs, vec, p.L, p.shared_bytes, p.scratch_off, p.per_warp, \
-                                                      work_counter);                                               \
-    } while (0)
-#define LAUNCH_V(...)                                                                                              \
-    do {                                                                                                           \
-        if (variant == 1) LAUNCH(8, 3, __VA_ARGS__);                                                               \
-        else if (variant == 2) LAUNCH(4, 6, __VA_ARGS__);                                                          \
-        else if (variant == 4) LAUNCH(2, 16, __VA_ARGS__);                                                         \
-        else LAUNCH(4, 8, __VA_ARGS__);                                                                            \
-    } while (0)
-    if (fmt == OBS_BITS) {
-        if (v.C == 6 && v.F == 9) { if (vec4) LAUNCH_V(6, 9, true, true); else LAUNCH_V(6, 9, false, true); }
-        else { if (vec4) LAUNCH_V(0, 0, true, true); else LAUNCH_V(0, 0, false, true); }
-    } else {
-        if (v.C == 6 && v.F == 9) { if (vec4) LAUNCH_V(6, 9, true, false); else LAUNCH_V(6, 9, false, false); }
-        else { if (vec4) LAUNCH_V(0, 0, true, false); else LAUNCH_V(0, 0, false, false); }
-    }
-#undef LAUNCH_V
-#undef LAUNCH
-    return cudaGetLastError();
+    return dispatch_obs(fmt, v.C, v.F, obs_vec4(fmt, v.N, p.L.PB, p.L.CH, obs), [&](auto t) {
+        using T = decltype(t);
+        auto launch = [&](auto kern, int cta_warps) {
+            return launch_persistent(kern, cta_warps * 32, p.smem, v.W, INT_MAX, stream, v, actions, out, obs, vec, p.L,
+                                     p.shared_bytes, p.scratch_off, p.per_warp, work_counter);
+        };
+        if (variant == 1) return launch(step_observe_wide_kernel<T::C_T, T::F_T, T::VEC4, T::BITS, 8, 3>, 8);
+        if (variant == 2) return launch(step_observe_wide_kernel<T::C_T, T::F_T, T::VEC4, T::BITS, 4, 6>, 4);
+        if (variant == 4) return launch(step_observe_wide_kernel<T::C_T, T::F_T, T::VEC4, T::BITS, 2, 16>, 2);
+        return launch(step_observe_wide_kernel<T::C_T, T::F_T, T::VEC4, T::BITS, 4, 8>, 4);
+    });
 }
 
 }  // namespace mapf

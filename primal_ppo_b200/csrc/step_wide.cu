@@ -14,7 +14,7 @@ using namespace sww;
 constexpr int WIDE_WARPS = 4;
 
 __host__ __device__ inline size_t wide_bytes(int HP, int RW, int GS) {
-    return al16((size_t)HP * RW * 4) + al16((size_t)HP * GS) + scratch_bytes();
+    return align16((size_t)HP * RW * 4) + align16((size_t)HP * GS) + scratch_bytes();
 }
 
 template <int MODE>
@@ -28,8 +28,8 @@ step_wide_kernel(const EnvView v, const int8_t *__restrict__ actions, const int8
     const int HP = v.HP, RW = v.RW, GS = v.GS;
     unsigned char *b = smem_raw + (size_t)warp * per_warp;
     WideSmem s;
-    s.obits = reinterpret_cast<uint32_t *>(b); b += al16((size_t)HP * RW * 4);
-    s.grid = b; b += al16((size_t)HP * GS);
+    s.obits = reinterpret_cast<uint32_t *>(b); b += align16((size_t)HP * RW * 4);
+    s.grid = b; b += align16((size_t)HP * GS);
     carve_scratch(s, b);
     expand_obstacle_rows(s.obits, v.obst_pack + (size_t)w * v.PW, v, lane, 32);
     uint4 *g4 = reinterpret_cast<uint4 *>(s.grid);

@@ -15,8 +15,6 @@ namespace sww {
 
 constexpr int NMAX = 128;
 
-__host__ __device__ inline size_t al16(size_t x) { return (x + 15) & ~(size_t)15; }
-
 enum { K_SHADOW = 0, K_C1, K_C2, K_C3, K_ARR, K_VIOL, K_FIX, K_TRIG, K_ERR, K_COUNT = 12 };
 
 struct WideSmem {

@@ -24,8 +24,6 @@ struct WarpSmem {
     int8_t *queue;     // [2G] problemAgents (ring buffer)
 };
 
-__host__ __device__ inline size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
-
 // scratch of the step phase for one group of G lanes (everything but obits / grid)
 __host__ __device__ inline size_t step_scratch_bytes(int G) { return align16((size_t)G * 5 * 4 + G * 4 + 5 * G + 2 * G); }
 
