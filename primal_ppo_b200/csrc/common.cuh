@@ -79,6 +79,7 @@ struct EnvView {
     int16_t *hnx;       // [W,4] the entry of the following tick (wrapped), so that a step has no dependent loads
     uint32_t *err;
     long long *counters;
+    int *order;         // [1] walk direction of the next world-claiming launch (see world_of)
 };
 
 __device__ __forceinline__ int dr_of(int a) { return (a == 2) - (a == 4); }   // mapf_gym.py:97
@@ -93,32 +94,84 @@ __device__ __forceinline__ uint32_t row_window(const uint32_t *row, int off, int
 }
 __device__ __forceinline__ uint32_t row_bit(const uint32_t *row, int off) { return (row[off >> 5] >> (off & 31)) & 1u; }
 
+// L2 residency rule.  The env state (cells, goals, obstacle bit rows, human tick: ~55 MB for 65 536 worlds) is re-read
+// every step while 4 GB of observations stream through the same L2.  DRAM reads interleaved with the write stream cost
+// far more than their bytes (read/write bus turnarounds: measured -13 % write bandwidth for 1.6 % read bytes), so:
+//   - env state that the next step reads is loaded AND stored with the evict_last policy (ld_keep* / st_keep*):
+//     pos, goal, rep, obst_pack, htick, hcur, hnx, nstep, hlen, counters and the htrace lookahead entry;
+//   - everything a step only produces is stored evict-first (st.global.cs, st_stream*): the observations, vec, the
+//     MapfStepOut fields (incl. the trainValid rows and the packed host slab), so that it does not compete with the state.
+// Rare-path accesses (err, qcur / goal_queue on arrival, tape, dims) stay plain.
+__device__ __forceinline__ uint64_t policy_evict_last() {
+    uint64_t p;
+    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
+    return p;
+}
+__device__ __forceinline__ uint32_t ld_keep(const void *p, uint64_t pol) {
+    uint32_t v;
+    asm volatile("ld.global.L2::cache_hint.b32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
+    return v;
+}
+__device__ __forceinline__ int ld_keep_s8(const void *p, uint64_t pol) {
+    int v;
+    asm volatile("ld.global.L2::cache_hint.s8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
+    return v;
+}
+__device__ __forceinline__ int2 ld_keep_v2(const void *p, uint64_t pol) {
+    int2 v;
+    asm volatile("ld.global.L2::cache_hint.v2.b32 {%0, %1}, [%2], %3;" : "=r"(v.x), "=r"(v.y) : "l"(p), "l"(pol));
+    return v;
+}
+__device__ __forceinline__ void st_keep(void *p, uint32_t v, uint64_t pol) {
+    asm volatile("st.global.L2::cache_hint.b32 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(pol) : "memory");
+}
+__device__ __forceinline__ void st_keep_s8(void *p, int v, uint64_t pol) {
+    asm volatile("st.global.L2::cache_hint.b8 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(pol) : "memory");
+}
+__device__ __forceinline__ void st_keep_v2(void *p, int2 v, uint64_t pol) {
+    asm volatile("st.global.L2::cache_hint.v2.b32 [%0], {%1, %2}, %3;" ::"l"(p), "r"(v.x), "r"(v.y), "l"(pol) : "memory");
+}
+// *p += x for state only this thread touches (the per-world counters)
+__device__ __forceinline__ void add_keep_s64(long long *p, long long x, uint64_t pol) {
+    long long v;
+    asm volatile("ld.global.L2::cache_hint.b64 %0, [%1], %2;" : "=l"(v) : "l"(p), "l"(pol));
+    asm volatile("st.global.L2::cache_hint.b64 [%0], %1, %2;" ::"l"(p), "l"(v + x), "l"(pol) : "memory");
+}
+__device__ __forceinline__ void add_keep_s32(int32_t *p, int x, uint64_t pol) { st_keep(p, ld_keep(p, pol) + x, pol); }
+
 // ---- packed obstacle bit matrix -> padded bit rows ---------------------------------------------------------------
-// bits [off, off + n), n <= 32, of a packed bit array of `nwords` words
-__device__ __forceinline__ uint32_t pack_extract(const uint32_t *p, int off, int n, int nwords) {
+// bits [off, off + n), n <= 32, of a packed bit array of `nwords` words; KEEP: `p` is the env's obst_pack in global
+// memory, read with the evict_last policy `pol` (residency rule above), else shared memory
+template <bool KEEP>
+__device__ __forceinline__ uint32_t pack_extract(const uint32_t *p, int off, int n, int nwords, uint64_t pol) {
     const int k = off >> 5;
-    const uint32_t lo = p[k], hi = (k + 1 < nwords) ? p[k + 1] : 0u;
+    const uint32_t lo = KEEP ? ld_keep(p + k, pol) : p[k];
+    const uint32_t hi = (k + 1 < nwords) ? (KEEP ? ld_keep(p + k + 1, pol) : p[k + 1]) : 0u;
     const uint32_t x = __funnelshift_r(lo, hi, off & 31);
     return n >= 32 ? x : (x & ((1u << n) - 1u));
 }
 // word q of padded row pr: 1 = obstacle or out of bounds
-__device__ __forceinline__ uint32_t padded_row_word(const uint32_t *packed, int H, int Wd, int P, int PW, int pr, int q) {
+template <bool KEEP>
+__device__ __forceinline__ uint32_t padded_row_word(const uint32_t *packed, int H, int Wd, int P, int PW, int pr, int q,
+                                                    uint64_t pol) {
     const int r = pr - P;
     if (r < 0 || r >= H) return 0xffffffffu;
     const int c0 = 32 * q - P;                                   // column held by bit 0 of this word
     const int lo = c0 > 0 ? c0 : 0, hi = c0 + 32 < Wd ? c0 + 32 : Wd;
     if (hi <= lo) return 0xffffffffu;
     const int n = hi - lo, sh = lo - c0;
-    const uint32_t bits = pack_extract(packed, r * Wd + lo, n, PW);
+    const uint32_t bits = pack_extract<KEEP>(packed, r * Wd + lo, n, PW, pol);
     const uint32_t mask = (n >= 32 ? 0xffffffffu : ((1u << n) - 1u)) << sh;
     return (bits << sh) | ~mask;
 }
-// all `nthreads` threads of a warp / CTA expand one world (packed may live in shared or global memory)
-__device__ __forceinline__ void expand_obstacle_rows(uint32_t *obits, const uint32_t *packed, const EnvView &v, int tid, int nthreads) {
+// all `nthreads` threads of a warp / CTA expand one world (packed lives in shared memory, or with KEEP in global memory)
+template <bool KEEP = false>
+__device__ __forceinline__ void expand_obstacle_rows(uint32_t *obits, const uint32_t *packed, const EnvView &v, int tid, int nthreads,
+                                                     uint64_t pol = 0) {
     const int nob = v.HP * v.RW;
     for (int k = tid; k < nob; k += nthreads) {
         const int pr = k / v.RW;
-        obits[k] = padded_row_word(packed, v.H, v.Wd, v.P, v.PW, pr, k - pr * v.RW);
+        obits[k] = padded_row_word<KEEP>(packed, v.H, v.Wd, v.P, v.PW, pr, k - pr * v.RW, pol);
     }
 }
 
@@ -164,49 +217,25 @@ __device__ __forceinline__ uint32_t goal_candidate(unsigned long long seed, uint
 }
 constexpr int GOAL_DRAW_CAP = 4096;   // draws per arrival before MAPF_ERR_NO_FREE_CELL (the reference would spin for ever)
 
-// L2 residency hints.  The env state (cells, goals, obstacle bit rows, human tick: ~55 MB for 65 536 worlds) is re-read
-// every step while 4 GB of observations stream through the same L2.  DRAM reads interleaved with the write stream cost
-// far more than their bytes (read/write bus turnarounds: measured -13 % write bandwidth for 1.6 % read bytes), so state
-// is loaded and stored with an evict_last policy and stays L2-resident across steps; observations are evict-first.
-__device__ __forceinline__ uint64_t policy_evict_last() {
-    uint64_t p;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-    return p;
-}
-__device__ __forceinline__ uint32_t ld_keep(const void *p, uint64_t pol) {
-    uint32_t v;
-    asm volatile("ld.global.L2::cache_hint.b32 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
-    return v;
-}
-__device__ __forceinline__ int ld_keep_s8(const void *p, uint64_t pol) {
-    int v;
-    asm volatile("ld.global.L2::cache_hint.s8 %0, [%1], %2;" : "=r"(v) : "l"(p), "l"(pol));
-    return v;
-}
-__device__ __forceinline__ int2 ld_keep_v2(const void *p, uint64_t pol) {
-    int2 v;
-    asm volatile("ld.global.L2::cache_hint.v2.b32 {%0, %1}, [%2], %3;" : "=r"(v.x), "=r"(v.y) : "l"(p), "l"(pol));
-    return v;
-}
-__device__ __forceinline__ void st_keep(void *p, uint32_t v, uint64_t pol) {
-    asm volatile("st.global.L2::cache_hint.b32 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void st_keep_s8(void *p, int v, uint64_t pol) {
-    asm volatile("st.global.L2::cache_hint.b8 [%0], %1, %2;" ::"l"(p), "r"(v), "l"(pol) : "memory");
-}
-__device__ __forceinline__ void st_keep_v2(void *p, int2 v, uint64_t pol) {
-    asm volatile("st.global.L2::cache_hint.v2.b32 [%0], {%1, %2}, %3;" ::"l"(p), "r"(v.x), "r"(v.y), "l"(pol) : "memory");
-}
-
 // Bulk L2 prefetch of a contiguous range (TMA unit, no registers, no completion to wait for).
 __device__ __forceinline__ void prefetch_l2_bulk(const void *p, size_t bytes, uint64_t pol) {
     bytes &= ~(size_t)15;
     if (bytes) asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(p), "r"((uint32_t)bytes), "l"(pol) : "memory");
 }
 
-// streaming 16-byte store: observations are written once and consumed by another kernel much later
+// streaming stores: step outputs and observations are written once and consumed by another kernel much later
 __device__ __forceinline__ void st_stream_v4(float *p, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
     asm volatile("st.global.cs.v4.b32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
+}
+__device__ __forceinline__ void st_stream(void *p, uint32_t v) {
+    asm volatile("st.global.cs.b32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+__device__ __forceinline__ void st_stream(float *p, float v) { st_stream(static_cast<void *>(p), __float_as_uint(v)); }
+__device__ __forceinline__ void st_stream_u16(void *p, uint32_t v) {
+    asm volatile("st.global.cs.b16 [%0], %1;" ::"l"(p), "h"((unsigned short)v) : "memory");
+}
+__device__ __forceinline__ void st_stream_u8(void *p, uint32_t v) {
+    asm volatile("st.global.cs.b8 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
 
 // Dynamic work distribution for the persistent kernels: counter[0] = next unit, counter[1] = warps that are done.
@@ -216,12 +245,27 @@ __device__ __forceinline__ int claim_work(int *counter, int n, int lane) {
     if (lane == 0) t = atomicAdd(counter, n);
     return __shfl_sync(FULL, t, 0);
 }
-__device__ __forceinline__ void finish_work(int *counter, int total_warps, int lane) {
+// `order`: the env's walk-direction word (world-claiming kernels), flipped by the last warp; every other warp has read it
+// before its first claim, so the flip takes effect at the next launch.
+__device__ __forceinline__ void finish_work(int *counter, int total_warps, int lane, int *order = nullptr) {
     if (lane == 0) {
         const int d = atomicAdd(counter + 1, 1);
-        if (d == total_warps - 1) { counter[0] = 0; counter[1] = 0; }
+        if (d == total_warps - 1) {
+            counter[0] = 0; counter[1] = 0;
+            if (order) *order ^= 1;
+        }
     }
 }
+
+// World order of the world-claiming persistent kernels (step, observe, step_observe, observe_wide, step_observe_wide):
+// serpentine.  Claims stay in claim space 0, 1, ...; a launch maps claim c to world c or W-1-c, and every launch reverses
+// the direction of the one before.  Worlds are independent, so no result depends on the order, but the state a launch
+// touched last is L2-resident and is what the next launch reads first (an ascending walk every time starts from the world
+// touched longest ago, with ~4 GB of observation stores since).  The direction is a device word, so a captured or
+// replayed launch sequence alternates too.  A claim c >= W stays c (no world).
+constexpr int DBG_ASCENDING = 1 << 12;     // MAPF_DBG_FLAGS bit 12: ascending order every launch (A/B runs)
+__device__ __forceinline__ int walk_dir(const EnvView &v) { return (v.dbg_flags & DBG_ASCENDING) ? 0 : *v.order; }
+__device__ __forceinline__ int world_of(const EnvView &v, int c, int dir) { return (dir && c < v.W) ? v.W - 1 - c : c; }
 
 // Launch of a persistent kernel: as many CTAs as are resident at once on the current device (at most max_per_sm per SM)
 // and no more than need_blocks.  A failed runtime call is returned and nothing is launched.
@@ -243,14 +287,17 @@ cudaError_t launch_persistent(void (*kern)(P...), int threads, size_t smem, long
 // Batched state prefetch.  A world's state is ~0.9 KB spread over a dozen SoA arrays; loaded world by world it reaches
 // DRAM as ~430 000 isolated 128-byte reads per step, interleaved with 4 GB of observation stores — and every isolated
 // read costs the HBM channel a write->read->write bus turnaround (measured: 1.6 % read bytes cost 13 % of the write
-// bandwidth).  Worlds are claimed in increasing order, so the warp that starts loading world w1 with w1 % PFB == 0 asks
-// the TMA unit to pull the state of worlds [w1 + ahead, w1 + ahead + PFB) into L2 as a few large contiguous reads; the
-// per-world register loads that follow a few microseconds later then hit L2.
+// bandwidth).  Claims are handed out in increasing order, so the warp that claims c1 with c1 % PFB == 0 asks the TMA unit
+// to pull the state of the worlds of claims [c1 + ahead, c1 + ahead + PFB) (in the launch's direction `dir`, world_of)
+// into L2 as a few large contiguous reads; the per-world register loads that follow a few microseconds later then hit L2.
 constexpr int PFB = 256;
 __device__ __forceinline__ int prefetch_batch(const EnvView &v) { return PFB << ((v.dbg_flags >> 8) & 7); }
-__device__ __forceinline__ void prefetch_world_batch(const EnvView &v, const int8_t *actions, int w0, uint64_t pol, int batch = 0) {
-    if (w0 >= v.W) return;
-    const size_t n = (size_t)min(batch > 0 ? batch : prefetch_batch(v), v.W - w0), wn = (size_t)w0 * v.N, nn = n * v.N;
+__device__ __forceinline__ void prefetch_world_batch(const EnvView &v, const int8_t *actions, int c0, int dir, uint64_t pol,
+                                                     int batch = 0) {
+    if (c0 >= v.W) return;
+    const int nb = min(batch > 0 ? batch : prefetch_batch(v), v.W - c0);
+    const int w0 = dir ? v.W - c0 - nb : c0;             // lowest world of the batch
+    const size_t n = (size_t)nb, wn = (size_t)w0 * v.N, nn = n * v.N;
     prefetch_l2_bulk(v.obst_pack + (size_t)w0 * v.PW, n * v.PW * 4, pol);
     prefetch_l2_bulk(reinterpret_cast<const uint32_t *>(v.pos) + wn, nn * 4, pol);
     prefetch_l2_bulk(reinterpret_cast<const uint32_t *>(v.goal) + wn, nn * 4, pol);

@@ -13,6 +13,8 @@ using namespace mapf;
 // work counters (2 ints each) of the persistent kernels: one per kernel family, so that a launch that aborted, or two
 // families in flight on different streams, can never hand a stale counter to another kernel
 enum { WC_STEP = 0, WC_OBSERVE = 1, WC_FUSED = 2, WC_BFS = 3, WC_FUSED_WIDE = 4, WC_COUNT = 8 };
+// ... followed by the walk-direction word shared by all world-claiming families (EnvView::order, common.cuh world_of)
+constexpr size_t WORK_BYTES = (WC_COUNT * 2 + 1) * sizeof(int);
 
 struct MapfEnv {
     MapfConfig cfg;
@@ -20,7 +22,7 @@ struct MapfEnv {
     bool has_scenario;
     // arrivals compaction scratch for mapf_bfs_refresh
     int32_t *d_list, *d_count;
-    int *d_work;   // [WC_COUNT][2] dynamic-scheduling counters
+    int *d_work;   // [WC_COUNT][2] dynamic-scheduling counters, then the walk direction
     // ---- staging of the *_host entry points (allocated by mapf_create) --------------------------------------------------
     // two result slots (layout: MapfHostLayout without train_valid) and two action buffers, used alternately
     unsigned char *d_slot[2];
@@ -167,7 +169,7 @@ int mapf_create(const MapfConfig *cfg, MapfEnv **out) {
     alloc((void **)&v.counters, W * 6 * 8);
     alloc((void **)&v.hcur, W * 8);
     alloc((void **)&v.hnx, W * 8);
-    alloc((void **)&e->d_work, WC_COUNT * 2 * sizeof(int));
+    alloc((void **)&e->d_work, WORK_BYTES);
     alloc((void **)&e->d_list, WN * 4);
     alloc((void **)&e->d_count, 4);
     // result-slot layout: f32 fields first, then the byte fields; every field 256-byte aligned
@@ -203,7 +205,8 @@ int mapf_create(const MapfConfig *cfg, MapfEnv **out) {
         if (err == cudaSuccess) err = cudaEventCreateWithFlags(&e->ev_h2d[k], cudaEventDisableTiming);
     }
     if (err != cudaSuccess) { mapf_destroy(e); return cuda_fail(err, "mapf_create: allocation"); }
-    cudaMemset(e->d_work, 0, WC_COUNT * 2 * sizeof(int));
+    cudaMemset(e->d_work, 0, WORK_BYTES);
+    v.order = e->d_work + WC_COUNT * 2;
     if (const char *f = getenv("MAPF_DBG_FLAGS")) v.dbg_flags = atoi(f);
     *out = e;
     return MAPF_OK;
@@ -238,7 +241,7 @@ int mapf_reset(MapfEnv *e, const MapfScenario *sc, void *stream) {
     v.hp5 = sc->hp5; v.tape = sc->tape; v.tape_len = sc->tape_len; v.dims = sc->dims;
     ON_DEVICE(e->cfg.device);
     // re-arm every work counter: a launch that faulted or was aborted must not leave later launches without work
-    CU(cudaMemsetAsync(e->d_work, 0, WC_COUNT * 2 * sizeof(int), (cudaStream_t)stream));
+    CU(cudaMemsetAsync(e->d_work, 0, WORK_BYTES, (cudaStream_t)stream));
     CU(launch_reset(v, (cudaStream_t)stream));
     e->has_scenario = true;
     return MAPF_OK;

@@ -40,20 +40,22 @@ observe_kernel(const EnvView v, float *__restrict__ obs, float *__restrict__ vec
     __syncthreads();
 
     // dynamic world scheduling: w (inputs in registers) is processed while w1, claimed at the top of the iteration, is
-    // being loaded.  Claim and load are adjacent in time so that worlds are LOADED in (nearly) index order, which is
+    // being loaded.  Claim and load are adjacent in time so that worlds are LOADED in (nearly) claim order, which is
     // what lets the batched L2 prefetch run a fixed distance ahead of the loads.
-    int w = claim_work(work_counter, 1, lane);
+    const int dir = walk_dir(v);
+    int w = world_of(v, claim_work(work_counter, 1, lane), dir);
     const uint64_t pol = policy_evict_last();
-    const int pf_ahead = prefetch_ahead(v), pf_batch = prefetch_batch(v);
     WorldRegs cur, nxt;
     load_world(v, w, lane, npw, pol, cur);
     const bool direct_ob = npw > OBW * 32;
     bool first = true;
 
     while (w < v.W) {
-        const int w1 = claim_work(work_counter, 1, lane);
+        const int c1 = claim_work(work_counter, 1, lane), w1 = world_of(v, c1, dir);
         load_world(v, w1, lane, npw, pol, nxt);                  // in flight while this world is processed
-        if (lane == 0 && pf_ahead >= 0 && (w1 & (pf_batch - 1)) == 0) prefetch_world_batch(v, nullptr, w1 + pf_ahead, pol);
+        // (the prefetch distance and batch are re-read from the kernel parameters: no registers held across the loop)
+        if (lane == 0 && prefetch_ahead(v) >= 0 && (c1 & (prefetch_batch(v) - 1)) == 0)
+            prefetch_world_batch(v, nullptr, c1 + prefetch_ahead(v), dir, pol);
 
         // ---- stage: packed obstacle words (registers -> scratch in the agent-presence rows -> padded rows), then clean
         //      agent rows / id grid
@@ -63,7 +65,7 @@ observe_kernel(const EnvView v, float *__restrict__ obs, float *__restrict__ vec
             __syncwarp();
             expand_obstacle_rows(obits, abits, v, lane, 32);
         } else {
-            expand_obstacle_rows(obits, v.obst_pack + (size_t)w * npw, v, lane, 32);
+            expand_obstacle_rows<true>(obits, v.obst_pack + (size_t)w * npw, v, lane, 32, pol);
         }
         __syncwarp();
         for (int k = lane; k < nob; k += 32) abits[k] = 0;
@@ -78,7 +80,7 @@ observe_kernel(const EnvView v, float *__restrict__ obs, float *__restrict__ vec
         w = w1;
         cur = nxt;
     }
-    finish_work(work_counter, gridDim.x * (blockDim.x >> 5), lane);
+    finish_work(work_counter, gridDim.x * (blockDim.x >> 5), lane, v.order);
 }
 
 }  // namespace

@@ -42,25 +42,27 @@ observe_wide_kernel(const EnvView v, float *__restrict__ obs, float *__restrict_
     for (int k = tid; k < nob; k += blockDim.x) m.abits[k] = 0;
     for (int k = tid; k < (HP * GS) / 16; k += blockDim.x) reinterpret_cast<uint4 *>(m.grid)[k] = make_uint4(0, 0, 0, 0);
     const int nchunks = (N + L.CH - 1) / L.CH;
+    const uint64_t pol = policy_evict_last();
+    const int dir = tid == 0 ? walk_dir(v) : 0;           // serpentine order (common.cuh world_of)
     for (;;) {
         __syncthreads();                                   // previous world fully written, scratch clean
-        if (tid == 0) s_world = atomicAdd(work_counter, 1);
+        if (tid == 0) s_world = world_of(v, atomicAdd(work_counter, 1), dir);
         __syncthreads();
         const int w = s_world;
         if (w >= v.W) break;
         // ---- stage the world once for the CTA ---------------------------------------------------------------------
-        expand_obstacle_rows(m.obits, v.obst_pack + (size_t)w * v.PW, v, tid, blockDim.x);
+        expand_obstacle_rows<true>(m.obits, v.obst_pack + (size_t)w * v.PW, v, tid, blockDim.x, pol);
         const uint32_t *posw = reinterpret_cast<const uint32_t *>(v.pos) + (size_t)w * N;
         const uint32_t *goalw = reinterpret_cast<const uint32_t *>(v.goal) + (size_t)w * N;
         for (int i = tid; i < N; i += blockDim.x) {
-            const uint32_t pw = __ldg(posw + i);
+            const uint32_t pw = ld_keep(posw + i, pol);
             const int r = (int16_t)(pw & 0xffff), c = (int16_t)(pw >> 16);
             m.grid[(r + P) * GS + c + P] = (uint8_t)(i + 1);
             atomicOr(&m.abits[(r + P) * RW + ((c + P) >> 5)], 1u << ((c + P) & 31));
-            m.sgoal[i] = __ldg(goalw + i);
+            m.sgoal[i] = ld_keep(goalw + i, pol);
             m.spos[i] = pw;
         }
-        const int2 ht = __ldg(reinterpret_cast<const int2 *>(v.hcur) + w);
+        const int2 ht = ld_keep_v2(reinterpret_cast<const int2 *>(v.hcur) + w, pol);
         const int nr = (int16_t)(ht.y & 0xffff), nc = (int16_t)((uint32_t)ht.y >> 16);            // human.getNextPos()
         int rows = v.H, cols = v.Wd;
         if (v.use_da | v.use_hp) { if (v.dims) { rows = v.dims[2 * w]; cols = v.dims[2 * w + 1]; } }
@@ -80,10 +82,7 @@ observe_wide_kernel(const EnvView v, float *__restrict__ obs, float *__restrict_
         }
     }
     __syncthreads();
-    if (tid == 0) {                                        // the last CTA to finish re-arms the counter
-        const int d = atomicAdd(work_counter + 1, 1);
-        if (d == (int)gridDim.x - 1) { work_counter[0] = 0; work_counter[1] = 0; }
-    }
+    finish_work(work_counter, gridDim.x, tid, v.order);   // the last CTA to finish re-arms the counter, flips the direction
 }
 
 }  // namespace

@@ -339,7 +339,7 @@ __device__ __forceinline__ void observe_chunk(const EnvView &v, const ObsLayout 
             o4.y = (float)(d != 0.0 ? dy_ / d : dy_);
             o4.z = (float)d;
             o4.w = 0.0f;
-            reinterpret_cast<float4 *>(vec)[(size_t)w * N + i] = o4;
+            st_stream_v4(vec + ((size_t)w * N + i) * 4, __float_as_uint(o4.x), __float_as_uint(o4.y), __float_as_uint(o4.z), __float_as_uint(o4.w));
         }
         g.sync();
         if (BITS) {

@@ -41,22 +41,24 @@ step_kernel(const EnvView v, const int8_t *__restrict__ actions, const int8_t *_
         uint4 *g4 = reinterpret_cast<uint4 *>(s.grid);
         for (int k = lane; k < (HP * GS) / 16; k += 32) g4[k] = make_uint4(0, 0, 0, 0);
     }
-    int w = claim_work(work_counter, 1, lane);      // claim-then-load: see observe.cu
+    const int dir = walk_dir(v);
+    int w = world_of(v, claim_work(work_counter, 1, lane), dir);      // claim-then-load: see observe.cu
     const uint64_t pol = policy_evict_last();
-    const int pf_ahead = prefetch_ahead(v), pf_batch = prefetch_batch(v);
     StepRegs cur, nxt;
     load_step_world<MODE>(v, actions, status_in, w, lane, npw, pol, cur);
     const bool direct_ob = npw > SOBW * 32;
     while (w < v.W) {
-        const int w1 = claim_work(work_counter, 1, lane);
+        const int c1 = claim_work(work_counter, 1, lane), w1 = world_of(v, c1, dir);
         load_step_world<MODE>(v, actions, status_in, w1, lane, npw, pol, nxt);
-        if (lane == 0 && pf_ahead >= 0 && (w1 & (pf_batch - 1)) == 0) prefetch_world_batch(v, actions, w1 + pf_ahead, pol);
+        // (the prefetch distance and batch are re-read from the kernel parameters: no registers held across the loop)
+        if (lane == 0 && prefetch_ahead(v) >= 0 && (c1 & (prefetch_batch(v) - 1)) == 0)
+            prefetch_world_batch(v, actions, c1 + prefetch_ahead(v), dir, pol);
         if (!direct_ob) {                       // the packed obstacle words are probed directly (resolve_world<.., true>)
 #pragma unroll
             for (int k = 0; k < SOBW; ++k) if (k * 32 + lane < npw) s.obits[k * 32 + lane] = cur.ob[k];
         } else {
             const uint32_t *src = v.obst_pack + (size_t)w * npw;
-            for (int k = lane; k < npw; k += 32) s.obits[k] = __ldg(src + k);
+            for (int k = lane; k < npw; k += 32) s.obits[k] = ld_keep(src + k, pol);
         }
         uint32_t new_pw, new_gw;
         resolve_world<MODE, true>(v, out, s, w, Grp<32>(lane), cur, pol, new_pw, new_gw);
@@ -64,7 +66,7 @@ step_kernel(const EnvView v, const int8_t *__restrict__ actions, const int8_t *_
         w = w1;
         cur = nxt;
     }
-    finish_work(work_counter, gridDim.x * (blockDim.x >> 5), lane);
+    finish_work(work_counter, gridDim.x * (blockDim.x >> 5), lane, v.order);
 }
 
 }  // namespace

@@ -51,10 +51,11 @@ step_observe_kernel(const EnvView v, const int8_t *__restrict__ actions, const M
     // groups of a warp start every world together and stay converged through the common path, so an instruction issues
     // once for all of them (groups that drift apart would each issue their own copy with G lanes active); only the rare
     // data-dependent sections (sequential status replay, fixActions queue, goal draws) run per group, under group masks.
+    // Worlds are claimed in claim space (wb) and mapped to worlds in the launch's direction (serpentine order, world_of).
+    const int dir = walk_dir(v);
     int wb = claim_work(work_counter, MPW, lane);
-    int w = wb + grp;
+    int w = world_of(v, wb + grp, dir);
     const uint64_t pol = policy_evict_last();
-    const int pf_ahead = prefetch_ahead(v), pf_batch = prefetch_batch(v);
     StepRegs cur, nxt;
     load_step_world<MODE_FUSED, G>(v, actions, nullptr, w, gl, npw, pol, cur);
     const bool direct_ob = npw > SOBW * G;
@@ -62,9 +63,11 @@ step_observe_kernel(const EnvView v, const int8_t *__restrict__ actions, const M
 
     while (wb < v.W) {
         const int wb1 = claim_work(work_counter, MPW, lane);
-        const int w1 = wb1 + grp;
+        const int w1 = world_of(v, wb1 + grp, dir);
         load_step_world<MODE_FUSED, G>(v, actions, nullptr, w1, gl, npw, pol, nxt);   // in flight during this world
-        if (lane == 0 && pf_ahead >= 0 && (wb1 & (pf_batch - 1)) == 0) prefetch_world_batch(v, actions, wb1 + pf_ahead, pol);
+        // (the prefetch distance and batch are re-read from the kernel parameters: no registers held across the loop)
+        if (lane == 0 && prefetch_ahead(v) >= 0 && (wb1 & (prefetch_batch(v) - 1)) == 0)
+            prefetch_world_batch(v, actions, wb1 + prefetch_ahead(v), dir, pol);
 
         if (w < v.W) {
             // packed obstacle words: registers -> scratch (the agent-presence rows, zeroed right after) -> padded rows
@@ -74,7 +77,7 @@ step_observe_kernel(const EnvView v, const int8_t *__restrict__ actions, const M
                 g.sync();
                 expand_obstacle_rows(m.obits, m.abits, v, gl, G);
             } else {
-                expand_obstacle_rows(m.obits, v.obst_pack + (size_t)w * npw, v, gl, G);
+                expand_obstacle_rows<true>(m.obits, v.obst_pack + (size_t)w * npw, v, gl, G, pol);
             }
             g.sync();
             for (int k = gl; k < nob; k += G) m.abits[k] = 0;
@@ -95,7 +98,7 @@ step_observe_kernel(const EnvView v, const int8_t *__restrict__ actions, const M
         w = w1;
         cur = nxt;
     }
-    finish_work(work_counter, gridDim.x * (blockDim.x >> 5), lane);
+    finish_work(work_counter, gridDim.x * (blockDim.x >> 5), lane, v.order);
 }
 
 }  // namespace

@@ -56,15 +56,19 @@ step_observe_wide_kernel(const EnvView v, const int8_t *__restrict__ actions, co
     const uint64_t pol = policy_evict_last();
     // prefetch distance: worlds here are 2..8 times larger than in the warp-per-world kernel, so fewer of them make a batch
     const int pf_batch = 64, pf_ahead = (v.dbg_flags & (1 << 29)) ? -1 : 128;
+    const int dir = tid == 0 ? walk_dir(v) : 0;           // serpentine order (common.cuh world_of)
     for (;;) {
         __syncthreads();                                   // previous world fully written, grid / abits clean
-        if (tid == 0) s_world = atomicAdd(work_counter, 1);
+        if (tid == 0) {
+            const int c = atomicAdd(work_counter, 1);
+            s_world = world_of(v, c, dir);
+            // batched L2 prefetch of the state a few hundred claims ahead (common.cuh)
+            if (pf_ahead >= 0 && (c & (pf_batch - 1)) == 0) prefetch_world_batch(v, actions, c + pf_ahead, dir, pol, pf_batch);
+        }
         __syncthreads();
         const int w = s_world;
         if (w >= v.W) break;
-        // batched L2 prefetch of the state a few hundred worlds ahead (worlds are claimed in increasing order; common.cuh)
-        if (tid == 0 && pf_ahead >= 0 && (w & (pf_batch - 1)) == 0) prefetch_world_batch(v, actions, w + pf_ahead, pol, pf_batch);
-        expand_obstacle_rows(m.obits, v.obst_pack + (size_t)w * v.PW, v, tid, blockDim.x);
+        expand_obstacle_rows<true>(m.obits, v.obst_pack + (size_t)w * v.PW, v, tid, blockDim.x, pol);
         int rows = v.H, cols = v.Wd;
         if (v.use_da | v.use_hp) { if (v.dims) { rows = v.dims[2 * w]; cols = v.dims[2 * w + 1]; } }
         __syncthreads();
@@ -95,10 +99,7 @@ step_observe_wide_kernel(const EnvView v, const int8_t *__restrict__ actions, co
         }
     }
     __syncthreads();
-    if (tid == 0) {                                        // the last CTA to finish re-arms the counter
-        const int d = atomicAdd(work_counter + 1, 1);
-        if (d == (int)gridDim.x - 1) { work_counter[0] = 0; work_counter[1] = 0; }
-    }
+    finish_work(work_counter, gridDim.x, tid, v.order);   // the last CTA to finish re-arms the counter, flips the direction
 }
 
 struct WidePlan {

@@ -31,7 +31,7 @@ step_wide_kernel(const EnvView v, const int8_t *__restrict__ actions, const int8
     s.obits = reinterpret_cast<uint32_t *>(b); b += align16((size_t)HP * RW * 4);
     s.grid = b; b += align16((size_t)HP * GS);
     carve_scratch(s, b);
-    expand_obstacle_rows(s.obits, v.obst_pack + (size_t)w * v.PW, v, lane, 32);
+    expand_obstacle_rows<true>(s.obits, v.obst_pack + (size_t)w * v.PW, v, lane, 32, policy_evict_last());
     uint4 *g4 = reinterpret_cast<uint4 *>(s.grid);
     for (int k = lane; k < (HP * GS) / 16; k += 32) g4[k] = make_uint4(0, 0, 0, 0);
     __syncwarp();

@@ -64,24 +64,25 @@ __device__ __forceinline__ void step_wide_world(const EnvView &v, const int8_t *
     const int N = v.N, P = v.P, GS = v.GS, RW = v.RW;
     const size_t base = (size_t)w * N;
     uint32_t errbits = 0;
+    const uint64_t pol = policy_evict_last();         // residency rule (common.cuh)
 
     // ---- stage the agents ---------------------------------------------------------------------------------------------
-    const int tick = v.htick[w];
-    const int hlen = v.hlen[w];
-    const int2 ht = reinterpret_cast<const int2 *>(v.hcur)[w];
-    const int2 ht2 = reinterpret_cast<const int2 *>(v.hnx)[w];
+    const int tick = (int)ld_keep(v.htick + w, pol);
+    const int hlen = (int)ld_keep(v.hlen + w, pol);
+    const int2 ht = ld_keep_v2(reinterpret_cast<const int2 *>(v.hcur) + w, pol);
+    const int2 ht2 = ld_keep_v2(reinterpret_cast<const int2 *>(v.hnx) + w, pol);
     const int hr = (int16_t)(ht.x & 0xffff), hc = (int16_t)((uint32_t)ht.x >> 16);
     const int nr = (int16_t)(ht.y & 0xffff), nc = (int16_t)((uint32_t)ht.y >> 16);
     hnr = (int16_t)(ht2.y & 0xffff); hnc = (int16_t)((uint32_t)ht2.y >> 16);
     if (tid < K_COUNT) s.cnt[tid] = 0;
     for (int i = tid; i < N; i += nthreads) {
-        const uint32_t pw = reinterpret_cast<const uint32_t *>(v.pos)[base + i];
+        const uint32_t pw = ld_keep(reinterpret_cast<const uint32_t *>(v.pos) + base + i, pol);
         s.pos[i] = pw;
-        s.goal[i] = reinterpret_cast<const uint32_t *>(v.goal)[base + i];
+        s.goal[i] = ld_keep(reinterpret_cast<const uint32_t *>(v.goal) + base + i, pol);
         int a = actions[base + i];
         if (a < 0 || a >= NA) { errbits |= MAPF_ERR_BAD_ACTION; a = 0; }
         s.act[i] = (int8_t)a;
-        s.rep[i] = v.rep[base + i];
+        s.rep[i] = (int8_t)ld_keep_s8(v.rep + base + i, pol);
         const int r = (int16_t)(pw & 0xffff), c = (int16_t)(pw >> 16);
         s.grid[(r + P) * GS + c + P] = (uint8_t)(i + 1);
     }
@@ -159,13 +160,13 @@ __device__ __forceinline__ void step_wide_world(const EnvView &v, const int8_t *
             n_c1 += st == ST_STATIC; n_c2 += st == ST_HUMAN; n_c3 += st == ST_AGENT;
             need_fix |= (st == ST_STATIC || st == ST_HUMAN || st == ST_AGENT);
             if (MODE != MODE_JOINT) {
-                if (out.status) out.status[base + i] = (int8_t)st;
+                if (out.status) st_stream_u8(out.status + base + i, (uint32_t)st);
                 if (out.cost) {
                     const int d2 = (nr - tr) * (nr - tr) + (nc - tc) * (nc - tc);
-                    out.cost[base + i] = d2 < 25 ? (float)((5.0 - sqrt((double)d2)) / 5.0) : 0.0f;
+                    st_stream(out.cost + base + i, d2 < 25 ? (float)((5.0 - sqrt((double)d2)) / 5.0) : 0.0f);
                 }
-                if (MODE == MODE_EVALUATE && out.reward) out.reward[base + i] = st == ST_REPEAT ? -0.35f : st == ST_OK ? -0.3f : -2.0f;
-                if (MODE == MODE_EVALUATE && out.good_actions) out.good_actions[base + i] = s.good[i];
+                if (MODE == MODE_EVALUATE && out.reward) st_stream(out.reward + base + i, st == ST_REPEAT ? -0.35f : st == ST_OK ? -0.3f : -2.0f);
+                if (MODE == MODE_EVALUATE && out.good_actions) st_stream_u8(out.good_actions + base + i, s.good[i]);
                 if (out.train_valid) {
                     const uint32_t good = s.good[i], restr = s.restr[i], confl = s.confl[i];
 #pragma unroll
@@ -184,10 +185,10 @@ __device__ __forceinline__ void step_wide_world(const EnvView &v, const int8_t *
     }
     group_sync<CTA>();
     if (MODE != MODE_JOINT) {
-        if (tid == 0 && out.shadow_goals) out.shadow_goals[w] = s.cnt[K_SHADOW];
+        if (tid == 0 && out.shadow_goals) st_stream(out.shadow_goals + w, (uint32_t)s.cnt[K_SHADOW]);
         if (out.train_valid) {
             float *dst = out.train_valid + base * NA;
-            for (int k = tid; k < N * NA; k += nthreads) dst[k] = s.tv[k];
+            for (int k = tid; k < N * NA; k += nthreads) st_stream(dst + k, s.tv[k]);
         }
         if (MODE == MODE_EVALUATE) {
             if (errbits) atomicOr(reinterpret_cast<unsigned int *>(&s.cnt[K_ERR]), errbits);
@@ -295,33 +296,33 @@ __device__ __forceinline__ void step_wide_world(const EnvView &v, const int8_t *
             const bool arrived = nr_ == (int16_t)(gw & 0xffff) && nc_ == (int16_t)(gw >> 16);
             const bool viol = (h2r - nr_) * (h2r - nr_) + (h2c - nc_) * (h2c - nc_) <= 24;
             const uint32_t npw = (uint32_t)(uint16_t)nr_ | ((uint32_t)(uint16_t)nc_ << 16);
-            reinterpret_cast<uint32_t *>(v.pos)[base + i] = npw;
+            st_keep(reinterpret_cast<uint32_t *>(v.pos) + base + i, npw, pol);
             s.npos[i] = npw;
             s.cls[i] = (int8_t)arrived;                 // (the class array is free again: arrival flags for goal sampling)
             s.grid[((int16_t)(pw & 0xffff) + P) * GS + (int16_t)(pw >> 16) + P] = 0;       // leave the id grid clean
-            v.rep[base + i] = (int8_t)opp_of(f);
+            st_keep_s8(v.rep + base + i, opp_of(f), pol);
             if (arrived && !v.goal_sampling) {                                     // Sequence.getNext util.py:33-39
                 int k = v.qcur[base + i];
                 if (k >= v.Q) k = v.Q - 1; else v.qcur[base + i] = k + 1;
                 const uint32_t ngw = reinterpret_cast<const uint32_t *>(v.goal_queue)[(base + i) * v.Q + k];
-                reinterpret_cast<uint32_t *>(v.goal)[base + i] = ngw;
+                st_keep(reinterpret_cast<uint32_t *>(v.goal) + base + i, ngw, pol);
                 s.goal[i] = ngw;
             }
-            if (out.goals_reached) out.goals_reached[base + i] = arrived;
-            if (out.violated) out.violated[base + i] = viol;
-            if (out.fixed_actions) out.fixed_actions[base + i] = (int8_t)f;
+            if (out.goals_reached) st_stream_u8(out.goals_reached + base + i, arrived);
+            if (out.violated) st_stream_u8(out.violated + base + i, viol);
+            if (out.fixed_actions) st_stream_u8(out.fixed_actions + base + i, (uint32_t)f);
             if (MODE == MODE_FUSED && out.reward) {
                 const int st = s.st[i];
                 const float reward = st == ST_REPEAT ? -0.35f : st == ST_OK ? -0.3f : -2.0f;
-                out.reward[base + i] = arrived ? __fadd_rn(reward, 1.5f) : reward;           // runner.py:89-91
+                st_stream(out.reward + base + i, arrived ? __fadd_rn(reward, 1.5f) : reward);    // runner.py:89-91
             }
             if (MODE == MODE_FUSED && out.packed) {                              // MAPF_PACKED_* (include/mapf_b200.h)
                 const int st = s.st[i], a = s.act[i];
                 const int tr = (int16_t)(pw & 0xffff) + dr_of(a), tc = (int16_t)(pw >> 16) + dc_of(a);
                 const int d2 = (nr - tr) * (nr - tr) + (nc - tc) * (nc - tc);
                 const uint32_t sc = st == ST_STATIC ? 0u : st == ST_HUMAN ? 1u : st == ST_AGENT ? 2u : st == ST_REPEAT ? 3u : 4u;
-                out.packed[base + i] = (uint16_t)(sc | ((uint32_t)arrived << 3) | ((uint32_t)viol << 4) | ((uint32_t)f << 5) |
-                                                  ((uint32_t)min(d2, 25) << 8));
+                st_stream_u16(out.packed + base + i, sc | ((uint32_t)arrived << 3) | ((uint32_t)viol << 4) | ((uint32_t)f << 5) |
+                                                     ((uint32_t)min(d2, 25) << 8));
             }
             n_arr += arrived; n_viol += viol;
         }
@@ -355,7 +356,7 @@ __device__ __forceinline__ void step_wide_world(const EnvView &v, const int8_t *
                 if (!found) errbits |= MAPF_ERR_NO_FREE_CELL;
                 else {
                     __syncwarp();
-                    if (lane == 0) { s.goal[i] = chosen; reinterpret_cast<uint32_t *>(v.goal)[base + i] = chosen; }
+                    if (lane == 0) { s.goal[i] = chosen; st_keep(reinterpret_cast<uint32_t *>(v.goal) + base + i, chosen, pol); }
                     __syncwarp();
                 }
             }
@@ -364,15 +365,15 @@ __device__ __forceinline__ void step_wide_world(const EnvView &v, const int8_t *
     if (errbits) atomicOr(reinterpret_cast<unsigned int *>(&s.cnt[K_ERR]), errbits);
     group_sync<CTA>();
     if (tid == 0) {
-        v.htick[w] = t2;
-        reinterpret_cast<int2 *>(v.hcur)[w] = ht2;
+        st_keep(v.htick + w, (uint32_t)t2, pol);
+        st_keep_v2(reinterpret_cast<int2 *>(v.hcur) + w, ht2, pol);
         const int t3 = (t2 + 1 >= hlen) ? 0 : t2 + 1;
-        reinterpret_cast<int2 *>(v.hnx)[w] = *reinterpret_cast<const int2 *>(v.htrace + ((size_t)w * v.L + t3) * 4);
-        v.nstep[w] += 1;
+        st_keep_v2(reinterpret_cast<int2 *>(v.hnx) + w, ld_keep_v2(v.htrace + ((size_t)w * v.L + t3) * 4, pol), pol);
+        add_keep_s32(v.nstep + w, 1, pol);
         if (s.cnt[K_ERR]) atomicOr(v.err + w, (uint32_t)s.cnt[K_ERR]);
         long long *cn = v.counters + (size_t)w * 6;                              // util.py:56-65, runner.py:66-99
-        cn[0] += s.cnt[K_ARR]; cn[1] += s.cnt[K_SHADOW]; cn[2] += s.cnt[K_C1]; cn[3] += s.cnt[K_C2]; cn[4] += s.cnt[K_C3];
-        cn[5] += s.cnt[K_VIOL];
+        add_keep_s64(cn + 0, s.cnt[K_ARR], pol); add_keep_s64(cn + 1, s.cnt[K_SHADOW], pol); add_keep_s64(cn + 2, s.cnt[K_C1], pol);
+        add_keep_s64(cn + 3, s.cnt[K_C2], pol); add_keep_s64(cn + 4, s.cnt[K_C3], pol); add_keep_s64(cn + 5, s.cnt[K_VIOL], pol);
     }
 }
 

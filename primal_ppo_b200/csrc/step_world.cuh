@@ -80,7 +80,7 @@ __device__ __forceinline__ void load_step_world(const EnvView &v, const int8_t *
         r.ht = ld_keep_v2(reinterpret_cast<const int2 *>(v.hcur) + w, pol);
         r.ht2 = ld_keep_v2(reinterpret_cast<const int2 *>(v.hnx) + w, pol);
         r.tick = (int)ld_keep(v.htick + w, pol);
-        r.hlen = __ldg(v.hlen + w);
+        r.hlen = (int)ld_keep(v.hlen + w, pol);
     }
 }
 
@@ -187,15 +187,15 @@ __device__ __forceinline__ void resolve_world(const EnvView &v, const MapfStepOu
     const int d2 = (nr - tgt_r) * (nr - tgt_r) + (nc - tgt_c) * (nc - tgt_c);    // |human.getNextPos() - T(a)|^2 (:519)
     if (MODE != MODE_JOINT) {
         if (active) {
-            if (out.status) out.status[idx] = (int8_t)st;
+            if (out.status) st_stream_u8(out.status + idx, (uint32_t)st);
             if (out.cost) {
                 // max(PENALTY_RADIUS - ||H' - T||, 0) / PENALTY_RADIUS in f64, then cast (:513-533)
-                out.cost[idx] = d2 < 25 ? (float)((5.0 - sqrt((double)d2)) / 5.0) : 0.0f;
+                st_stream(out.cost + idx, d2 < 25 ? (float)((5.0 - sqrt((double)d2)) / 5.0) : 0.0f);
             }
-            if (MODE == MODE_EVALUATE && out.reward) out.reward[idx] = reward;
-            if (MODE == MODE_EVALUATE && out.good_actions) out.good_actions[idx] = (uint8_t)good;   // allGoodActions (:404-430)
+            if (MODE == MODE_EVALUATE && out.reward) st_stream(out.reward + idx, reward);
+            if (MODE == MODE_EVALUATE && out.good_actions) st_stream_u8(out.good_actions + idx, good);   // allGoodActions (:404-430)
         }
-        if (lane == 0 && out.shadow_goals) out.shadow_goals[w] = __popc(sgm);
+        if (lane == 0 && out.shadow_goals) st_stream(out.shadow_goals + w, (uint32_t)__popc(sgm));
         if (out.train_valid) {
             if (active) {
 #pragma unroll
@@ -206,7 +206,7 @@ __device__ __forceinline__ void resolve_world(const EnvView &v, const MapfStepOu
             }
             g.sync();
             float *dst = out.train_valid + (size_t)w * N * NA;
-            for (int k = lane; k < N * NA; k += G) dst[k] = s.tv[k];
+            for (int k = lane; k < N * NA; k += G) st_stream(dst + k, s.tv[k]);
         }
         if (MODE == MODE_EVALUATE) {
             const uint32_t eb = g.reduce_or(errbits);
@@ -408,14 +408,14 @@ __device__ __forceinline__ void resolve_world(const EnvView &v, const MapfStepOu
             }
             st_keep(reinterpret_cast<uint32_t *>(v.goal) + idx, new_gw, pol);
         }
-        if (out.goals_reached) out.goals_reached[idx] = arrived;
-        if (out.violated) out.violated[idx] = viol;
-        if (out.fixed_actions) out.fixed_actions[idx] = (int8_t)f;
-        if (MODE == MODE_FUSED && out.reward) out.reward[idx] = arrived ? __fadd_rn(reward, 1.5f) : reward;  // runner.py:89-91
+        if (out.goals_reached) st_stream_u8(out.goals_reached + idx, arrived);
+        if (out.violated) st_stream_u8(out.violated + idx, viol);
+        if (out.fixed_actions) st_stream_u8(out.fixed_actions + idx, (uint32_t)f);
+        if (MODE == MODE_FUSED && out.reward) st_stream(out.reward + idx, arrived ? __fadd_rn(reward, 1.5f) : reward);  // runner.py:89-91
         if (MODE == MODE_FUSED && out.packed) {                                  // MAPF_PACKED_* (include/mapf_b200.h)
             const uint32_t sc = st == ST_STATIC ? 0u : st == ST_HUMAN ? 1u : st == ST_AGENT ? 2u : st == ST_REPEAT ? 3u : 4u;
-            out.packed[idx] = (uint16_t)(sc | ((uint32_t)arrived << 3) | ((uint32_t)viol << 4) | ((uint32_t)f << 5) |
-                                         ((uint32_t)min(d2, 25) << 8));
+            st_stream_u16(out.packed + idx, sc | ((uint32_t)arrived << 3) | ((uint32_t)viol << 4) | ((uint32_t)f << 5) |
+                                                ((uint32_t)min(d2, 25) << 8));
         }
     }
     const uint32_t vm_ = g.ballot(viol);
@@ -426,11 +426,12 @@ __device__ __forceinline__ void resolve_world(const EnvView &v, const MapfStepOu
         st_keep(v.htick + w, (uint32_t)t2, pol);
         st_keep_v2(reinterpret_cast<int2 *>(v.hcur) + w, ht2, pol);
         const int t3 = (t2 + 1 >= in.hlen) ? 0 : t2 + 1;          // keep the entry after next resident too
-        st_keep_v2(reinterpret_cast<int2 *>(v.hnx) + w, *reinterpret_cast<const int2 *>(v.htrace + ((size_t)w * v.L + t3) * 4), pol);
-        v.nstep[w] += 1;
+        st_keep_v2(reinterpret_cast<int2 *>(v.hnx) + w, ld_keep_v2(v.htrace + ((size_t)w * v.L + t3) * 4, pol), pol);
+        add_keep_s32(v.nstep + w, 1, pol);
         if (eb) atomicOr(v.err + w, eb);
         long long *cn = v.counters + (size_t)w * 6;                              // util.py:56-65, runner.py:66-99
-        cn[0] += __popc(am); cn[1] += __popc(sgm); cn[2] += __popc(c1); cn[3] += __popc(c2b); cn[4] += __popc(c3); cn[5] += __popc(vm_);
+        add_keep_s64(cn + 0, __popc(am), pol); add_keep_s64(cn + 1, __popc(sgm), pol); add_keep_s64(cn + 2, __popc(c1), pol);
+        add_keep_s64(cn + 3, __popc(c2b), pol); add_keep_s64(cn + 4, __popc(c3), pol); add_keep_s64(cn + 5, __popc(vm_), pol);
     }
     g.sync();
     if (active) s.grid[gr * GS + gc] = 0;      // leave the id grid clean for the next world of this warp
