@@ -21,6 +21,15 @@ def _ptr(t):
     return None if t is None else C.c_void_p(t.data_ptr())
 
 
+def _mean_std(s: float, s2: float, n: float) -> Tuple[float, float]:
+    """Mean and unbiased std of n values from their sum and sum of squares.  The std of a single value is NaN, as
+    `x.std()` gives it in model.py:106 and loss.py, so a one-element minibatch yields a NaN loss instead of an error."""
+    mean = s / n
+    if n <= 1.0:
+        return mean, float("nan")
+    return mean, max((s2 - n * mean * mean) / (n - 1.0), 0.0) ** 0.5
+
+
 class _FusedPPOLoss(torch.autograd.Function):
     @staticmethod
     def forward(ctx, policy, value, cost_value, policy_sig, returns, cost_returns, old_v, old_cv, actions, old_ps, train_valid,
@@ -44,9 +53,8 @@ class _FusedPPOLoss(torch.autograd.Function):
                 dist.all_reduce(m, group=group)            # (sum a, sum a^2, sum c, sum c^2, count) of the GLOBAL minibatch
             m = m.tolist()
             ng = m[4]
-            am, cm = m[0] / ng, m[2] / ng
-            astd = max((m[1] - ng * am * am) / (ng - 1.0), 0.0) ** 0.5
-            cstd = max((m[3] - ng * cm * cm) / (ng - 1.0), 0.0) ** 0.5
+            am, astd = _mean_std(m[0], m[1], ng)
+            cm, cstd = _mean_std(m[2], m[3], ng)
             kc = _cabi.MapfPpoLossConfig(clip_range=cfg.clip_range, entropy_coef=cfg.entropy_coef, value_coef=cfg.value_coef,
                                          valid_coef=cfg.valid_coef, cost_value_coef=cfg.cost_value_coef, cost_coef=cfg.cost_coef,
                                          lagrangian=float(lagrangian), minus_adv_with_cadv=int(cfg.minus_adv_with_cadv),

@@ -9,6 +9,7 @@ import torch
 
 from golden_util import ENV_CASES, GOLDEN_DIR, Golden
 from oracle import OracleMapfGym, gae_oracle
+from ppo_loss_ref import gae_masked_ref
 from primal_ppo_b200 import random_actions, random_scenario
 
 pytestmark = pytest.mark.gpu
@@ -480,16 +481,7 @@ def test_gpu_gae_with_terminal_mask():
     r = rng.normal(size=(T, cols)).astype(np.float32); v = rng.normal(size=(T, cols)).astype(np.float32)
     lv = rng.normal(size=(cols,)).astype(np.float32)
     nt = (rng.random((T, cols)) > 0.1).astype(np.uint8)
-    g, gl = np.float32(0.95), np.float32(0.95 * 0.95)
-    ret = np.zeros_like(r); adv = np.zeros_like(r)
-    last = np.zeros(cols, dtype=np.float32); nv = lv.copy()
-    for t in range(T - 1, -1, -1):
-        m = nt[t].astype(bool)
-        m1 = np.where(m, g * nv, np.float32(0)).astype(np.float32)
-        delta = ((r[t] + m1).astype(np.float32) - v[t]).astype(np.float32)
-        m2 = np.where(m, gl * last, np.float32(0)).astype(np.float32)
-        last = (delta + m2).astype(np.float32)
-        adv[t] = last; ret[t] = (last + v[t]).astype(np.float32); nv = v[t]
+    ret, adv = gae_masked_ref(r, v, lv, nt)
     out, a = gae(torch.from_numpy(r).cuda(), torch.from_numpy(v).cuda(), torch.from_numpy(lv).cuda(),
                  nonterminal=torch.from_numpy(nt).cuda(), return_advantages=True)
     _eq(_np(out), ret, "masked returns"); _eq(_np(a), adv, "masked advantages")
