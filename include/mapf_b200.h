@@ -240,7 +240,8 @@ int mapf_get_counters(MapfEnv *env, int64_t *counters, void *stream);
  * map_generator.py:127-138, or the PRIMAL density map, map_generator.py:13-28), the human's entrance / goal / walk
  * (mapf_gym.py:9-50, astar_4.py) and the agents' starts and goals (populateMap mapf_gym.py:175-190, getFreeCell
  * util.py:67-76).  Philox4x32-10 keyed by (seed; world_offset + w, stream, draw): equal to the reference in distribution,
- * not in bits; the warehouse layout for a drawn length is bit-identical to generateWarehouse. */
+ * not in bits; the warehouse layout for a drawn length is bit-identical to generateWarehouse.  With human_path = 1 the
+ * walk between the drawn cells is astar_4's path, bit for bit. */
 typedef struct MapfGenConfig {
     int32_t num_worlds, height, width, num_agents; /* array shapes: every world is stored as height x width */
     int32_t kind;          /* 0 = density map, 1 = warehouse */
@@ -252,6 +253,9 @@ typedef struct MapfGenConfig {
     int32_t trace_len;     /* L ticks of human trace per world */
     int32_t human_loops;   /* 1 = LoopingHuman (one out-and-back walk, repeated); k > 1 = up to k walks with re-drawn goals
                               (Human.getNextGoal, mapf_gym.py:41-43) before the trace wraps */
+    int32_t human_path;    /* the human's walk to each goal: 0 = descent of the BFS field with neighbour order E, S, W, N (a
+                              shortest path, not astar_4's); 1 = astar_4 itself, bit-exact with its tie-breaking (the
+                              reference's MapfGym).  The draws, maps and walk lengths are the same for both. */
     uint64_t seed;
     int32_t world_offset;  /* global index of world 0 (sharded jobs) */
     int32_t device;
@@ -263,6 +267,14 @@ int mapf_generate_scenario(const MapfGenConfig *cfg, uint8_t *obst /*[W,H,Wd]*/,
                            int16_t *starts /*[W,N,2]*/, int16_t *goal_queue /*[W,N,Q,2]*/, int16_t *htrace /*[W,L,4]*/,
                            int32_t *hlen /*[W]*/, int16_t *hp5 /*[W,5,2] or NULL*/, uint32_t *gen_err /*[W] or NULL*/,
                            void *stream);
+
+/* astar_4 (astar_4.py:21-109) for n (map, start, goal) triples at once, bit-exact with its tie-breaking; one warp per
+ * triple.  obst [n,H,Wd] (nonzero = wall; 1 <= H, Wd <= 128), start_goal [n,2,2] as (row, col) pairs.  lens[i] = k >= 1
+ * for a path of k cells from start to goal inclusive, written to paths[i, :k]; 0 = start == goal; -1 = no path (the goal
+ * is a wall or unreachable; a walled start is still expanded); -2 = the path has more than max_len cells; -3 = start or
+ * goal outside the map.  Unused path cells are -1.  Asynchronous on stream; allocates nothing. */
+int mapf_astar4_paths(const uint8_t *obst, int64_t n, int32_t H, int32_t Wd, const int16_t *start_goal, int32_t max_len,
+                      int16_t *paths /*[n,max_len,2]*/, int32_t *lens /*[n]*/, void *stream);
 
 /* ---- host-buffer entry points (what a CPU-side runner calls; copies are inside the call) ---------------- */
 

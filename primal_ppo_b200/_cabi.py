@@ -16,7 +16,7 @@ EXPORTED = ["mapf_abi_version", "mapf_last_error", "mapf_create", "mapf_destroy"
             "mapf_sample_actions", "mapf_generate_scenario",
             "mapf_observe_bf16", "mapf_step_observe_bf16", "mapf_state_bytes", "mapf_save_state", "mapf_load_state",
             "mapf_get_human", "mapf_host_layout", "mapf_step_observe_host_begin", "mapf_step_observe_host_wait", "mapf_decode_results_host", "mapf_checksum_rows", "mapf_adv_moments", "mapf_ppo_loss",
-            "mapf_observe_bits", "mapf_step_observe_bits", "mapf_unpack_obs", "mapf_unpack_obs_host"]
+            "mapf_observe_bits", "mapf_step_observe_bits", "mapf_unpack_obs", "mapf_unpack_obs_host", "mapf_astar4_paths"]
 ABI_VERSION = 2
 
 def obs_bits_words(C: int, F: int) -> int:
@@ -39,7 +39,7 @@ class MapfGenConfig(C.Structure):
     _fields_ = [("num_worlds", C.c_int32), ("height", C.c_int32), ("width", C.c_int32), ("num_agents", C.c_int32),
                 ("kind", C.c_int32), ("density_mode", C.c_int32), ("density_lo", C.c_float), ("density_hi", C.c_float),
                 ("size_lo", C.c_int32), ("size_hi", C.c_int32), ("queue_len", C.c_int32), ("trace_len", C.c_int32),
-                ("human_loops", C.c_int32), ("seed", C.c_uint64), ("world_offset", C.c_int32), ("device", C.c_int32)]
+                ("human_loops", C.c_int32), ("human_path", C.c_int32), ("seed", C.c_uint64), ("world_offset", C.c_int32), ("device", C.c_int32)]
 
 
 class MapfScenario(C.Structure):
@@ -116,6 +116,7 @@ def load_library():
     lib.mapf_ppo_loss.argtypes = [C.POINTER(MapfPpoLossConfig), i64] + [vp] * 17
     lib.mapf_sample_actions.argtypes = [vp, i64, C.c_uint64, C.c_uint32, vp, vp, vp]
     lib.mapf_generate_scenario.argtypes = [C.POINTER(MapfGenConfig)] + [vp] * 9
+    lib.mapf_astar4_paths.argtypes = [vp, i64, i32, i32, vp, i32, vp, vp, vp]
     lib.mapf_state_bytes.argtypes = [vp]
     lib.mapf_save_state.argtypes = [vp, vp, vp]
     lib.mapf_load_state.argtypes = [vp, vp, vp]

@@ -20,7 +20,8 @@ OBJ = os.path.join(CSRC, "_obj")
 LIB_PATH = os.path.join(_PKG, "libmapf_b200.so")
 HEADER = os.path.join(os.path.dirname(_PKG), "include", "mapf_b200.h")
 SOURCES = ["mapf_api.cu", "step.cu", "step_wide.cu", "observe.cu", "observe_wide.cu", "step_observe.cu",
-           "step_observe_wide.cu", "bfs.cu", "gae.cu", "glue.cu", "scenario_gen.cu", "ppo_loss.cu", "obs_bits.cu"]
+           "step_observe_wide.cu", "bfs.cu", "gae.cu", "glue.cu", "scenario_gen.cu", "ppo_loss.cu", "obs_bits.cu",
+           "astar4.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC,-fvisibility=default"]
 LINK_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-shared", "-cudart", "shared"]

@@ -364,6 +364,8 @@ cudaError_t launch_checksum_rows(const uint32_t *data, long long rows, long long
 
 cudaError_t launch_scenario_gen(const MapfGenConfig &c, uint8_t *obst, int16_t *dims, int16_t *starts, int16_t *goal_queue,
                                 int16_t *htrace, int32_t *hlen, int16_t *hp5, uint32_t *gen_err, cudaStream_t s);
+cudaError_t launch_astar4_paths(const uint8_t *obst, long long n, int H, int Wd, const int16_t *start_goal, int max_len,
+                                int16_t *paths, int32_t *lens, cudaStream_t s);
 
 constexpr int MODE_EVALUATE = 0, MODE_JOINT = 1, MODE_FUSED = 2;
 

@@ -473,8 +473,19 @@ int mapf_generate_scenario(const MapfGenConfig *c, uint8_t *obst, int16_t *dims,
         if (c->size_lo > 0 && (c->size_hi < c->size_lo || c->size_hi > c->height || c->size_hi > c->width))
             return fail(MAPF_E_BAD_CONFIG, "mapf_generate_scenario: size range does not fit height x width");
     } else return fail(MAPF_E_BAD_CONFIG, "mapf_generate_scenario: kind must be 0 (density) or 1 (warehouse)");
+    if (c->human_path != 0 && c->human_path != 1)
+        return fail(MAPF_E_BAD_CONFIG, "mapf_generate_scenario: human_path must be 0 (BFS descent) or 1 (astar_4)");
     ON_DEVICE(c->device);
     CU(launch_scenario_gen(*c, obst, dims, starts, goal_queue, htrace, hlen, hp5, gen_err, (cudaStream_t)stream));
+    return MAPF_OK;
+}
+
+int mapf_astar4_paths(const uint8_t *obst, int64_t n, int32_t H, int32_t Wd, const int16_t *start_goal, int32_t max_len,
+                      int16_t *paths, int32_t *lens, void *stream) {
+    if (!obst || !start_goal || !paths || !lens) return fail(MAPF_E_NULL, "mapf_astar4_paths: null argument");
+    if (n < 0 || H < 1 || H > 128 || Wd < 1 || Wd > 128 || max_len < 1)
+        return fail(MAPF_E_BAD_CONFIG, "mapf_astar4_paths: need n >= 0, 1 <= H, Wd <= 128 and max_len >= 1");
+    CU(launch_astar4_paths(obst, n, H, Wd, start_goal, max_len, paths, lens, (cudaStream_t)stream));
     return MAPF_OK;
 }
 

@@ -8,12 +8,15 @@
 //   agents     starts and first goals: sequential rejection sampling on a scratch map that marks the human, earlier
 //              starts and earlier goals (populateMap, mapf_gym.py:175-190); later goals: free cells (mapf_gym.py:626)
 // Here one warp builds one world with Philox4x32-10 keyed by (seed; global world index, stream, draw).  The results are
-// EQUAL IN DISTRIBUTION to the reference's, not in bits (different generator; astar_4's tie-breaking among equally
-// short paths is replaced by a fixed neighbour order on the BFS field; later goals are drawn at reset, so they avoid
-// obstacles and the previous goal but cannot avoid the agents' future cells).  The warehouse layout itself is a
+// EQUAL IN DISTRIBUTION to the reference's, not in bits (different generator; later goals are drawn at reset, so they
+// avoid obstacles and the previous goal but cannot avoid the agents' future cells).  The walk between the drawn cells
+// depends on human_path: 1 is astar_4's path itself, bit-exact with its tie-breaking (astar4.cuh), so for the same map,
+// entrance and goals the walk is the reference's; 0 (the default) descends the BFS field with a fixed neighbour order,
+// another shortest path.  Both have the same length, so every draw and the trace's timing are the same in both modes.  The warehouse layout itself is a
 // deterministic function of the drawn length and is bit-identical to generateWarehouse (tests/golden/warehouse_maps.npz).
 // Output arrays are exactly the MapfScenario arrays of include/mapf_b200.h, written in HBM, so mapf_reset consumes
 // them without a host round trip.
+#include "astar4.cuh"
 #include "common.cuh"
 
 namespace mapf {
@@ -22,7 +25,7 @@ namespace {
 
 struct GenView {
     int W, H, Wd, N, Q, L;
-    int kind, density_mode, size_lo, size_hi, human_loops;
+    int kind, density_mode, size_lo, size_hi, human_loops, human_path;
     float dlo, dhi;
     unsigned long long seed;
     int world_offset;
@@ -51,13 +54,17 @@ __device__ __forceinline__ float u01(uint32_t r) { return (float)(r >> 8) * 5.96
 
 enum { S_DIMS = 0, S_CELLS = 1, S_HUMAN = 2, S_START = 3, S_GOAL = 4, S_QUEUE = 5 };
 
-// per-warp shared memory: free-cell flags (1 = free and inside dims), occupancy flags, BFS distances
+// per-warp shared memory: free-cell flags (1 = free and inside dims), occupancy flags, BFS distances; with human_path = 1
+// the A* search reuses dist as its g and fw / nf as its open / closed sets, and adds a level set and the parents
 struct GenSmem {
     uint8_t *freec;     // [H*Wd]
     uint8_t *occ;       // [H*Wd]
     int16_t *dist;      // [H*Wd]
     uint32_t *fw, *nf;  // [ceil(H*Wd/32)] frontier bit sets of the current / next BFS level
+    uint32_t *lvl, *par;
 };
+__host__ __device__ constexpr int gen_set_words(int cells) { return (astar4_words(cells) + 3) & ~3; }
+__host__ __device__ constexpr int gen_par_words(int cells) { return ((cells + 15) / 16 + 3) & ~3; }
 
 __global__ void __launch_bounds__(128) scenario_gen_kernel(const GenView g, const int per_warp) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -72,7 +79,10 @@ __global__ void __launch_bounds__(128) scenario_gen_kernel(const GenView g, cons
     s.dist = reinterpret_cast<int16_t *>(base + 2 * ((cells + 15) & ~15));
     const int fwords = (cells + 31) / 32;
     s.fw = reinterpret_cast<uint32_t *>(base + 2 * ((cells + 15) & ~15) + ((cells * 2 + 15) & ~15));
-    s.nf = s.fw + ((fwords + 3) & ~3);
+    s.nf = s.fw + gen_set_words(cells);
+    s.lvl = s.nf + gen_set_words(cells);          // only inside the per-warp block when human_path = 1
+    s.par = s.lvl + gen_set_words(cells);
+    const Astar4Smem as{s.dist, s.fw, s.nf, s.lvl, s.par};
     const uint32_t gw = (uint32_t)(w + g.world_offset);
     uint32_t err = 0;
 
@@ -177,6 +187,12 @@ __global__ void __launch_bounds__(128) scenario_gen_kernel(const GenView g, cons
         for (int attempt = 0; attempt < 4 && d < 0; ++attempt) {
             goal = draw_cell(S_HUMAN, 2 + (uint32_t)loop * 8 + attempt, false);
             if (goal < 0 || goal == cur) { goal = -1; continue; }
+            if (g.human_path == 1) {
+                // astar_path(map, cur, goal): a shortest path, so d is the BFS distance and every draw stays the same
+                d = astar4_search(as, H, Wd, cur, goal, [&](int c) { return s.freec[c] != 0; });
+                if (d >= 0 && tick + 2 * d + 1 > g.L && loop == 0 && attempt < 3) d = -1;
+                continue;
+            }
             // BFS distance field from the goal: level-synchronous, the frontier kept as a bit set so that a level
             // costs work proportional to the frontier, not to the grid
             for (int c = lane; c < cells; c += 32) s.dist[c] = -1;
@@ -216,8 +232,15 @@ __global__ void __launch_bounds__(128) scenario_gen_kernel(const GenView g, cons
             break;
         }
         if (tick + 2 * d + 1 > g.L) break;               // a further loop that does not fit: wrap the trace here
-        // out: follow decreasing distance (neighbour order E, S, W, N); back: the same cells reversed
-        if (lane == 0) {
+        // out: astar_4's path, or decreasing distance (neighbour order E, S, W, N); back: the same cells reversed
+        if (lane == 0 && g.human_path == 1) {
+            for (int c = goal;; c = astar4_parent(as, Wd, c)) {    // cell c is the k-th of the path, k = its g
+                const int k = as.g[c];
+                tr[(tick + k) * 4 + 0] = tr[(tick + 2 * d - k) * 4 + 0] = (int16_t)(c / Wd);
+                tr[(tick + k) * 4 + 1] = tr[(tick + 2 * d - k) * 4 + 1] = (int16_t)(c % Wd);
+                if (k == 0) break;
+            }
+        } else if (lane == 0) {
             int c = cur;
             for (int k = 0; k <= d; ++k) {
                 tr[(tick + k) * 4 + 0] = (int16_t)(c / Wd); tr[(tick + k) * 4 + 1] = (int16_t)(c % Wd);
@@ -229,6 +252,8 @@ __global__ void __launch_bounds__(128) scenario_gen_kernel(const GenView g, cons
                 else if (x > 0 && s.dist[c - 1] == want) c = c - 1;
                 else c = c - Wd;
             }
+        }
+        if (lane == 0) {
             // next = path[s+1], or path[-1] on the last tick of the loop (getNextPos, mapf_gym.py:46-50)
             for (int k = 0; k < 2 * d + 1; ++k) {
                 const int nk = k + 1 < 2 * d + 1 ? k + 1 : k;
@@ -305,12 +330,13 @@ cudaError_t launch_scenario_gen(const MapfGenConfig &c, uint8_t *obst, int16_t *
     g.W = c.num_worlds; g.H = c.height; g.Wd = c.width; g.N = c.num_agents; g.Q = c.queue_len; g.L = c.trace_len;
     g.kind = c.kind; g.density_mode = c.density_mode; g.size_lo = c.size_lo; g.size_hi = c.size_hi;
     g.human_loops = c.human_loops < 1 ? 1 : c.human_loops;
+    g.human_path = c.human_path;
     g.dlo = c.density_lo; g.dhi = c.density_hi; g.seed = c.seed; g.world_offset = c.world_offset;
     g.obst = obst; g.dims = dims; g.starts = starts; g.goal_queue = goal_queue; g.htrace = htrace; g.hp5 = hp5;
     g.hlen = hlen; g.gen_err = gen_err;
     const int cells = c.height * c.width;
-    const int fwords = (cells + 31) / 32;
-    const int per_warp = 2 * ((cells + 15) & ~15) + ((cells * 2 + 15) & ~15) + 2 * ((fwords + 3) & ~3) * 4;
+    const int per_warp = 2 * ((cells + 15) & ~15) + ((cells * 2 + 15) & ~15) + 2 * gen_set_words(cells) * 4 +
+                         (c.human_path == 1 ? (gen_set_words(cells) + gen_par_words(cells)) * 4 : 0);
     int wpb = 4;
     while (wpb > 1 && per_warp * wpb > 160 * 1024) wpb >>= 1;
     const size_t smem = (size_t)per_warp * wpb;

@@ -65,16 +65,19 @@ def generate_scenario_device(num_worlds: int, height: int, width: int, num_agent
                              density=(0.0, 0.3), triangular: bool = False, size_range=None, queue_len: int = 16,
                              trace_len: Optional[int] = None, human_loops: int = 1, seed: int = 0, world_offset: int = 0,
                              device=None, fov: int = 9, num_channel: int = 6, use_da: bool = False,
-                             use_hp: bool = False) -> DeviceScenario:
+                             use_hp: bool = False, human_path: str = "bfs") -> DeviceScenario:
     """kind="warehouse": `generateWarehouse(num_block=size_range)` worlds (training env; default size_range (10, 40)
     needs height >= 40, width >= 60).  kind="density": `rand < p` maps, p per world from `density`; `size_range` =
-    (lo, hi) draws the side like `random_generator`, None keeps height x width."""
+    (lo, hi) draws the side like `random_generator`, None keeps height x width.
+    human_path="astar4" walks the human along astar_4's path to each goal, bit-exact with the reference's `MapfGym()`;
+    "bfs" (the default) along another shortest path (a BFS descent).  Everything else is the same for both."""
     if not torch.cuda.is_available():
         raise _cabi.MapfError("generate_scenario_device needs a CUDA device; there is no CPU fallback")
     lib = _cabi.load_library()
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     W, H, Wd, N, Q = num_worlds, height, width, num_agents, queue_len
     k = {"density": 0, "warehouse": 1}[kind]
+    hp = {"bfs": 0, "astar4": 1}[human_path]
     if k == 1 and size_range is None:
         size_range = (10, 40)
     lo, hi = (0, 0) if size_range is None else (int(size_range[0]), int(size_range[1]))
@@ -84,10 +87,12 @@ def generate_scenario_device(num_worlds: int, height: int, width: int, num_agent
                         goal_queue=z(W, N, Q, 2, dt=torch.int16), htrace=z(W, L, 4, dt=torch.int16),
                         hlen=z(W, dt=torch.int32), dims=z(W, 2, dt=torch.int16), hp5=z(W, 5, 2, dt=torch.int16),
                         gen_err=z(W, dt=torch.int32), fov=fov, num_channel=num_channel, use_da=use_da, use_hp=use_hp,
-                        meta=dict(kind=kind, density=list(density), size_range=[lo, hi], seed=seed, generator="device"))
+                        meta=dict(kind=kind, density=list(density), size_range=[lo, hi], seed=seed, generator="device",
+                                  human_path=human_path))
     cfg = _cabi.MapfGenConfig(num_worlds=W, height=H, width=Wd, num_agents=N, kind=k, density_mode=int(triangular),
                               density_lo=float(density[0]), density_hi=float(density[1]), size_lo=lo, size_hi=hi,
-                              queue_len=Q, trace_len=L, human_loops=int(human_loops), seed=int(seed) & (2 ** 64 - 1),
+                              queue_len=Q, trace_len=L, human_loops=int(human_loops), human_path=hp,
+                              seed=int(seed) & (2 ** 64 - 1),
                               world_offset=int(world_offset), device=dev.index or 0)
     p = lambda t: C.c_void_p(t.data_ptr())
     stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
@@ -96,3 +101,28 @@ def generate_scenario_device(num_worlds: int, height: int, width: int, num_agent
                                                p(sc.htrace), p(sc.hlen), p(sc.hp5), p(sc.gen_err), stream),
                     "mapf_generate_scenario")
     return sc
+
+
+def astar_paths_device(obst: torch.Tensor, start_goal: torch.Tensor, max_len: Optional[int] = None):
+    """astar_4 paths for n (map, start, goal) triples in one `mapf_astar4_paths` call, bit-exact with
+    `episode_io.astar_path`.  obst: CUDA uint8 [n,H,Wd] (nonzero = wall), start_goal: int16 [n,2,2] (row, col) pairs on
+    the same device.  Returns (paths i16 [n,max_len,2], lens i32 [n]) on that device: lens k >= 1 is a path of k cells,
+    0 start == goal, -1 no path, -2 longer than max_len (default H * Wd, every path fits), -3 a cell outside the map;
+    unused path cells are -1.  Asynchronous on the current stream."""
+    lib = _cabi.load_library()
+    if not (obst.is_cuda and obst.dtype == torch.uint8 and obst.dim() == 3):
+        raise ValueError("astar_paths_device: obst must be a CUDA uint8 tensor [n,H,Wd]")
+    n, H, Wd = obst.shape
+    if start_goal.shape != (n, 2, 2) or start_goal.dtype != torch.int16 or start_goal.device != obst.device:
+        raise ValueError("astar_paths_device: start_goal must be int16 [n,2,2] on the device of obst")
+    L = H * Wd if max_len is None else int(max_len)
+    obst, start_goal = obst.contiguous(), start_goal.contiguous()
+    paths = torch.empty((n, max(L, 0), 2), dtype=torch.int16, device=obst.device)
+    lens = torch.empty((n,), dtype=torch.int32, device=obst.device)
+    if n == 0:
+        return paths, lens
+    p = lambda t: C.c_void_p(t.data_ptr())
+    with torch.cuda.device(obst.device):
+        stream = C.c_void_p(torch.cuda.current_stream(obst.device).cuda_stream)
+        _cabi.check(lib.mapf_astar4_paths(p(obst), n, H, Wd, p(start_goal), L, p(paths), p(lens), stream), "mapf_astar4_paths")
+    return paths, lens

@@ -99,10 +99,11 @@ def astar_path(world: np.ndarray, start: Cell, goal: Cell) -> Optional[List[Cell
     return None
 
 
-def looping_human_ticks(world: np.ndarray, start: Cell, goal: Cell) -> np.ndarray:
+def looping_human_ticks(world: np.ndarray, start: Cell, goal: Cell, astar=astar_path) -> np.ndarray:
     """(pos, next) per tick of `LoopingHuman(world, start, goal)` (`mapf_gym.py:52-70`): out along the A* path, back along
-    the same cells, then from the top.  i16 [L, 4]."""
-    out = astar_path(world, start, goal)
+    the same cells, then from the top.  i16 [L, 4].  `astar(world, a, b)` plans the walk (`astar_path` or its results
+    looked up from the device)."""
+    out = astar(world, start, goal)
     if out is None:
         raise ValueError(f"no path from {start} to {goal}")
     if not out:
@@ -113,16 +114,16 @@ def looping_human_ticks(world: np.ndarray, start: Cell, goal: Cell) -> np.ndarra
     return np.concatenate([p, nxt], axis=1)
 
 
-def fixed_path_human_ticks(world: np.ndarray, pose_sequence: Seq[Cell], ticks: int):
+def fixed_path_human_ticks(world: np.ndarray, pose_sequence: Seq[Cell], ticks: int, astar=astar_path):
     """(pos, next) and `path[1:6]` per tick of `FixedPathHuman(world, humanPoseSequence)` (`mapf_gym.py:72-94` on top of
     `Human.nextStep/getNextPos`, `:25-50`) for `ticks` ticks: walk to each pose in turn; once the sequence is exhausted the
     walker jumps back to the start of its last path and repeats it (reference quirk, SURVEY Appendix B).
-    Returns (i16 [ticks, 4], i16 [ticks, 5, 2])."""
+    `astar` as in `looping_human_ticks`.  Returns (i16 [ticks, 4], i16 [ticks, 5, 2])."""
     seq = [(int(p[0]), int(p[1])) for p in pose_sequence]
     pos, idx = seq[0], 1
 
     def plan(a, b):
-        p = astar_path(world, a, b)
+        p = astar(world, a, b)
         if p is None:
             raise ValueError(f"no path from {a} to {b}")
         return p
@@ -150,12 +151,15 @@ def fixed_path_human_ticks(world: np.ndarray, pose_sequence: Seq[Cell], ticks: i
 # ---- fixture -> batched scenario ------------------------------------------------------------------------------------
 def scenario_from_fixed_episode_infos(infos: Dict, *, human_movement_type: int = 0, max_steps: int = 256,
                                       num_channel: int = 6, use_da: bool = False, use_hp: bool = False,
-                                      fov: int = 9, episodes: Optional[Seq[int]] = None) -> Scenario:
+                                      fov: int = 9, episodes: Optional[Seq[int]] = None, device=None) -> Scenario:
     """All (or the selected) fixed episodes as the worlds of one `Scenario` — what `evaluate.py:212-218` passes to
     `FixedMapfGym`, batched.  `human_movement_type` 0 = looping human between humanStart / humanGoal, 1 = the fixed pose
     sequence (`EvalParameters.HUMAN_MOVEMENT_TYPE`, `alg_parameters.py:10`, `evaluate.py:216-217`).
     Maps of different sizes are padded to the largest (`dims` keeps each world's true size); goal sequences of different
-    lengths are padded by repeating the last goal, which is what `Sequence.getNext` does (`util.py:33-36`)."""
+    lengths are padded by repeating the last goal, which is what `Sequence.getNext` does (`util.py:33-36`).
+    With a CUDA `device`, every A* leg the host would plan is solved in one `mapf_astar4_paths` call (bit-exact with
+    `astar_path`) and the same arrays are built from those paths; the result is byte-identical to `device=None` and the
+    same errors are raised, for the same legs."""
     eps = list(range(int(infos["numEpisodes"]))) if episodes is None else list(episodes)
     maps = [np.asarray(infos["obstacleMap"][e]) for e in eps]
     W = len(eps)
@@ -168,9 +172,12 @@ def scenario_from_fixed_episode_infos(infos: Dict, *, human_movement_type: int =
     dims = np.zeros((W, 2), dtype=np.int16)
     starts = np.zeros((W, N, 2), dtype=np.int16)
     queue = np.zeros((W, N, Q, 2), dtype=np.int16)
-    traces, hp5s = [], []
-    for w, (e, m) in enumerate(zip(eps, maps)):
+    for w, m in enumerate(maps):
         obst[w, :m.shape[0], :m.shape[1]] = (m != 0)
+    traces, hp5s = [], []
+    plan = ((lambda w, world, a, b: astar_path(world, a, b)) if device is None else
+            _device_planner(infos, eps, maps, obst, human_movement_type, max_steps + 2, device))
+    for w, (e, m) in enumerate(zip(eps, maps)):
         dims[w] = m.shape
         for i, items in enumerate(seqs[w]):
             if len(items) < 2:
@@ -181,13 +188,15 @@ def scenario_from_fixed_episode_infos(infos: Dict, *, human_movement_type: int =
             queue[w, i, len(g):] = g[-1]
         world = np.where(m != 0, -1, 0)
         if human_movement_type == 0:
-            tr = looping_human_ticks(world, infos["humanStart"][e], infos["humanGoal"][e])
+            tr = looping_human_ticks(world, infos["humanStart"][e], infos["humanGoal"][e],
+                                     lambda world, a, b: plan(w, world, a, b))
             h5 = np.full((5, 2), -1, dtype=np.int16)
             k = min(5, tr.shape[0] - 1)
             h5[:k] = tr[1:1 + k, :2]
             hp5s.append(h5)
         else:
-            tr, h5 = fixed_path_human_ticks(world, infos["humanSequence"][e], max_steps + 2)
+            tr, h5 = fixed_path_human_ticks(world, infos["humanSequence"][e], max_steps + 2,
+                                           lambda world, a, b: plan(w, world, a, b))
             hp5s.append(h5)
         traces.append(tr)
     L = max(t.shape[0] for t in traces)
@@ -209,6 +218,42 @@ def scenario_from_fixed_episode_infos(infos: Dict, *, human_movement_type: int =
                   meta=dict(kind="fixed_episode_infos", episodes=eps, human_movement_type=human_movement_type))
     sc.validate()
     return sc
+
+
+def _device_planner(infos, eps, maps, obst, mtype, ticks, device):
+    """plan(w, world, a, b) = astar_path(world, a, b) for world w of the batch, answered from one device call that solves
+    every leg the host could plan: humanStart -> humanGoal (LoopingHuman), or the consecutive poses of humanSequence a
+    FixedPathHuman can reach within `ticks` ticks (leg j starts no earlier than tick 2 (j - 1): every leg lasts at least
+    two ticks, and an empty one raises).  A leg with a cell outside its world's own map is malformed input that the
+    padded device map cannot represent; it is planned by astar_path itself, so it behaves as on the host."""
+    import torch
+    from .device_scenario import astar_paths_device
+    reqs = {}
+    for w, e in enumerate(eps):
+        if mtype == 0:
+            pairs = [(infos["humanStart"][e], infos["humanGoal"][e])]
+        else:
+            seq = infos["humanSequence"][e]
+            pairs = list(zip(seq[:-1], seq[1:]))[:ticks // 2 + 1]
+        for a, b in pairs:
+            a, b = (int(a[0]), int(a[1])), (int(b[0]), int(b[1]))
+            h, wd = maps[w].shape
+            if all(0 <= r < h and 0 <= c < wd for r, c in (a, b)):
+                reqs.setdefault((w, a, b), len(reqs))
+    keys = list(reqs)
+    sg = np.array([[a, b] for _, a, b in keys], dtype=np.int16).reshape(-1, 2, 2)
+    dev = torch.device(device)
+    widx = torch.tensor([w for w, _, _ in keys], dtype=torch.int64, device=dev)
+    paths, lens = astar_paths_device(torch.from_numpy(obst).to(dev)[widx], torch.from_numpy(sg).to(dev))
+    paths, lens = paths.cpu().numpy(), lens.cpu().numpy()
+
+    def plan(w, world, a, b):
+        i = reqs.get((w, (int(a[0]), int(a[1])), (int(b[0]), int(b[1]))))
+        if i is None:
+            return astar_path(world, a, b)
+        k = int(lens[i])
+        return None if k < 0 else [(int(r), int(c)) for r, c in paths[i, :k]]
+    return plan
 
 
 # ---- a plain frame renderer (own design; the reference's `_render` draws cv2 polygons, mapf_gym.py:639-646) --------------
